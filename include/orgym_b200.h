@@ -160,6 +160,33 @@ int orgym_invmgmt_export_state(orgym_handle_t h, const void* state_dev, int64_t*
 #define ORGYM_POLICY_ACTIONS 0    /* pre-staged actions */
 #define ORGYM_POLICY_BASE_STOCK 1 /* benchmark_InvManagementBacklogEnv.py:142-198; param[0] = safety factor, param[1] = mu */
 #define ORGYM_POLICY_RANDOM 2     /* a_i ~ U{0..c_i} from a separate Philox sub-stream */
+#define ORGYM_POLICY_MLP 3        /* actor network evaluated on the device, in->mlp */
+
+/* A trained multilayer-perceptron actor (e.g. stable-baselines3's MlpPolicy: policy_net + action_net), evaluated inside
+ * the fused rollout.  Each period the network sees exactly the observation step() returns (inventory_management.py:
+ * 354-391): I[t] first, then the last min(t, lt_max) requested orders, left-aligned and oldest first, zeros after them.
+ * Numerics:
+ *   x   = float32(obs)                  round to nearest (= torch .float())
+ *   h_l = act(W_l h_{l-1} + b_l)        float32; each output: acc = b, then acc = fmaf(w_k, x_k, acc) for k = 0..K-1
+ *                                       ascending (no split-K, no cross-env reduction); act = tanhf (the accurate one,
+ *                                       not tanh.approx) or max(x, 0) with NaN kept
+ *   y   = W_L h_{L-1} + b_L             no activation after the last Linear
+ *   q_i = (int64) trunc(min(max((double)y_i, 0), (double)c_i)),   NaN -> 0
+ * i.e. SB3's deterministic predict for a Box action space (the Gaussian mean clipped to [low, high]) followed by the
+ * env's own float-action rule (max(a, 0), truncation, :250).  Requests lie in [0, c_i], so sampled-demand MLP rollouts
+ * use the compact int32 arithmetic exactly like the base-stock policy, and results are a pure function of (weights,
+ * seed, global env id, episode): independent of batch size, launch geometry and env_offset sharding. */
+#define ORGYM_MLP_MAX_LAYERS 4
+#define ORGYM_MLP_MAX_WIDTH 256
+#define ORGYM_MLP_TANH 1
+#define ORGYM_MLP_RELU 2
+typedef struct {
+    int32_t num_layers;                            /* Linear layers, 1..ORGYM_MLP_MAX_LAYERS */
+    int32_t activation;                            /* ORGYM_MLP_TANH | ORGYM_MLP_RELU, after every Linear but the last */
+    int32_t width[ORGYM_MLP_MAX_LAYERS + 1];       /* width[0] = obs_dim, width[num_layers] = m-1 */
+    const float* weight_dev[ORGYM_MLP_MAX_LAYERS]; /* [width[l+1]][width[l]] row-major = torch.nn.Linear.weight */
+    const float* bias_dev[ORGYM_MLP_MAX_LAYERS];   /* [width[l+1]] or NULL */
+} orgym_mlp_t;
 
 typedef struct {
     int32_t policy;
@@ -172,6 +199,10 @@ typedef struct {
     int64_t dem_stride_env, dem_stride_t;
     /* device scratch of orgym_invmgmt_rollout_scratch_bytes(h) bytes; may be NULL when that is 0 (almost always) */
     void* scratch_dev;
+    /* HOST pointer, read only when policy == ORGYM_POLICY_MLP.  ORGYM_E_INVALID for a malformed network (layer count,
+     * widths outside 1..ORGYM_MLP_MAX_WIDTH or not matching obs_dim / m-1, null weights); ORGYM_E_UNSUPPORTED when the
+     * weights, activations, observation tile and lead-time rings of one CTA do not fit in shared memory. */
+    const orgym_mlp_t* mlp;
 } orgym_invmgmt_rollout_in_t;
 
 /* per-episode results; every pointer may be NULL.  stats columns are the reference evaluator's metrics
@@ -184,6 +215,7 @@ typedef struct {
     int64_t* final_B_dev;    /* [N,m] */
     double* summary_dev;     /* [8] batch sums: n, sum ret, sum ret^2, sum sales, sum demand, sum stockout, sum end inv, 0 */
     int32_t* stats32_dev;    /* [N,4] the same statistics as stats_dev, saturated to int32 (halves the result traffic) */
+    int64_t* action_traj_dev; /* [N,T,m-1] requested orders per period (the reference's action_log, :268); any policy */
 } orgym_invmgmt_rollout_out_t;
 
 /* fused reset + `periods` steps of every env with state held on chip (no state_dev needed).
@@ -201,9 +233,11 @@ int64_t orgym_invmgmt_rollout_scratch_bytes(orgym_handle_t h);
  * generated as straight-line CUDA (lead-time rings in registers, every index, price and base-stock level a literal, so
  * the compiler folds whatever does not depend on the demand; the profit in integer arithmetic when the generator can
  * prove that no float64 operation of the reference's expression rounds) and compiled for sm_100a with NVRTC.  Results
- * are bit-identical to the ahead-of-time kernel.
+ * are bit-identical to the ahead-of-time kernel.  Rollouts that request reward_traj, final_I/B or action_traj, and
+ * ORGYM_POLICY_MLP rollouts, always run the ahead-of-time kernels (also under ORGYM_INV_JIT=2).
  *   orgym_invmgmt_specialise  builds the kernel for in->policy / in->param now (ORGYM_OK), or says why it cannot:
- *                             ORGYM_E_UNSUPPORTED = configuration / policy outside the specialiser's range,
+ *                             ORGYM_E_UNSUPPORTED = configuration / policy outside the specialiser's range
+ *                             (ORGYM_POLICY_MLP is never specialised),
  *                             ORGYM_E_CUDA = NVRTC unavailable or the compile failed; orgym_last_error() has the log.
  *                             Without this call the first eligible rollout builds it (up to 16 variants per handle).
  *   environment ORGYM_INV_JIT 0 = ahead-of-time kernels only; 1 (default) = specialise, fall back silently to the

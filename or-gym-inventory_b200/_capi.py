@@ -40,15 +40,26 @@ class InvInfo(C.Structure):
                 ("profit", C.c_void_p), ("final_obs", C.c_void_p), ("info_ld", C.c_int64)]
 
 
+MLP_MAX_LAYERS, MLP_MAX_WIDTH, MLP_TANH, MLP_RELU = 4, 256, 1, 2
+
+
+class Mlp(C.Structure):
+    """orgym_mlp_t: an actor network evaluated inside the fused rollout (device pointers to float32 weights)."""
+    _fields_ = [("num_layers", C.c_int32), ("activation", C.c_int32), ("width", C.c_int32 * (MLP_MAX_LAYERS + 1)),
+                ("weight", C.c_void_p * MLP_MAX_LAYERS), ("bias", C.c_void_p * MLP_MAX_LAYERS)]
+
+
 class InvRolloutIn(C.Structure):
     _fields_ = [("policy", C.c_int32), ("param", C.c_double * 4), ("actions", C.c_void_p),
                 ("act_stride_env", C.c_int64), ("act_stride_t", C.c_int64), ("demand", C.c_void_p),
-                ("dem_stride_env", C.c_int64), ("dem_stride_t", C.c_int64), ("scratch", C.c_void_p)]
+                ("dem_stride_env", C.c_int64), ("dem_stride_t", C.c_int64), ("scratch", C.c_void_p),
+                ("mlp", C.POINTER(Mlp))]
 
 
 class InvRolloutOut(C.Structure):
     _fields_ = [("ep_return", C.c_void_p), ("stats", C.c_void_p), ("reward_traj", C.c_void_p),
-                ("final_I", C.c_void_p), ("final_B", C.c_void_p), ("summary", C.c_void_p), ("stats32", C.c_void_p)]
+                ("final_I", C.c_void_p), ("final_B", C.c_void_p), ("summary", C.c_void_p), ("stats32", C.c_void_p),
+                ("action_traj", C.c_void_p)]
 
 
 class NvConfig(C.Structure):

@@ -578,12 +578,109 @@ struct InvRolloutArgs {
     int64_t* final_I;
     int64_t* final_B;
     int32_t* stats32;
-    double* partials;  // [gridDim.x][8]
+    int64_t* action_traj;  // [N][T][n]
+    double* partials;  // [ceil(N / ROLL_THREADS)][8]: one row per 128 envs, whatever the CTA size
     void* ring_scratch;    // non-null: the rings do not fit in shared memory and live here as [slot][ring_stride]
     int64_t ring_stride;   // >= round_up(N, ROLL_THREADS)
 };
 
 #define ROLL_THREADS 128
+
+// ---- pieces shared by the fused rollout kernels (inv_rollout_kernel, inv_mlp_rollout_kernel) --------------------------
+// per-episode accumulators of one env; the statistics are kept in the state type: the int32 instantiations are only
+// launched when the host has bounded every per-episode sum below 2^31 (orgym_invmgmt_rollout), otherwise S = int64
+template <typename S>
+struct InvRollAcc {
+    double ret;
+    S sales, dem, stock, inv;
+};
+
+// one period after the policy has chosen req[]: lead-time ring slot rbase + rpos holds R[t - L_i] (zero before t = L_i)
+// and receives this period's fulfilled order; demand is replayed, a user trace or one Philox block per four periods
+// through the alias table.  The caller advances the ring positions.
+template <int NS, bool EXACT, typename S, typename RI>
+__device__ __forceinline__ void inv_roll_period(const InvDev& P, const InvRolloutArgs& A, const uint2* tab, uint64_t key,
+                                                int64_t e, bool valid, int t, int n, const S (&req)[NS], S* rring,
+                                                const RI (&rbase)[NS], const RI (&rpos)[NS], S (&I)[NS], S (&B)[NS + 1],
+                                                uint4& w, InvRollAcc<S>& acc, double* rtraj) {
+    S arr[NS], Rf[NS], U[NS + 1];
+#pragma unroll
+    for (int i = 0; i < NS; i++)
+        if (EXACT || i < n) arr[i] = rring[rbase[i] + rpos[i]];
+    long long dl;
+    if (A.demand)
+        dl = valid ? A.demand[e * A.d_se + (int64_t)t * A.d_st] : 0;
+    else if (P.dem.kind == ORGYM_DIST_USER)
+        dl = t < P.dem.user_D_len ? P.dem.user_D[t] : 0;
+    else {
+        if ((t & 3) == 0) w = philox_block(key, (uint32_t)t >> 2, A.episode, STREAM_DEMAND, 0u);
+        dl = alias_draw(tab, P.dem.log2k, P.dem.base, pick_word(w, t & 3));
+    }
+    S s0;
+    double profit = inv_period<NS, EXACT, S>(P, req, arr, (S)dl, I, B, Rf, s0, U);
+    double reward = P.disc[t] * profit;
+    acc.ret += reward;  // Python: total += reward, in period order
+    if (rtraj) rtraj[t] = reward;
+    acc.sales += s0;
+    acc.dem += (S)dl > 0 ? (S)dl : (S)0;
+    acc.stock += U[0];
+#pragma unroll
+    for (int i = 0; i < NS; i++)
+        if (EXACT || i < n) acc.inv += I[i] > 0 ? I[i] : (S)0;
+#pragma unroll
+    for (int i = 0; i < NS; i++)
+        if (EXACT || i < n) rring[rbase[i] + rpos[i]] = Rf[i];
+}
+
+// per-episode outputs of one env
+template <int NS, typename S>
+__device__ __forceinline__ void inv_roll_outputs(const InvRolloutArgs& A, int64_t e, int n, const InvRollAcc<S>& acc,
+                                                 const S (&I)[NS], const S (&B)[NS + 1]) {
+    if (A.ep_return) A.ep_return[e] = acc.ret;
+    if (A.stats) {
+        longlong4 v = make_longlong4((long long)acc.sales, (long long)acc.dem, (long long)acc.stock, (long long)acc.inv);
+        *reinterpret_cast<longlong4*>(A.stats + e * 4) = v;
+    }
+    if (A.stats32) {
+        auto sat = [](long long v) { return (int)(v > 2147483647LL ? 2147483647LL : (v < -2147483648LL ? -2147483648LL : v)); };
+        *reinterpret_cast<int4*>(A.stats32 + e * 4) =
+            make_int4(sat((long long)acc.sales), sat((long long)acc.dem), sat((long long)acc.stock), sat((long long)acc.inv));
+    }
+    if (A.final_I)
+        for (int i = 0; i < n; i++) A.final_I[e * n + i] = (int64_t)I[i];
+    if (A.final_B)
+        for (int j = 0; j <= n; j++) A.final_B[e * (n + 1) + j] = (int64_t)B[j];
+}
+
+// batch summary, first stage: the 7 sums of one warp of 32 consecutive envs (butterfly shuffles) into red[7]
+template <typename S>
+__device__ __forceinline__ void inv_roll_warp_sums(bool valid, const InvRollAcc<S>& acc, double* red) {
+    double v[7];
+    v[0] = valid ? 1.0 : 0.0;
+    v[1] = valid ? acc.ret : 0.0;
+    v[2] = valid ? acc.ret * acc.ret : 0.0;
+    v[3] = valid ? (double)acc.sales : 0.0;
+    v[4] = valid ? (double)acc.dem : 0.0;
+    v[5] = valid ? (double)acc.stock : 0.0;
+    v[6] = valid ? (double)acc.inv : 0.0;
+#pragma unroll
+    for (int q = 0; q < 7; q++) {
+        double x = v[q];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+        if ((threadIdx.x & 31) == 0) red[q] = x;
+    }
+}
+
+// second stage (threads 0..6, after a barrier): the four warp rows of 128 envs, in warp order, into one partials row
+__device__ __forceinline__ void inv_roll_partials_row(const double (*red)[7], double* row) {
+    const int q = threadIdx.x;
+    if (q < 7) {
+        double x = 0.0;
+        for (int wv = 0; wv < ROLL_THREADS / 32; wv++) x += red[wv][q];
+        row[q] = x;
+    }
+}
 
 template <int NS, bool EXACT, typename S>
 __global__ void __launch_bounds__(ROLL_THREADS) inv_rollout_kernel(const __grid_constant__ InvDev P,
@@ -628,15 +725,13 @@ __global__ void __launch_bounds__(ROLL_THREADS) inv_rollout_kernel(const __grid_
     }
 #pragma unroll
     for (int j = 0; j <= NS; j++) B[j] = 0;
-    double ret = 0.0;
-    // episode statistics in the state type: the int32 instantiation is only launched when the host has bounded every
-    // per-episode sum below 2^31 (orgym_invmgmt_rollout), otherwise S = int64
-    S s_sales = 0, s_dem = 0, s_stock = 0, s_inv = 0;
+    InvRollAcc<S> acc = {0.0, 0, 0, 0, 0};
     uint4 w = make_uint4(0, 0, 0, 0);
     double* const rtraj = (A.reward_traj && valid) ? A.reward_traj + e * P.T : nullptr;
+    int64_t* const atraj = (A.action_traj && valid) ? A.action_traj + e * P.T * n : nullptr;
 
     for (int t = 0; t < P.T; t++) {
-        S req[NS], arr[NS], Rf[NS], U[NS + 1];
+        S req[NS];
         // ---- policy ---------------------------------------------------------------------------------------
         if (A.policy == ORGYM_POLICY_BASE_STOCK) {
             // benchmark_InvManagementBacklogEnv.py:152-198: position = on-hand + requested orders of the last L_i
@@ -680,38 +775,17 @@ __global__ void __launch_bounds__(ROLL_THREADS) inv_rollout_kernel(const __grid_
                     req[i] = (S)a;
                 }
         }
-        // ---- lead-time rings: slot rpos holds R[t - L_i] (zero before t = L_i) ----------------------------------
+        if (atraj)
 #pragma unroll
-        for (int i = 0; i < NS; i++)
-            if (EXACT || i < n) arr[i] = rring[rbase[i] + rpos[i]];
-        // ---- demand: one Philox block serves four periods ---------------------------------------------------------
-        long long dl;
-        if (A.demand)
-            dl = valid ? A.demand[e * A.d_se + (int64_t)t * A.d_st] : 0;
-        else if (P.dem.kind == ORGYM_DIST_USER)
-            dl = t < P.dem.user_D_len ? P.dem.user_D[t] : 0;
-        else {
-            if ((t & 3) == 0) w = philox_block(key, (uint32_t)t >> 2, A.episode, STREAM_DEMAND, 0u);
-            dl = alias_draw(tab, P.dem.log2k, P.dem.base, pick_word(w, t & 3));
-        }
-        S s0;
-        double profit = inv_period<NS, EXACT, S>(P, req, arr, (S)dl, I, B, Rf, s0, U);
-        double reward = P.disc[t] * profit;
-        ret += reward;  // Python: total += reward, in period order
-        if (rtraj) rtraj[t] = reward;
-        s_sales += s0;
-        s_dem += (S)dl > 0 ? (S)dl : (S)0;
-        s_stock += U[0];
-#pragma unroll
-        for (int i = 0; i < NS; i++)
-            if (EXACT || i < n) s_inv += I[i] > 0 ? I[i] : (S)0;
-        // ---- ring updates (branch-free) ------------------------------------------------------------------------
+            for (int i = 0; i < NS; i++)
+                if (EXACT || i < n) atraj[t * n + i] = (int64_t)req[i];
+        inv_roll_period<NS, EXACT, S, RI>(P, A, tab, key, e, valid, t, n, req, rring, rbase, rpos, I, B, w, acc, rtraj);
+        // ---- request ring (base-stock position) and ring advance (branch-free) ----------------------------------
 #pragma unroll
         for (int i = 0; i < NS; i++)
             if (EXACT || i < n) {
-                const RI slot = rbase[i] + rpos[i];
-                rring[slot] = Rf[i];
                 if (need_aring) {
+                    const RI slot = rbase[i] + rpos[i];
                     S old = aring[slot];
                     aring[slot] = req[i];
                     psum[i] = (psum[i] + req[i] - old) & lmask[i];  // stays 0 for a stage without lead time
@@ -721,46 +795,214 @@ __global__ void __launch_bounds__(ROLL_THREADS) inv_rollout_kernel(const __grid_
             }
     }
     // ---- per-episode outputs --------------------------------------------------------------------------------------
-    if (valid) {
-        if (A.ep_return) A.ep_return[e] = ret;
-        if (A.stats) {
-            longlong4 v = make_longlong4((long long)s_sales, (long long)s_dem, (long long)s_stock, (long long)s_inv);
-            *reinterpret_cast<longlong4*>(A.stats + e * 4) = v;
-        }
-        if (A.stats32) {
-            auto sat = [](long long v) { return (int)(v > 2147483647LL ? 2147483647LL : (v < -2147483648LL ? -2147483648LL : v)); };
-            *reinterpret_cast<int4*>(A.stats32 + e * 4) =
-                make_int4(sat((long long)s_sales), sat((long long)s_dem), sat((long long)s_stock), sat((long long)s_inv));
-        }
-        if (A.final_I)
-            for (int i = 0; i < n; i++) A.final_I[e * n + i] = (int64_t)I[i];
-        if (A.final_B)
-            for (int j = 0; j <= n; j++) A.final_B[e * (n + 1) + j] = (int64_t)B[j];
-    }
+    if (valid) inv_roll_outputs<NS, S>(A, e, n, acc, I, B);
     // ---- batch summary: warp shuffles -> one row of partials per CTA (summed in fixed order afterwards) -------
     if (A.partials) {
-        double v[7];
-        v[0] = valid ? 1.0 : 0.0;
-        v[1] = valid ? ret : 0.0;
-        v[2] = valid ? ret * ret : 0.0;
-        v[3] = valid ? (double)s_sales : 0.0;
-        v[4] = valid ? (double)s_dem : 0.0;
-        v[5] = valid ? (double)s_stock : 0.0;
-        v[6] = valid ? (double)s_inv : 0.0;
         __shared__ double red[ROLL_THREADS / 32][7];
+        inv_roll_warp_sums<S>(valid, acc, red[tid >> 5]);
+        __syncthreads();
+        inv_roll_partials_row(red, A.partials + (size_t)blockIdx.x * 8);
+    }
+}
+
+// ---- fused rollout driven by an MLP actor (ORGYM_POLICY_MLP) ----------------------------------------------------------
+// One CTA = 128 consecutive envs (one row of the partial sums, like inv_rollout_kernel), run as 128/E sub-tiles of E
+// envs one after the other; weights and biases are staged in shared memory once per CTA.  Thread tid < E owns env
+// e0 + tid of the current sub-tile (integer state in registers, lead-time ring in shared memory).  Per period the whole
+// CTA evaluates the network on the sub-tile's observations as a register-tiled SGEMM: activations are feature-major
+// [feature][env] float32 tiles, each thread computes blocks of MLP_TE envs x MLP_TN neurons, so one 16-byte load of
+// activations and one of weights feed 16 FMAs.  The observation tile itself is the request window (shifted in place).
+#define MLP_THREADS 256
+#define MLP_TE 4
+#define MLP_TN 4
+
+struct InvMlpPlan {
+    int L, act, E, log2E;
+    int K[ORGYM_MLP_MAX_LAYERS + 1];   // widths
+    int Np[ORGYM_MLP_MAX_LAYERS];      // output widths of the hidden layers padded to MLP_TN (zero weights and biases)
+    const float* W[ORGYM_MLP_MAX_LAYERS];
+    const float* b[ORGYM_MLP_MAX_LAYERS];
+    // shared memory: alias table at 0 | float area at fbase (offsets in floats) | lead-time ring at ring_off (bytes)
+    int w_off[ORGYM_MLP_MAX_LAYERS], b_off[ORGYM_MLP_MAX_LAYERS], obs_off, buf_off[2], y_off;
+    int fbase, ring_off;
+};
+
+__device__ __forceinline__ float mlp_act(float x, int act) {
+    // accurate tanhf (tanh.approx.f32 has ~2^-11 relative error: far more truncated actions would flip); ReLU keeps NaN
+    return act == ORGYM_MLP_TANH ? tanhf(x) : (x < 0.f ? 0.f : x);
+}
+
+// out[n][e] = act(b[n] + sum_k Wt[k][n] in[k][e]) for the E envs of the tile; each output accumulates in k order
+__device__ __forceinline__ void mlp_hidden_layer(const float* __restrict__ in, float* __restrict__ out,
+                                                 const float* __restrict__ Wt, const float* __restrict__ bias, int K,
+                                                 int Np, int E, int log2E, int act) {
+    const int egs = E / MLP_TE, log2egs = log2E - 2;
+    const int ntile = egs * (Np / MLP_TN);
+    for (int tile = threadIdx.x; tile < ntile; tile += MLP_THREADS) {
+        const int eg = tile & (egs - 1), ng = tile >> log2egs;
+        const float* xp = in + eg * MLP_TE;
+        const float* wp = Wt + ng * MLP_TN;
+        const float4 bv = *reinterpret_cast<const float4*>(bias + ng * MLP_TN);
+        float acc[MLP_TE][MLP_TN];
 #pragma unroll
-        for (int q = 0; q < 7; q++) {
-            double x = v[q];
+        for (int i = 0; i < MLP_TE; i++) {
+            acc[i][0] = bv.x;
+            acc[i][1] = bv.y;
+            acc[i][2] = bv.z;
+            acc[i][3] = bv.w;
+        }
+#pragma unroll 4
+        for (int k = 0; k < K; k++) {
+            const float4 x4 = *reinterpret_cast<const float4*>(xp + k * E);
+            const float4 w4 = *reinterpret_cast<const float4*>(wp + k * Np);
+            const float x[4] = {x4.x, x4.y, x4.z, x4.w}, w[4] = {w4.x, w4.y, w4.z, w4.w};
 #pragma unroll
-            for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
-            if ((tid & 31) == 0) red[tid >> 5][q] = x;
+            for (int i = 0; i < MLP_TE; i++)
+#pragma unroll
+                for (int j = 0; j < MLP_TN; j++) acc[i][j] = __fmaf_rn(w[j], x[i], acc[i][j]);
+        }
+#pragma unroll
+        for (int j = 0; j < MLP_TN; j++)
+            *reinterpret_cast<float4*>(out + (ng * MLP_TN + j) * E + eg * MLP_TE) =
+                make_float4(mlp_act(acc[0][j], act), mlp_act(acc[1][j], act), mlp_act(acc[2][j], act),
+                            mlp_act(acc[3][j], act));
+    }
+}
+
+template <int NS, bool EXACT, typename S>
+__global__ void __launch_bounds__(MLP_THREADS, (EXACT && NS <= 4 && sizeof(S) == 4) ? 3 : 2) inv_mlp_rollout_kernel(const __grid_constant__ InvDev P,
+                                                                      const __grid_constant__ InvRolloutArgs A,
+                                                                      const __grid_constant__ InvMlpPlan M) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ double red[ROLL_THREADS / 32][7];
+    const int n = EXACT ? NS : P.n;
+    const int tid = threadIdx.x;
+    const int E = M.E, L = M.L;
+    uint2* tab = (uint2*)smem;
+    float* fs = (float*)(smem + M.fbase);
+    S* rring = (S*)(smem + M.ring_off);
+    float* obs = fs + M.obs_off;
+    float* y = fs + M.y_off;
+    const int K = (P.dem.kind == ORGYM_DIST_USER) ? 0 : (1 << P.dem.log2k);
+    for (int i = tid; i < K; i += MLP_THREADS) tab[i] = P.dem.table[i];
+    // weights: hidden layers transposed to [k][Np] (zero-padded columns), the last layer as given ([n][K] row-major)
+    for (int l = 0; l < L; l++) {
+        const int Kl = M.K[l], Nl = M.K[l + 1];
+        const float* Wg = M.W[l];
+        const float* bg = M.b[l];
+        float* Ws = fs + M.w_off[l];
+        float* bs = fs + M.b_off[l];
+        if (l < L - 1) {
+            const int Np = M.Np[l];
+            for (int idx = tid; idx < Kl * Np; idx += MLP_THREADS) {
+                const int k = idx / Np, j = idx - k * Np;
+                Ws[idx] = j < Nl ? Wg[(size_t)j * Kl + k] : 0.f;
+            }
+            for (int j = tid; j < Np; j += MLP_THREADS) bs[j] = (j < Nl && bg) ? bg[j] : 0.f;
+        } else {
+            for (int idx = tid; idx < Kl * Nl; idx += MLP_THREADS) Ws[idx] = Wg[idx];
+            for (int j = tid; j < Nl; j += MLP_THREADS) bs[j] = bg ? bg[j] : 0.f;
+        }
+    }
+    const int Lm = P.lt_max, od = P.obs_dim;
+    const int Klast = M.K[L - 1];
+    const float* Wlast = fs + M.w_off[L - 1];
+    const float* blast = fs + M.b_off[L - 1];
+    const float* hin = L == 1 ? obs : fs + M.buf_off[(L - 2) & 1];  // input of the last layer
+    const int nsub = ROLL_THREADS / E;
+    for (int sub = 0; sub < nsub; sub++) {
+        const int64_t e0 = (int64_t)blockIdx.x * ROLL_THREADS + (int64_t)sub * E;
+        const bool owner = tid < E;
+        const int64_t e = e0 + tid;
+        const bool valid = owner && e < A.N;
+        if (e0 >= A.N) {  // CTA-uniform: the sums of the missing warps are zero, like idle lanes of inv_rollout_kernel
+            if (tid < 7 * (E / 32)) red[sub * (E / 32) + tid / 7][tid % 7] = 0.0;
+            continue;
+        }
+        const uint64_t key = A.seed + (uint64_t)(A.env_offset + e);
+        S I[NS], B[NS + 1];
+        int rbase[NS], rpos[NS], rlen[NS];
+#pragma unroll
+        for (int i = 0; i < NS; i++) {
+            I[i] = (EXACT || i < n) ? (S)P.I0[i] : (S)0;
+            rbase[i] = A.rroff[i] * E + tid;
+            rpos[i] = 0;
+            rlen[i] = (P.L[i] > 0 ? P.L[i] : 1) * E;
+        }
+#pragma unroll
+        for (int j = 0; j <= NS; j++) B[j] = 0;
+        InvRollAcc<S> acc = {0.0, 0, 0, 0, 0};
+        uint4 w = make_uint4(0, 0, 0, 0);
+        double* const rtraj = (A.reward_traj && valid) ? A.reward_traj + e * P.T : nullptr;
+        int64_t* const atraj = (A.action_traj && valid) ? A.action_traj + e * P.T * n : nullptr;
+        if (owner) {  // first observation [I0, 0, ...] and empty rings
+            for (int k = 0; k < od; k++) obs[k * E + tid] = k < n ? (float)(S)P.I0[k] : 0.f;
+            for (int k = 0; k < A.rslots; k++) rring[k * E + tid] = 0;
         }
         __syncthreads();
-        if (tid < 7) {
-            double x = 0.0;
-            for (int wv = 0; wv < ROLL_THREADS / 32; wv++) x += red[wv][tid];
-            A.partials[(size_t)blockIdx.x * 8 + tid] = x;
+        for (int t = 0; t < P.T; t++) {
+            // ---- policy: the network on the observation tile ------------------------------------------------------
+            const float* in = obs;
+            for (int l = 0; l < L - 1; l++) {
+                float* out = fs + M.buf_off[l & 1];
+                mlp_hidden_layer(in, out, fs + M.w_off[l], fs + M.b_off[l], M.K[l], M.Np[l], E, M.log2E, M.act);
+                __syncthreads();
+                in = out;
+            }
+            for (int idx = tid; idx < n * E; idx += MLP_THREADS) {  // last layer: one output of one env per thread
+                const int i = idx >> M.log2E, ee = idx & (E - 1);
+                const float* wr = Wlast + i * Klast;
+                float a = blast[i];
+                for (int k = 0; k < Klast; k++) a = __fmaf_rn(wr[k], hin[k * E + ee], a);
+                y[idx] = a;
+            }
+            __syncthreads();
+            if (owner) {
+                S req[NS];
+#pragma unroll
+                for (int i = 0; i < NS; i++)
+                    if (EXACT || i < n) {  // clip to [0, c_i] in float64 (NaN -> 0), truncate (:250)
+                        double v = (double)y[i * E + tid];
+                        v = v > 0.0 ? v : 0.0;
+                        const double cap = (double)P.c[i];
+                        v = v < cap ? v : cap;
+                        req[i] = (S)(long long)v;
+                    }
+                if (atraj)
+#pragma unroll
+                    for (int i = 0; i < NS; i++)
+                        if (EXACT || i < n) atraj[t * n + i] = (int64_t)req[i];
+                inv_roll_period<NS, EXACT, S, int>(P, A, tab, key, e, valid, t, n, req, rring, rbase, rpos, I, B, w, acc,
+                                                   rtraj);
+#pragma unroll
+                for (int i = 0; i < NS; i++)
+                    if (EXACT || i < n) {
+                        const int np1 = rpos[i] + E;
+                        rpos[i] = np1 == rlen[i] ? 0 : np1;
+                    }
+                // ---- observation of period t+1: I, then the window of the last min(t+1, lt_max) requests -----------
+#pragma unroll
+                for (int i = 0; i < NS; i++)
+                    if (EXACT || i < n) obs[i * E + tid] = (float)I[i];
+                if (Lm > 0) {
+                    int q = t;
+                    if (t >= Lm) {  // full window: drop the oldest request
+                        for (int k = n; k < od - n; k++) obs[k * E + tid] = obs[(k + n) * E + tid];
+                        q = Lm - 1;
+                    }
+#pragma unroll
+                    for (int i = 0; i < NS; i++)
+                        if (EXACT || i < n) obs[(n + q * n + i) * E + tid] = (float)req[i];
+                }
+            }
+            __syncthreads();
         }
+        if (valid) inv_roll_outputs<NS, S>(A, e, n, acc, I, B);
+        if (A.partials && owner) inv_roll_warp_sums<S>(valid, acc, red[sub * (E / 32) + (tid >> 5)]);
+    }
+    if (A.partials) {
+        __syncthreads();
+        inv_roll_partials_row(red, A.partials + (size_t)blockIdx.x * 8);
     }
 }
 
@@ -801,6 +1043,94 @@ static void launch_rollout(const InvHandle* H, const InvRolloutArgs& A, size_t s
             inv_rollout_kernel<MAXN, false, S><<<grid, ROLL_THREADS, smem, s>>>(P, A);
     }
 #undef ROLL_CASE
+}
+
+template <typename S>
+static void launch_mlp_rollout(const InvHandle* H, const InvRolloutArgs& A, const InvMlpPlan& M, size_t smem,
+                               cudaStream_t s) {
+    const InvDev& P = H->dev;
+    unsigned grid = (unsigned)((A.N + ROLL_THREADS - 1) / ROLL_THREADS);
+#define MLP_CASE(NSV)                                                                                                  \
+    case NSV:                                                                                                          \
+        orgym_ensure_dyn_smem<inv_mlp_rollout_kernel<NSV, true, S>>(smem);                                           \
+        inv_mlp_rollout_kernel<NSV, true, S><<<grid, MLP_THREADS, smem, s>>>(P, A, M);                                 \
+        break;
+    switch (P.n) {
+        MLP_CASE(1) MLP_CASE(2) MLP_CASE(3) MLP_CASE(4) MLP_CASE(5) MLP_CASE(6)
+        default:
+            orgym_ensure_dyn_smem<inv_mlp_rollout_kernel<MAXN, false, S>>(smem);
+            inv_mlp_rollout_kernel<MAXN, false, S><<<grid, MLP_THREADS, smem, s>>>(P, A, M);
+    }
+#undef MLP_CASE
+}
+
+// Checks an orgym_mlp_t against the handle (ORGYM_E_INVALID) and lays out one CTA's shared memory for it: the largest
+// sub-tile of E in {64, 32} envs whose working set fits (ORGYM_E_UNSUPPORTED, with the sizes, when none does).
+#define MLP_SMEM_BUDGET (227 * 1024 - 1024)  // sm_100 opt-in limit per block, less the static partial-sum rows
+static int inv_mlp_plan(const InvDev& P, const orgym_mlp_t* mlp, int rslots, size_t ring_elem, InvMlpPlan* M,
+                        size_t* smem_out) {
+    ORGYM_REQUIRE(mlp, "policy ORGYM_POLICY_MLP needs in->mlp");
+    const int L = mlp->num_layers;
+    ORGYM_REQUIRE(L >= 1 && L <= ORGYM_MLP_MAX_LAYERS, "mlp: num_layers = %d, must be 1..%d", L, ORGYM_MLP_MAX_LAYERS);
+    ORGYM_REQUIRE(L == 1 || mlp->activation == ORGYM_MLP_TANH || mlp->activation == ORGYM_MLP_RELU,
+                  "mlp: activation %d is neither ORGYM_MLP_TANH nor ORGYM_MLP_RELU", mlp->activation);
+    for (int l = 0; l <= L; l++)
+        ORGYM_REQUIRE(mlp->width[l] >= 1 && mlp->width[l] <= ORGYM_MLP_MAX_WIDTH, "mlp: width[%d] = %d outside 1..%d", l,
+                      mlp->width[l], ORGYM_MLP_MAX_WIDTH);
+    ORGYM_REQUIRE(mlp->width[0] == P.obs_dim, "mlp: width[0] = %d differs from obs_dim = %d", mlp->width[0], P.obs_dim);
+    ORGYM_REQUIRE(mlp->width[L] == P.n, "mlp: width[%d] = %d differs from the action dimension m-1 = %d", L, mlp->width[L],
+                  P.n);
+    for (int l = 0; l < L; l++) ORGYM_REQUIRE(mlp->weight_dev[l], "mlp: weight_dev[%d] is NULL", l);
+    memset(M, 0, sizeof(*M));
+    M->L = L;
+    M->act = L > 1 ? mlp->activation : ORGYM_MLP_TANH;
+    int hmax = 0;
+    for (int l = 0; l <= L; l++) M->K[l] = mlp->width[l];
+    for (int l = 0; l < L; l++) {
+        M->W[l] = mlp->weight_dev[l];
+        M->b[l] = mlp->bias_dev[l];
+        if (l < L - 1) {
+            M->Np[l] = (int)round_up(M->K[l + 1], MLP_TN);
+            hmax = std::max(hmax, M->Np[l]);
+        }
+    }
+    auto a4 = [](int x) { return (int)round_up(x, 4); };  // float offsets stay 16-byte aligned
+    int f = 0;
+    for (int l = 0; l < L; l++) {
+        M->w_off[l] = f;
+        f += a4(M->K[l] * (l < L - 1 ? M->Np[l] : M->K[l + 1]));
+        M->b_off[l] = f;
+        f += a4(l < L - 1 ? M->Np[l] : M->K[l + 1]);
+    }
+    const int wfloats = f;
+    const size_t tab = P.dem.kind == ORGYM_DIST_USER ? 0 : (size_t(8) << P.dem.log2k);
+    const int nbuf = L >= 3 ? 2 : (L == 2 ? 1 : 0);
+    size_t smem = 0;
+    for (int E = 64; E >= 32; E /= 2) {
+        int g = wfloats;
+        M->obs_off = g;
+        g += P.obs_dim * E;
+        M->buf_off[0] = g;
+        g += nbuf >= 1 ? hmax * E : 0;
+        M->buf_off[1] = g;
+        g += nbuf >= 2 ? hmax * E : 0;
+        M->y_off = g;
+        g += a4(P.n * E);
+        M->fbase = (int)round_up((int64_t)tab, 16);
+        M->ring_off = (int)round_up(M->fbase + (int64_t)g * 4, 16);
+        smem = (size_t)M->ring_off + (size_t)rslots * E * ring_elem;
+        M->E = E;
+        M->log2E = E == 64 ? 6 : 5;
+        if (smem <= MLP_SMEM_BUDGET) break;
+    }
+    if (smem > MLP_SMEM_BUDGET) {
+        orgym_set_error("mlp: one CTA of 32 envs needs %zu bytes of shared memory (weights and biases %d floats, observation "
+                        "tile %d x 32, %d activation tile(s) %d x 32, lead-time rings %d slots); this build's limit is %d",
+                        smem, wfloats, P.obs_dim, nbuf, hmax, rslots, MLP_SMEM_BUDGET);
+        return ORGYM_E_UNSUPPORTED;
+    }
+    *smem_out = smem;
+    return ORGYM_OK;
 }
 
 extern "C" int orgym_invmgmt_create(const orgym_invmgmt_config_t* cfg, int64_t num_envs, int device,
@@ -1187,6 +1517,10 @@ extern "C" int orgym_invmgmt_codegen(const orgym_invmgmt_config_t* cfg, const or
     // policy to bake in: the caller's, or the benchmark's default base-stock (levels (L+1) * p0, SF = 1)
     int policy = 0;
     double param[4] = {1.0, cfg->dist.p0, 0.0, 0.0};
+    if (in && in->policy == ORGYM_POLICY_MLP) {
+        orgym_set_error("the MLP policy runs the ahead-of-time kernel (inv_mlp_rollout_kernel); it is not specialised");
+        return ORGYM_E_UNSUPPORTED;
+    }
     if (in) {
         ORGYM_REQUIRE(in->policy == ORGYM_POLICY_BASE_STOCK || in->policy == ORGYM_POLICY_RANDOM,
                       "only the on-device base-stock and random policies are specialised");
@@ -1370,7 +1704,7 @@ extern "C" int orgym_invmgmt_rollout(orgym_handle_t h, uint64_t seed, int64_t en
     if (orgym_check_handle(h, FAM_INVMGMT)) return ORGYM_E_INVALID;
     InvHandle* H = (InvHandle*)h;
     ORGYM_REQUIRE(in && out, "null argument");
-    ORGYM_REQUIRE(in->policy >= 0 && in->policy <= 2, "unknown policy %d", in->policy);
+    ORGYM_REQUIRE(in->policy >= 0 && in->policy <= ORGYM_POLICY_MLP, "unknown policy %d", in->policy);
     ORGYM_REQUIRE(in->policy != ORGYM_POLICY_ACTIONS || in->actions_dev, "policy ACTIONS needs actions_dev");
     if (in->policy == ORGYM_POLICY_RANDOM)
         for (int i = 0; i < ((InvHandle*)h)->dev.n; i++)
@@ -1402,6 +1736,7 @@ extern "C" int orgym_invmgmt_rollout(orgym_handle_t h, uint64_t seed, int64_t en
     A.final_I = out->final_I_dev;
     A.final_B = out->final_B_dev;
     A.stats32 = out->stats32_dev;
+    A.action_traj = out->action_traj_dev;
     A.partials = out->summary_dev ? H->partials : nullptr;
     // int32 arithmetic only when every state value and per-episode sum is provably below 2^31: on-device policy
     // (requests within [0, c]), sampled demand (bounded support) and (T+1) * n * (c_max + I0_max + d_max) * 4 < 2^31;
@@ -1421,7 +1756,24 @@ extern "C" int orgym_invmgmt_rollout(orgym_handle_t h, uint64_t seed, int64_t en
     // fast path: kernels specialised for this configuration (register-resident rings, straight-line periods)
     H->last_rollout_jit = 0;
     const int jit_mode = inv_jit_mode();
-    if (jit_mode && !wide && inv_jit_policy_ok(in, A.target_is_int) && !A.reward_traj && !A.final_I && !A.final_B) {
+    if (in->policy == ORGYM_POLICY_MLP) {
+        InvMlpPlan M;
+        size_t smem = 0;
+        if (int rc = inv_mlp_plan(P, in->mlp, A.rslots, wide ? 8 : 4, &M, &smem)) return rc;
+        if (wide)
+            launch_mlp_rollout<long long>(H, A, M, smem, (cudaStream_t)stream);
+        else
+            launch_mlp_rollout<int>(H, A, M, smem, (cudaStream_t)stream);
+        ORGYM_CUDA(cudaGetLastError());
+        if (out->summary_dev) {
+            int rr = orgym_launch_reduce(H->partials, (int)((A.N + ROLL_THREADS - 1) / ROLL_THREADS), out->summary_dev,
+                                         (cudaStream_t)stream);
+            if (rr != ORGYM_OK) return rr;
+        }
+        return ORGYM_OK;
+    }
+    if (jit_mode && !wide && inv_jit_policy_ok(in, A.target_is_int) && !A.reward_traj && !A.final_I && !A.final_B &&
+        !A.action_traj) {
         cudaKernel_t fn = nullptr;
         const int jrc = inv_jit_get(H, in->policy == ORGYM_POLICY_BASE_STOCK ? 0 : 1, A.target_int, &fn);
         if (jrc != ORGYM_OK && jit_mode == 2) return jrc;  // strict: the reason is in orgym_last_error()

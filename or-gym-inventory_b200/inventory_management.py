@@ -11,6 +11,7 @@ from typing import Any, Dict, List, Optional
 import numpy as np
 
 from . import _capi
+from ._capi import MLP_RELU, MLP_TANH
 from .spaces import Box
 from .vector import BatchedEnv, _AUTORESET, _torch
 
@@ -129,7 +130,85 @@ class InvManagementParams:
         return cfg
 
 
-POLICY_ACTIONS, POLICY_BASE_STOCK, POLICY_RANDOM = 0, 1, 2
+POLICY_ACTIONS, POLICY_BASE_STOCK, POLICY_RANDOM, POLICY_MLP = 0, 1, 2, 3
+
+
+def mlp_layers(policy):
+    """The Linear layers and the activation of an actor network, in evaluation order: (linears, activation code).
+
+    Accepted: a `torch.nn.Sequential` of the form Linear, act, Linear, act, ..., Linear with one activation type (Tanh or
+    ReLU) throughout, or a stable-baselines3 `ActorCriticPolicy`-shaped object (duck-typed: `.mlp_extractor.policy_net`, a
+    Sequential ending in its activation, followed by `.action_net`, a Linear) without output squashing and with a flatten
+    features extractor -- SB3's deterministic `predict` for a Box action space.  Anything else raises ValueError naming
+    the offending layer or attribute."""
+    import torch.nn as nn
+    if isinstance(policy, nn.Sequential):
+        mods, where = list(policy), "Sequential"
+    elif hasattr(policy, "mlp_extractor") and hasattr(policy, "action_net"):
+        if getattr(policy, "squash_output", False):
+            raise ValueError("policy.squash_output is True: a tanh-squashed action is not the clipped Gaussian mean "
+                             "the device evaluates")
+        fe = getattr(policy, "features_extractor", None)
+        if fe is not None and not (isinstance(fe, nn.Flatten) or type(fe).__name__ == "FlattenExtractor"):
+            raise ValueError(f"policy.features_extractor is {type(fe).__name__}, only a flatten is supported")
+        pn = getattr(policy.mlp_extractor, "policy_net", None)
+        if not isinstance(pn, nn.Sequential):
+            raise ValueError("policy.mlp_extractor.policy_net is not a torch.nn.Sequential")
+        if not isinstance(policy.action_net, nn.Linear):
+            raise ValueError(f"policy.action_net is {type(policy.action_net).__name__}, not a Linear")
+        mods, where = list(pn) + [policy.action_net], "policy_net + action_net"
+    else:
+        raise ValueError(f"policy {type(policy).__name__!r} is neither a policy name, a torch.nn.Sequential nor an "
+                         "SB3 ActorCriticPolicy")
+    acts = {nn.Tanh: MLP_TANH, nn.ReLU: MLP_RELU}
+    linears, act = [], None
+    for i, mod in enumerate(mods):
+        want_linear = i % 2 == 0
+        if want_linear and not isinstance(mod, nn.Linear):
+            raise ValueError(f"{where}[{i}] is {type(mod).__name__}, expected Linear")
+        if not want_linear:
+            if type(mod) not in acts:
+                raise ValueError(f"{where}[{i}] is {type(mod).__name__}, expected Tanh or ReLU")
+            if act is not None and acts[type(mod)] != act:
+                raise ValueError(f"{where}[{i}] is {type(mod).__name__}: one activation type throughout")
+            act = acts[type(mod)]
+        if want_linear:
+            linears.append(mod)
+    if not mods or not isinstance(mods[-1], nn.Linear):
+        raise ValueError(f"{where} must end with a Linear (no activation after the last layer)")
+    if len(linears) > _capi.MLP_MAX_LAYERS:
+        raise ValueError(f"{where} has {len(linears)} Linear layers, at most {_capi.MLP_MAX_LAYERS} are supported")
+    for i in range(1, len(linears)):
+        if linears[i].in_features != linears[i - 1].out_features:
+            raise ValueError(f"{where}: Linear {i} has in_features {linears[i].in_features}, the layer before has "
+                             f"out_features {linears[i - 1].out_features}")
+    return linears, (act if act is not None else MLP_TANH)
+
+
+def pack_mlp(policy, obs_dim, act_dim, device):
+    """orgym_mlp_t for `policy` (see mlp_layers) with the current weights, plus the tensors it points into (keep them
+    alive until the rollout is enqueued).  Weights are detached, cast to float32, moved to `device` and made contiguous
+    with device-side torch ops: no host synchronisation, so a network being trained is evaluated as it is now."""
+    linears, act = mlp_layers(policy)
+    if linears[0].in_features != obs_dim:
+        raise ValueError(f"first Linear has in_features {linears[0].in_features}, the observation has {obs_dim}")
+    if linears[-1].out_features != act_dim:
+        raise ValueError(f"last Linear has out_features {linears[-1].out_features}, the action has {act_dim}")
+    import torch
+    m = _capi.Mlp()
+    m.num_layers, m.activation = len(linears), act
+    m.width[0] = obs_dim
+    keep = []
+    for l, lin in enumerate(linears):
+        m.width[l + 1] = lin.out_features
+        w = lin.weight.detach().to(device=device, dtype=torch.float32).contiguous()
+        keep.append(w)
+        m.weight[l] = w.data_ptr()
+        if lin.bias is not None:
+            b = lin.bias.detach().to(device=device, dtype=torch.float32).contiguous()
+            keep.append(b)
+            m.bias[l] = b.data_ptr()
+    return m, keep
 
 
 class InvManagementMasterEnv(BatchedEnv):
@@ -279,9 +358,16 @@ class InvManagementMasterEnv(BatchedEnv):
         base-stock with integer levels or random policy, sampled demand, no trajectory outputs)."""
         return bool(_capi.lib().orgym_invmgmt_is_specialised(self._h))
 
-    def _policy_struct(self, policy, safety_factor=1.0, mu=None):
+    def _policy_struct(self, policy, safety_factor=1.0, mu=None, keep=None):
         rin = _capi.InvRolloutIn()
-        if policy == "base_stock":
+        if not isinstance(policy, str):
+            P = self.params
+            mlp, tensors = pack_mlp(policy, P.pipeline_length, P.num_stages - 1, self.device)
+            if keep is not None:
+                keep += [mlp, tensors]
+            rin.policy = POLICY_MLP
+            rin.mlp = C.pointer(mlp)
+        elif policy == "base_stock":
             rin.policy = POLICY_BASE_STOCK
             rin.param[0] = float(safety_factor)
             rin.param[1] = float(self.params.dist_param.get("mu", 10) if mu is None else mu)
@@ -297,7 +383,8 @@ class InvManagementMasterEnv(BatchedEnv):
         """Build the rollout kernel specialised for this configuration and policy now (NVRTC, about a second; cached on
         disk) instead of inside the first rollout.  Raises OrgymError with the reason (NVRTC log included) when the
         configuration or policy is outside the specialiser's range or the compile fails."""
-        rin = self._policy_struct(policy, safety_factor, mu)
+        keep = []
+        rin = self._policy_struct(policy, safety_factor, mu, keep)
         _capi.check(_capi.lib().orgym_invmgmt_specialise(self._h, C.byref(rin)))
         return True
 
@@ -323,18 +410,23 @@ class InvManagementMasterEnv(BatchedEnv):
         """Fused reset + `periods` steps with state held on chip (K4).
 
         policy: 'base_stock' (benchmark_InvManagementBacklogEnv.py:142-198), 'random' (a_i ~ U{0..c_i}),
-                or 'actions' with `actions` int64 [N,T,m-1] ([T,N,m-1] if time_major).
+                'actions' with `actions` int64 [N,T,m-1] ([T,N,m-1] if time_major), or a trained actor network -- a
+                torch.nn.Sequential (Linear, Tanh|ReLU, ..., Linear) or an SB3 ActorCriticPolicy -- evaluated on the
+                device every period on the observation step() would return (float32, SB3's deterministic predict:
+                mean clipped to [0, c], then truncated like a float action; include/orgym_b200.h states the numerics).
+                Its weights are read at every call.
         demand: optional int64 [N,T] ([T,N] if time_major) replayed demand; default = on-device Philox sampling.
         Returns a dict of device tensors: ep_return f64[N], stats i64[N,4] (sum sales[0], sum demand,
         sum unfulfilled[0], sum_t sum_i max(0,I_i)), summary f64[8], and on request reward_traj f64[N,T],
-        final_I, final_B, stats32 (the statistics as int32).  The result tensors are owned by the env and reused by
+        final_I, final_B, stats32 (the statistics as int32), action_traj i64[N,T,m-1] (the requested orders, the
+        reference's action_log).  The result tensors are owned by the env and reused by
         the next rollout that uses the same `buffer_set`.
         """
         torch = _torch()
         P = self.params
         N, T, n, m = self.num_envs, int(P.num_periods), P.num_stages - 1, P.num_stages
-        rin = self._policy_struct(policy, safety_factor, mu)
         keep = []
+        rin = self._policy_struct(policy, safety_factor, mu, keep)
         if "_ring_scratch" not in self.__dict__:      # caller-owned scratch for very long lead-time rings (rare)
             nb = int(_capi.lib().orgym_invmgmt_rollout_scratch_bytes(self._h))
             self._ring_scratch = torch.empty(nb, dtype=torch.uint8, device=self.device) if nb > 0 else None
@@ -356,7 +448,8 @@ class InvManagementMasterEnv(BatchedEnv):
         dev = self.device
         shapes = dict(ep_return=((N,), torch.float64), stats=((N, 4), torch.int64),
                       reward_traj=((N, T), torch.float64), final_I=((N, n), torch.int64),
-                      final_B=((N, m), torch.int64), summary=((8,), torch.float64), stats32=((N, 4), torch.int32))
+                      final_B=((N, m), torch.int64), summary=((8,), torch.float64), stats32=((N, 4), torch.int32),
+                      action_traj=((N, T, n), torch.int64))
         cache = self.__dict__.setdefault("_rollout_buf", {}).setdefault(int(buffer_set), {})
         for name in want:
             shp, dt = shapes[name]
