@@ -377,277 +377,6 @@ __global__ void net_export_kernel(const __grid_constant__ NetDev P, int64_t N, c
     if (period) period[e] = st.period[el];
 }
 
-
-// ---- streaming STEP kernel for large graphs (network_management.py:436-635), table-driven ------------------------------------
-// A 64-node graph has ~650 float64 state values per instance: they cannot live in registers, and a launch of 2^17
-// instances is only 28 warps per SM -- ONE wave.  What bounds such a launch is therefore the latency chain of a single
-// warp, and the first version of this kernel (straight-line code generated per topology, netinv_jit.cu) spent it waiting
-// for its own instructions: 15 000 SASS instructions executed once per warp thrash the instruction cache (ncu: 7 of 18
-// stall cycles per issue `no_instruction`), at 128 registers and 16 resident warps.  This form walks the same passes as
-// loops over the flattened graph in the constant bank (uniform loads, a few hundred instructions in total), fits 7 CTAs
-// of 128 threads on an SM -- the whole batch resident at once -- and keeps the state in HBM:
-//   pass A  sorted reorder links: greedy allocation per supplier (:448-490), R_t / consumed parked in the scratch rows of
-//           the state tile (L2-resident until pass B reads them); the on-hand inventory of the NEXT supplier is loaded
-//           while the current segment is processed; the row-major action block moves through a 32-column tile that
-//           every warp transposes for its own 32 instances
-//   pass B  main nodes: arrivals, pipeline + ring commit, market sales in adjacency order fused with the node's profit
-//           terms (:494-613) -- same operations in the same order as the other kernels
-// The observation is assembled by net_obs_kernel below.
-#define NET_STREAM_THREADS 128
-#define NET_STREAM_PFD 6  // pass B prefetches the rows of the node this many iterations ahead into L2
-__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-// rows pass B reads for node j that pass A does not produce: pipeline inventory and arriving ring slot of its inbound
-// links, backlog of its market links
-__device__ __forceinline__ void net_stream_prefetch_node(const NetDev& P, const NetState& st, int j, int t, int el) {
-    for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
-        const int i = P.pred_idx[z], L = P.L[i];
-        prefetch_l2(st.Y + i * NET_TILE + el);
-        if (L > 0) prefetch_l2(st.ring + (size_t)(P.roff[i] + net_mod(t, L, P.Lmagic[i])) * NET_TILE + el);
-    }
-    for (int z = P.succ_ptr[j]; z < P.succ_ptr[j + 1]; z++) {
-        const int l = P.succ_idx[z];
-        if (l >= P.E) prefetch_l2(st.U + (l - P.E) * NET_TILE + el);
-    }
-}
-__global__ void __launch_bounds__(NET_STREAM_THREADS, 7) net_stream_step_kernel(const __grid_constant__ NetDev P,
-                                                                               const __grid_constant__ NetSimArgs A) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    float* tile = (float*)smem_raw;  // [threads][33] staging tile (+1 padding column: conflict-free)
-    constexpr int NTHR = NET_STREAM_THREADS, NP = NET_TILE;
-    const int tid = threadIdx.x, ln = tid & 31;
-    const int J = P.J, E = P.E, M = P.M;
-    const int64_t e0 = (int64_t)blockIdx.x * NTHR, e = e0 + tid;
-    const int nvalid = (int)((A.N - e0) < NTHR ? (A.N - e0) : NTHR);
-    const bool valid = tid < nvalid;
-    const int64_t ec = valid ? e : 0;
-    const int el = (int)(ec % NP);
-    NetState st((char*)A.state + (ec / NP) * net_tile_bytes(P), P);
-    double* const ring = st.ring;
-    double* const sc_R = (double*)(st.episode + NP);  // scratch rows of the tile: R_t [E], consumed [J]
-    double* const sc_C = sc_R + (size_t)E * NP;
-    float* const trow = tile + tid * 33;
-    const int wrow0 = tid & ~31, wrow1 = nvalid < wrow0 + 32 ? (nvalid > wrow0 ? nvalid : wrow0) : wrow0 + 32;
-    bool do_step = valid;
-    int t = 0;
-    uint32_t episode = 0;
-    uint64_t key = 0;
-    if (valid) {
-        t = st.period[el];
-        episode = st.episode[el];
-        key = st.key[el];
-        if (t >= P.T) {  // episode already over
-            do_step = false;
-            if (A.autoreset == ORGYM_AUTORESET_NEXT_STEP) {
-                for (int j = 0; j < J; j++) st.X[j * NP + el] = P.I0[j];
-                for (int i = 0; i < E; i++) st.Y[i * NP + el] = 0.0;
-                for (int r = 0; r < M; r++) st.U[r * NP + el] = 0.0;
-                for (int k = 0; k < P.sumL; k++) ring[k * NP + el] = 0.0;
-                if (st.ring32)
-                    for (int k = 0; k < P.sumL; k++) st.ring32[k * NP + el] = 0.0f;
-                st.period[el] = 0;
-                st.episode[el] = episode + 1;
-                A.reward[e] = 0.0; A.terminated[e] = 0; A.truncated[e] = 0;
-            } else {
-                atomicOr(A.err, ORGYM_ERR_STEP_PAST_END);
-                A.reward[e] = 0.0; A.terminated[e] = 0; A.truncated[e] = 1;
-            }
-        }
-    }
-    // The launch is one wave (28 warps per SM for 2^17 instances): its duration is the latency chain of a single warp.
-    // Everything the passes will read is therefore prefetched into L2 ahead of its use -- the on-hand inventory rows and
-    // this lane's action row now, the per-node rows NET_STREAM_PFD nodes ahead inside pass B -- so that the dependent
-    // loads of the loops below are L2 hits; a prefetch costs an instruction but no register and no scoreboard slot.
-    if (do_step) {
-        for (int j = 0; j < J; j++) prefetch_l2(st.X + j * NP + el);
-        const char* arow = (const char*)(A.actions + e * A.a_se);
-        for (int b = 0; b < E * 4; b += 128) prefetch_l2(arow + b);
-        for (int j = 0; j < NET_STREAM_PFD && j < J; j++) net_stream_prefetch_node(P, st, j, t, el);
-    }
-    // ---- pass A: orders (:448-490)
-    {
-        double cons = 0.0, xs = 0.0, xs_next = 0.0;
-        int s_next = -1;
-        if (do_step)
-            for (int k = 0; k < E; k++)
-                if (P.sup[k] >= 0) {  // first supplier: load ahead of the action staging
-                    s_next = P.sup[k];
-                    xs_next = st.X[s_next * NP + el];
-                    break;
-                }
-        for (int c0 = 0; c0 < E; c0 += 32) {
-            const int c1 = c0 + 32 < E ? c0 + 32 : E;
-            __syncwarp();
-            for (int r = wrow0; r < wrow1; r++)
-                if (c0 + ln < E) tile[r * 33 + ln] = A.actions[(e0 + r) * A.a_se + c0 + ln];
-            __syncwarp();
-            if (do_step) {
-                for (int i = c0; i < c1; i++) {
-                    const int s = P.sup[i];
-                    double req = rint((double)trow[i - c0]);  // Python round(): half to even
-                    req = req > 0.0 ? req : 0.0;
-                    double f = 0.0;
-                    if (s == -1)
-                        f = req;  // raw material: unlimited (:453-455)
-                    else if (s >= 0) {
-                        if (i == 0 || P.sup[i - 1] != s) {  // segment start: take the pre-loaded X, pre-load the next one
-                            cons = 0.0;
-                            xs = s == s_next ? xs_next : st.X[s * NP + el];
-                            int k = i + 1;
-                            while (k < E && (P.sup[k] == s || P.sup[k] < 0)) k++;
-                            if (k < E) {
-                                s_next = P.sup[k];
-                                xs_next = st.X[s_next * NP + el];
-                            }
-                        }
-                        double avail = xs - cons;  // :459
-                        avail = avail > 0.0 ? avail : 0.0;
-                        double oa = avail;
-                        const double vs = P.v[s];
-                        if (P.is_factory[s]) {  // :464-478
-                            const double mp = vs * avail;
-                            const double lim = mp < P.C[s] ? mp : P.C[s];
-                            oa = lim < oa ? lim : oa;
-                        }
-                        f = oa < req ? oa : req;           // :481
-                        cons += vs == 1.0 ? f : f / vs;    // :484-485 (x / 1.0 == x)
-                        if (i == E - 1 || P.sup[i + 1] != s) sc_C[s * NP + el] = cons;
-                    }
-                    sc_R[i * NP + el] = f;  // R[t] = S[t] = f (:488-490)
-                    if (A.info_sales) A.info_sales[NET_IIDX(A, e, E + M, i)] = f;
-                }
-            }
-        }
-    }
-    // ---- pass B: nodes
-    if (do_step) {
-        double total = 0.0;
-        for (int j = 0; j < J; j++) {
-            if (j + NET_STREAM_PFD < J) net_stream_prefetch_node(P, st, j + NET_STREAM_PFD, t, el);
-            double x = st.X[j * NP + el];
-            const double c = P.has_seg[j] ? sc_C[j * NP + el] : 0.0;
-            double arr = 0.0, PC = 0.0, HCp = 0.0;
-            // arrivals (:516-528), pipeline (:494-511), ring commit -- two inbound links per trip, all six loads first
-            for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z += 2) {
-                const bool two = z + 1 < P.pred_ptr[j + 1];
-                const int i0 = P.pred_idx[z], i1 = two ? P.pred_idx[z + 1] : i0;
-                const int L0 = P.L[i0], L1 = P.L[i1];
-                double* const slot0 = ring + (size_t)(P.roff[i0] + net_mod(t, L0, P.Lmagic[i0])) * NP + el;
-                double* const slot1 = ring + (size_t)(P.roff[i1] + net_mod(t, L1, P.Lmagic[i1])) * NP + el;
-                const double rt0 = sc_R[i0 * NP + el], y0 = st.Y[i0 * NP + el];
-                const double rt1 = sc_R[i1 * NP + el], y1 = st.Y[i1 * NP + el];
-                double ar0 = rt0, ar1 = rt1;
-                if (L0 > 0) ar0 = *slot0;
-                if (L1 > 0 && two) ar1 = *slot1;
-                {
-                    if (L0 > 0) {
-                        *slot0 = rt0;
-                        if (st.ring32) st.ring32[slot0 - ring] = (float)rt0;
-                    }
-                    arr += ar0;
-                    const double yn = (y0 - ar0) + rt0;
-                    st.Y[i0 * NP + el] = yn;
-                    PC += P.p[i0] * rt0;                    // :586
-                    HCp += P.g[i0] * (yn > 0.0 ? yn : 0.0);  // :591
-                }
-                if (two) {
-                    if (L1 > 0) {
-                        *slot1 = rt1;
-                        if (st.ring32) st.ring32[slot1 - ring] = (float)rt1;
-                    }
-                    arr += ar1;
-                    const double yn = (y1 - ar1) + rt1;
-                    st.Y[i1 * NP + el] = yn;
-                    PC += P.p[i1] * rt1;
-                    HCp += P.g[i1] * (yn > 0.0 ? yn : 0.0);
-                }
-            }
-            x = (x + arr) - c;
-            double SR = 0.0, sold = 0.0, UP = 0.0;
-            // successors in adjacency order = Python sum order (:582); four per trip, their loads first
-            for (int z0 = P.succ_ptr[j]; z0 < P.succ_ptr[j + 1]; z0 += 4) {
-                int l[4];
-                double q[4];
-#pragma unroll
-                for (int k = 0; k < 4; k++) {
-                    l[k] = z0 + k < P.succ_ptr[j + 1] ? P.succ_idx[z0 + k] : -1;
-                    q[k] = 0.0;
-                    if (l[k] >= 0) q[k] = l[k] < E ? sc_R[l[k] * NP + el] : st.U[(l[k] - E) * NP + el];
-                }
-#pragma unroll
-                for (int k = 0; k < 4; k++) {
-                    if (l[k] < 0) continue;
-                    if (l[k] < E) {
-                        SR += P.p[l[k]] * q[k];
-                        sold += q[k];
-                    } else {  // market link (:536-566): a node's market links come in the same relative order in both lists
-                        const int r = l[k] - E;
-                        double d;
-                        if (A.demand)
-                            d = rint(A.demand[e * A.d_se + r]);
-                        else
-                            d = (double)sample_fixed(P.dem[r], P.dem[r].table, key, episode, t, (uint32_t)r);
-                        d = d > 0.0 ? d : 0.0;
-                        const double fill = d + q[k];  // U[r]: one market link feeds one retailer, nothing else wrote it
-                        const double invr = x > 0.0 ? x : 0.0;
-                        const double sl = invr < fill ? invr : fill;
-                        x = x - sl;
-                        const double un = fill - sl;
-                        const double u = P.backlog ? un : 0.0;
-                        st.U[r * NP + el] = u;
-                        if (A.info_demand) A.info_demand[NET_IIDX(A, e, M, r)] = d;
-                        if (A.info_sales) A.info_sales[NET_IIDX(A, e, E + M, E + r)] = sl;
-                        if (P.is_retail[j]) UP += P.rt_b[r] * u;  // :608
-                        SR += P.rt_p[r] * sl;
-                        sold += sl;
-                    }
-                }
-            }
-            st.X[j * NP + el] = x;
-            const double xp = x > 0.0 ? x : 0.0;
-            const double HC = P.h[j] * xp + HCp;  // :590-593
-            double OC = 0.0;
-            if (P.is_factory[j]) {  // :597-601
-                const double vj = P.v[j];
-                OC = vj > 0.0 ? P.o[j] * (vj == 1.0 ? sold : sold / vj) : 0.0;
-            }
-            const double pj = (((SR - PC) - OC) - HC) - UP;  // :611
-            total += pj;
-            if (A.info_profit) A.info_profit[NET_IIDX(A, e, J, j)] = pj;
-        }
-        for (int i = 0; i < E; i++) {  // reorder links whose purchaser holds no inventory: pipeline bookkeeping only
-            if (P.pur[i] >= 0) continue;
-            const int L = P.L[i];
-            const double rt = sc_R[i * NP + el];
-            double ar = rt;
-            if (L > 0) {
-                double* slot = ring + (size_t)(P.roff[i] + net_mod(t, L, P.Lmagic[i])) * NP + el;
-                ar = *slot;
-                *slot = rt;
-                if (st.ring32) st.ring32[slot - ring] = (float)rt;
-            }
-            st.Y[i * NP + el] = (st.Y[i * NP + el] - ar) + rt;
-        }
-        const int tn = t + 1;
-        const bool trunc = tn >= P.T;  // :624
-        if (A.info_profit_total) A.info_profit_total[e] = total;
-        A.reward[e] = P.disc[t] * total;  // :619
-        A.terminated[e] = 0;
-        A.truncated[e] = trunc ? 1 : 0;
-        if (trunc && A.autoreset == ORGYM_AUTORESET_SAME_STEP) {
-            if (A.final_obs) net_write_obs<NET_TILE>(P, st.U, st.X, el, ring, el, tn, A.final_obs + e * P.obs_dim);
-            for (int j = 0; j < J; j++) st.X[j * NP + el] = P.I0[j];
-            for (int i = 0; i < E; i++) st.Y[i * NP + el] = 0.0;
-            for (int r = 0; r < M; r++) st.U[r * NP + el] = 0.0;
-            for (int k = 0; k < P.sumL; k++) ring[k * NP + el] = 0.0;
-                if (st.ring32)
-                    for (int k = 0; k < P.sumL; k++) st.ring32[k * NP + el] = 0.0f;
-            st.period[el] = 0;
-            st.episode[el] = episode + 1;
-        } else
-            st.period[el] = tn;
-    }
-}
-
 // ---- observation assembly for large graphs (network_management.py:334-413) --------------------------------------------------
 // The streaming STEP path for large graphs leaves the new state in HBM; this kernel turns it into row-major float32
 // observation rows.  One CTA owns NET_OBS_ROWS = 32 instances (a quarter of a 128-instance state tile).  A state tile is
@@ -666,16 +395,14 @@ __global__ void __launch_bounds__(NET_STREAM_THREADS, 7) net_stream_step_kernel(
 // Which slot feeds which column depends on the period only through t mod L_i of every link (ring rotation); a group of
 // instances that are not all in the same period (possible only after masked resets) takes the per-instance fallback.
 #define NET_OBS_ROWS 32    // instances per CTA
-#ifndef NET_OBS_THREADS
 #define NET_OBS_THREADS 384
-#endif
 #define NET_OBS_BATCH 12   // independent column loads in flight per thread
-#ifndef NET_OBS_BATCH32
 #define NET_OBS_BATCH32 22  // ... for the float32 ring columns (one register each)
-#endif
-size_t net_obs_smem(const NetDev& P) {
+static size_t net_obs_smem(const NetDev& P) {
     return 128 + (((size_t)P.obs_dim * 2 + 127) & ~(size_t)127) + (((size_t)NET_OBS_ROWS * P.obs_dim * 4 + 127) & ~(size_t)127);
 }
+int net_obs_kernel_fits(const NetDev& P) { return net_jit_uses_stream(P) && net_obs_smem(P) <= 200 * 1024; }
+__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 
 __global__ void __launch_bounds__(NET_OBS_THREADS) net_obs_kernel(const __grid_constant__ NetDev P, int64_t N,
                                                                   const void* __restrict__ state, float* __restrict__ obs) {
@@ -702,8 +429,9 @@ __global__ void __launch_bounds__(NET_OBS_THREADS) net_obs_kernel(const __grid_c
             net_write_obs<NET_TILE>(P, st.U, st.X, el0 + tid, st.ring, el0 + tid, st.period[el0 + tid], obs + (e0 + tid) * W);
         return;
     }
-    // rows of the tile, in units of 1 KB: [0] keys, [1, J] X, then Y (E), U (M), ring (sumL)
-    const int rowX = 1, rowU = 1 + P.J + P.E, rowR = rowU + P.M;
+    // float64 columns: rows of the tile, in units of 1 KB: [0] keys, [1, J] X, then Y (E), U (M); window columns: slots
+    // of the float32 ring copy (512-byte rows of st.ring32), 4 instead of 8 bytes read per column and instance
+    const int rowX = 1, rowU = 1 + P.J + P.E;
     for (int c = tid; c < P.M; c += NET_OBS_THREADS) colrow[c] = (uint16_t)(rowU + c);
     for (int c = tid; c < P.J; c += NET_OBS_THREADS) colrow[P.M + c] = (uint16_t)(rowX + c);
     for (int i = tid; i < P.E; i += NET_OBS_THREADS) {
@@ -712,16 +440,14 @@ __global__ void __launch_bounds__(NET_OBS_THREADS) net_obs_kernel(const __grid_c
         int sl = net_mod(t0, L, P.Lmagic[i]);  // window element q (oldest first) lives in ring slot (t + q) % L
         uint16_t* dst = colrow + P.M + P.J + P.roff[i];
         for (int q = 0; q < L; q++) {
-            dst[q] = (uint16_t)((P.ring32 ? 0 : rowR) + P.roff[i] + sl);
+            dst[q] = (uint16_t)(P.roff[i] + sl);
             sl = sl + 1 == L ? 0 : sl + 1;
         }
     }
     __syncthreads();
     const double* src = (const double*)tile + el0 + lane;  // + row * 128
     float* orow = out + (size_t)lane * W;
-    // The window columns come from the float32 copy of the rings when the tile carries one (colrow then holds the ring
-    // slot, a 512-byte row of st.ring32): 4 instead of 8 bytes read per column and instance.
-    const int WD = st.ring32 ? P.M + P.J : W;  // columns [0, WD) are float64 rows, [WD, W) float32 rows
+    const int WD = P.M + P.J;  // columns [0, WD) are float64 rows, [WD, W) float32 rows
     const float* src32 = st.ring32 + el0 + lane;
     // all of this warp's columns are requested into L2 at once (one instruction each, no register, no scoreboard slot):
     // the batched loads below then wait for L2, not for HBM, and the CTA's share is in flight from the first cycle
@@ -767,11 +493,6 @@ __global__ void __launch_bounds__(NET_OBS_THREADS) net_obs_kernel(const __grid_c
         const int total = nvalid * W;
         for (int i = tid; i < total; i += NET_OBS_THREADS) g[i] = out[i];
     }
-}
-
-static int net_wants_ring32(const NetDev& P) {
-    const char* rv = getenv("ORGYM_NET_RING32");
-    return net_jit_uses_stream(P) && net_obs_smem(P) <= 200 * 1024 && !(rv && rv[0] == '0') ? 1 : 0;
 }
 
 static int net_obs_launch(const NetHandle* H, const void* state, float* obs, cudaStream_t s) {
@@ -938,10 +659,8 @@ extern "C" int orgym_netinv_create(const orgym_netinv_config_t* c, int64_t num_e
             cudaFuncSetAttribute(net_sim_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(220 * 1024));
             cudaFuncSetAttribute(net_sim_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(220 * 1024));
             cudaFuncSetAttribute(net_obs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(220 * 1024));
-            H->stream_aot = 0;
             // large graphs whose observation is assembled by net_obs_kernel keep a float32 copy of the rings in the tile
-            // (ORGYM_NET_RING32=0: off, for comparison)
-            P.ring32 = net_wants_ring32(P);
+            P.ring32 = net_obs_kernel_fits(P);
             // kernel specialised for this topology (NVRTC); any failure falls back to the generic kernel above
             H->jit_threads = 0;
             H->dem_dev = nullptr;
@@ -949,14 +668,6 @@ extern "C" int orgym_netinv_create(const orgym_netinv_config_t* c, int64_t num_e
             // 10-15 s, once: cubins are cached on disk); ORGYM_NET_JIT=0 never, =1 always, =2 always and fail loudly
             const char* jv = getenv("ORGYM_NET_JIT");
             const bool want_jit = jv ? jv[0] != '0' : (P.E <= 128);
-            // large graphs: ORGYM_NET_STREAM_AOT=1 steps through the table-driven streaming kernel (no NVRTC needed for
-            // STEP; measured 0.44 ms on the 64-node graph against 0.29 ms for the generated kernel of netinv_jit.cu, which
-            // therefore stays the default); ORGYM_NET_JIT=0 selects the generic kernel
-            {
-                const char* av = getenv("ORGYM_NET_STREAM_AOT");
-                H->stream_aot = net_jit_uses_stream(P) && (av && av[0] == '1') && !(jv && jv[0] == '0') &&
-                                net_obs_smem(P) <= 200 * 1024;
-            }
             if (want_jit) {
                 std::string jerr;
                 if (net_jit_build(H, &jerr) != 0) {
@@ -1056,12 +767,6 @@ extern "C" int orgym_netinv_step(orgym_handle_t h, void* state_dev, const float*
         A.final_obs = info->final_obs_dev;
     }
     A.err = H->base.err_dev;
-    if (H->stream_aot) {  // large graphs: table-driven streaming kernel + observation kernel
-        const unsigned grid = (unsigned)((A.N + NET_STREAM_THREADS - 1) / NET_STREAM_THREADS);
-        net_stream_step_kernel<<<grid, NET_STREAM_THREADS, NET_STREAM_THREADS * 33 * 4, (cudaStream_t)stream>>>(H->dev, A);
-        ORGYM_CUDA(cudaGetLastError());
-        return net_obs_launch(H, state_dev, obs_dev, (cudaStream_t)stream);
-    }
     if (H->jit.fn) {
         int jrc = net_jit_launch(H, A, (cudaStream_t)stream);
         if (jrc != ORGYM_OK) return jrc;
@@ -1146,7 +851,7 @@ extern "C" int orgym_netinv_codegen(const orgym_netinv_config_t* cfg, int compil
         delete P;
         return rc;
     }
-    P->ring32 = net_wants_ring32(*P);
+    P->ring32 = net_obs_kernel_fits(*P);
     std::string src = net_jit_source(*P, 128);
     delete P;
     if (needed) *needed = (int64_t)src.size();

@@ -38,7 +38,6 @@ struct NetHandle {
     cudaKernel_t jit_rollout;  // ROLLOUT kernel of the same module
     int jit_threads;
     int jit_stream;            // STEP kernel is the streaming variant (large graphs)
-    int stream_aot;            // large graphs: STEP runs the table-driven ahead-of-time streaming kernel (netinv.cu)
     int jit_obs_split;         // streaming variant without its observation pass: net_obs_kernel (TMA-staged) follows it
     int jit_onepass;           // streaming variant in its single-pass form (no scratch rows, no action tile)
     AliasDev* dem_dev;  // device copy of dev.dem[] for the specialised kernel
@@ -51,9 +50,7 @@ struct NetHandle {
 // between slots is a compile-time constant (every access of the specialised kernels becomes base + immediate, no
 // 64-bit index arithmetic) and the ~1700 slots of a 64-node graph that one CTA touches per period lie in one
 // contiguous 1.7 MB region instead of being spread over as many distinct 1 MB-apart rows (TLB reach, DRAM pages).
-#ifndef NET_TILE
 #define NET_TILE 128
-#endif
 struct NetState {
     uint64_t* key;
     double *X, *Y, *U, *ring;
@@ -95,6 +92,8 @@ int net_jit_build(NetHandle* H, std::string* err);
 int net_jit_launch(const NetHandle* H, const struct NetSimArgs& A, cudaStream_t s);
 std::string net_jit_source(const NetDev& P, int nthr);
 int net_jit_uses_stream(const NetDev& P);
-size_t net_obs_smem(const NetDev& P);    // netinv.cu: shared memory of the TMA-staged observation kernel
-int net_jit_onepass(const NetDev& P);    // ORGYM_NET_JIT_ONEPASS (default 1) and suppliers follow their purchasers in node order
-int net_jit_obs_split(const NetDev& P);  // ORGYM_NET_OBS_TMA (default 1) and the observation rows fit in shared memory
+// netinv.cu: the streaming STEP form is used and 32 observation rows fit net_obs_kernel's shared memory.  Such handles
+// keep the float32 ring copy (NetDev::ring32) that net_obs_kernel reads.
+int net_obs_kernel_fits(const NetDev& P);
+int net_jit_onepass(const NetDev& P);    // suppliers follow their purchasers in node order (test hook: ORGYM_NET_JIT_ONEPASS=0)
+int net_jit_obs_split(const NetDev& P);  // net_obs_kernel_fits (test hook: ORGYM_NET_OBS_TMA=0 keeps the fused observation pass)

@@ -36,29 +36,32 @@ std::string lit(double v) {
 void emit_step_stream(Src& o, const NetDev& P, int min_blocks);
 }  // namespace
 
+// graph size selects the streaming STEP form; ORGYM_NET_JIT_STREAM=1 / 0 forces it on / off, so that small graphs can
+// test it
 int net_jit_uses_stream(const NetDev& P) {
     int stream = 2 * P.J + 3 * P.E + 2 * P.M > 128 ? 1 : 0;
     if (const char* sv = getenv("ORGYM_NET_JIT_STREAM")) stream = atoi(sv) ? 1 : 0;
     return stream;
 }
 
-// streaming STEP kernel, observation pass: geometry of the asynchronous staging (cp.async)
 static int env_int(const char* name, int dflt, int lo, int hi) {
     const char* v = getenv(name);
     if (!v) return dflt;
     const int x = atoi(v);
     return x < lo || x > hi ? dflt : x;
 }
-// 1 (default): the streaming STEP kernel stops after the state update and netinv.cu's TMA-staged net_obs_kernel writes
-// the observation; 0: the kernel's own observation pass (round-1 form, kept for comparison)
+// The streaming STEP kernel stops after the state update and netinv.cu's TMA-staged net_obs_kernel writes the
+// observation, unless the observation rows are too wide for that kernel: then the kernel's own pass C writes it
+// (ORGYM_NET_OBS_TMA=0 forces pass C, so that small graphs can test it).
 int net_jit_obs_split(const NetDev& P) {
-    return env_int("ORGYM_NET_OBS_TMA", 1, 0, 1) && net_obs_smem(P) <= 200 * 1024;
+    return env_int("ORGYM_NET_OBS_TMA", 1, 0, 1) && net_obs_kernel_fits(P);
 }
 // Single-pass form of the streaming STEP kernel (see emit_step_stream): usable when every inventory-holding supplier comes
 // after its purchasers in main-node order (true of the reference's graphs, which number nodes market -> raw material),
-// so that a purchaser still finds its suppliers' start-of-period inventory in the state tile.
+// so that a purchaser still finds its suppliers' start-of-period inventory in the state tile.  ORGYM_NET_JIT_ONEPASS=0
+// forces the two-pass form, so that graphs in the reference's numbering can test it.
 int net_jit_onepass(const NetDev& P) {
-    if (!env_int("ORGYM_NET_JIT_ONEPASS", 1, 0, 1) || env_int("ORGYM_NET_JIT_LDGSTS", 0, 0, 1)) return 0;
+    if (!env_int("ORGYM_NET_JIT_ONEPASS", 1, 0, 1)) return 0;
     for (int j = 0; j < P.J; j++)
         for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
             const int s = P.sup[P.pred_idx[z]];
@@ -69,20 +72,6 @@ int net_jit_onepass(const NetDev& P) {
             if (P.sup[i] >= 0 && P.sup[k] == P.sup[i] && P.sup[i + 1] != P.sup[i]) return 0;
     return 1;
 }
-// measured on the 64-node graph: the register-staged pass (0) beats the cp.async one (1) by 6 % -- kept as a knob
-static int stream_async() { return env_int("ORGYM_NET_JIT_ASYNC", 0, 0, 1); }
-static int stream_cw() {
-    const int c = env_int("ORGYM_NET_JIT_CW", 16, 8, 32);
-    return c >= 32 ? 32 : (c >= 16 ? 16 : 8);
-}
-static int stream_nst() { return env_int("ORGYM_NET_JIT_NST", 3, 2, 6); }
-size_t net_jit_stream_smem(int nthr) {
-    const size_t act = (size_t)nthr * 33 * 4;
-    if (!stream_async()) return act;
-    const size_t st = (size_t)stream_nst() * nthr * (stream_cw() + 1) * 8;
-    return st > act ? st : act;
-}
-
 std::string net_jit_source(const NetDev& P, int nthr) {
     const int J = P.J, E = P.E, M = P.M;
     Src o;
@@ -343,25 +332,15 @@ std::string net_jit_source(const NetDev& P, int nthr) {
     // small graphs: STEP 5 CTAs/SM (<= 102 registers), ROLLOUT 3; large graphs (hundreds of live float64 values per
     // instance) spill either way and run best with all 255 registers (measured on the 64-node synthetic graph)
     const bool big = 2 * J + 3 * E + 2 * M > 128;
-    int mb_step = big ? 2 : 5, mb_roll = big ? 1 : 3;
-    if (const char* mb = getenv("ORGYM_NET_JIT_MINBLOCKS_STEP")) mb_step = atoi(mb) > 0 ? atoi(mb) : 1;
-    if (const char* mb = getenv("ORGYM_NET_JIT_MINBLOCKS_ROLLOUT")) mb_roll = atoi(mb) > 0 ? atoi(mb) : 1;
     const int stream = net_jit_uses_stream(P);  // large graphs: state stays in HBM, coalesced 32-column tiles
-    const char* aotv = getenv("ORGYM_NET_STREAM_AOT");
-    if (stream && (aotv && aotv[0] == '1') && net_obs_smem(P) <= 200 * 1024) {
-        // STEP runs netinv.cu's ahead-of-time streaming kernel: only the fused rollout is generated for this topology
-        o("extern \"C\" __global__ void net_jit_step(const NetSimArgs A, const double* __restrict__ disc, const AliasDev* __restrict__ dem) {}");
-    } else if (stream) {
-        // 64 registers per thread: a launch of 2^17 instances is 28 warps per SM, so with 8 CTAs per SM the whole batch
-        // is resident in one wave (measured on the 64-node graph: 0.470 vs 0.486 ms for the step pair at 128 registers;
-        // (256, 4) and (64, 16) are equivalent)
-        int mb = nthr >= 512 ? 2 : (nthr >= 256 ? 4 : 8);
-        if (const char* mbv = getenv("ORGYM_NET_JIT_MINBLOCKS_STEP")) mb = atoi(mbv) > 0 ? atoi(mbv) : mb;
-        emit_step_stream(o, P, mb);
-    }
+    if (stream)
+        // 64 registers per thread: a launch of 2^17 instances is 28 warps per SM, so with 8 CTAs of 128 threads per SM the
+        // whole batch is resident in one wave (measured on the 64-node graph: 0.470 vs 0.486 ms for the step pair at 128
+        // registers)
+        emit_step_stream(o, P, 8);
     else
-        emit_kernel("net_jit_step", 0, mb_step);
-    emit_kernel("net_jit_rollout", 1, mb_roll);
+        emit_kernel("net_jit_step", 0, big ? 2 : 5);
+    emit_kernel("net_jit_rollout", 1, big ? 1 : 3);
     o("// step_kernel_kind=%s", stream ? "stream" : "register");
     return o.s;
 }
@@ -424,33 +403,6 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
     o("      }");
     o("    }");
     o("  }");
-    // Software prefetch into L2 (ORGYM_NET_JIT_PREFETCH: 0 = off, 1 = every row this instance will read, issued before
-    // pass A, d >= 2 = the rows of node group g + d - 1 issued before group g): the kernel is bound by the latency of
-    // dependent global loads at 16 warps per SM; a prefetch costs one instruction and no register or scoreboard slot.
-    const int PF = env_int("ORGYM_NET_JIT_PREFETCH", 0, 0, 8);  // measured: no gain (0.435 / 0.428 vs 0.419 ms), off by default
-    // nodes per load group in pass B: with the 64-register budget below, one node per group measured fastest on the
-    // 64-node graph (0.419 ms for the step pair; 2: 0.433, 3: 0.449, 4: 0.470) -- fewer live values, fewer spills
-    int GROUP = 1;
-    if (const char* gv = getenv("ORGYM_NET_JIT_GROUP")) GROUP = atoi(gv) > 0 ? atoi(gv) : 1;
-    auto emit_prefetch_node = [&](int j, const char* ind) {  // rows pass B reads for node j that pass A does not produce
-        for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
-            const int i = P.pred_idx[z], L = P.L[i];
-            o("%sPF_L2(s_Y + %d * NP + el);", ind, i);
-            if (L > 0) o("%sPF_L2(ring + (%d + t %% %d) * NP + el);", ind, P.roff[i], L);
-        }
-        for (int r = 0; r < M; r++)
-            if (P.rt_node[r] == j) o("%sPF_L2(s_U + %d * NP + el);", ind, r);
-    };
-    if (PF) {
-        o("#define PF_L2(p) asm volatile(\"prefetch.global.L2 [%%0];\" ::\"l\"(p))");
-        o("  if (do_step) {");
-        for (int j = 0; j < J; j++) o("    PF_L2(s_X + %d * NP + el);", j);
-        if (PF == 1)
-            for (int j = 0; j < J; j++) emit_prefetch_node(j, "    ");
-        else
-            for (int j = 0; j < std::min(J, GROUP * (PF - 1)); j++) emit_prefetch_node(j, "    ");
-        o("  }");
-    }
     const int ONEPASS = net_jit_onepass(P);
     o("  // stream_form=%s", ONEPASS ? "onepass" : "twopass");
     std::vector<int> link_done(E, 0);
@@ -580,34 +532,21 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
                 o("      s_Y[%d * NP + el] = (s_Y[%d * NP + el] - ar) + rt%d; }", i, i, i);
             }
         }
-        // ORGYM_NET_JIT_AHEAD = d (default 0, measured no gain): the loads of node j + d are written BEFORE the arithmetic of
-        // node j.  Each node ends in stores and (uniform) branches around the optional info outputs, basic-block boundaries
-        // the compiler does not hoist loads across, so a warp pays one memory round trip per node; but at the 64 registers
-        // that keep the whole batch resident the looked-ahead values are spilled as they arrive, which waits for them all
-        // the same (0.417 / 0.417 / 0.443 ms for d = 0 / 1 / 2).  What did help is ORGYM_NET_JIT_SYNC below.
-        const int AHEAD = env_int("ORGYM_NET_JIT_AHEAD", 0, 0, 4);
-        const int SYNC1 = env_int("ORGYM_NET_JIT_SYNC", 4, 0, 64);  // measured: 0.417 ms without, 0.389-0.393 with (any cadence 1..8)
-        auto emit_loads_outer = [&](int j) {
-            const NodeLd& n = nld[(size_t)j];
-            for (const auto& d : n.d8) o("    const double p_%s = *(%s);", d.first.c_str(), d.second.c_str());
-            for (int l : n.acts) o("    const float pa%d_%d = __ldg(arow + %d);", j, l, l);
-        };
-        for (int j = 0; j < std::min(J, AHEAD); j++) emit_loads_outer(j);
+        // Each node ends in stores and (uniform) branches around the optional info outputs, basic-block boundaries the
+        // compiler does not hoist loads across, so a warp pays one memory round trip per node.  Writing the loads of node
+        // j + 1 or j + 2 before the arithmetic of node j does not shorten that: at the 64 registers that keep the whole
+        // batch resident the looked-ahead values are spilled as they arrive (0.417 / 0.417 / 0.443 ms for a look-ahead of
+        // 0 / 1 / 2 nodes).
         for (int j = 0; j < J; j++) {
-            if (AHEAD > 0 && j + AHEAD < J) emit_loads_outer(j + AHEAD);
             o("    {");
             const NodeLd& n = nld[(size_t)j];
             for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
                 const int i = P.pred_idx[z], L = P.L[i];
                 if (L > 0) o("      double* const slot%d = ring + (%d + t %% %d) * NP + el;", i, P.roff[i], L);
             }
-            if (AHEAD > 0) {
-                for (const auto& d : n.d8) o("      const double %s = p_%s;", d.first.c_str(), d.first.c_str());
-                for (int l : n.acts) o("      const double rq%d = net_reqf(pa%d_%d);", l, j, l);
-            } else {  // loads first (all independent)
-                for (const auto& d : n.d8) o("      const double %s = *(%s);", d.first.c_str(), d.second.c_str());
-                for (int l : n.acts) o("      const double rq%d = REQ(%d);", l, l);
-            }
+            // loads first (all independent)
+            for (const auto& d : n.d8) o("      const double %s = *(%s);", d.first.c_str(), d.second.c_str());
+            for (int l : n.acts) o("      const double rq%d = REQ(%d);", l, l);
             // R_t of the inbound links, own allocation chain
             for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
                 const int i = P.pred_idx[z];
@@ -674,9 +613,10 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
             o("        (void)sold; const double pj = (((SR - PC) - OC) - HC) - UP; total += pj;");
             o("        if (A.info_profit) A.info_profit[NET_IIDX(A, e, NJ, %d)] = pj; }", j);
             o("    }");
-            // ORGYM_NET_JIT_SYNC=k: a CTA-wide barrier after every k-th node keeps the warps of a CTA within the same stretch of
-            // this long straight-line kernel, so an instruction line is fetched once per CTA rather than once per warp
-            if (SYNC1 > 0 && AHEAD == 0 && (j + 1) % SYNC1 == 0 && j + 1 < J) {
+            // a CTA-wide barrier after every 4th node keeps the warps of a CTA within the same stretch of this long
+            // straight-line kernel, so an instruction line is fetched once per CTA rather than once per warp (measured:
+            // 0.417 ms without, 0.389-0.393 with, for any cadence from 1 to 8 nodes)
+            if ((j + 1) % 4 == 0 && j + 1 < J) {
                 o("  }");
                 o("  __syncthreads();");
                 o("  if (do_step) {");
@@ -689,7 +629,7 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
         if (has_seg[j]) o("  double xs%d = 0.0;", j);
     for (int c0 = 0; c0 < E; c0 += 32) {
         const int c1 = std::min(E, c0 + 32);
-        o(env_int("ORGYM_NET_JIT_SYNC", 0, 0, 1) ? "  __syncthreads();" : "  __syncwarp();");
+        o("  __syncwarp();");
         o("  for (int r = wrow0; r < wrow1; r++)");
         o("    if (%d + ln < NE) tile[r * 33 + ln] = A.actions[(e0 + r) * NE + %d + ln];", c0, c0);
         o("  __syncwarp();");
@@ -725,148 +665,109 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
         o("  }");
     }
     // ---- pass B: nodes
-    // ORGYM_NET_JIT_SYNC=1: a CTA-wide barrier after every node group keeps the warps of a CTA inside the same few hundred
-    // instructions, so that a line of this long straight-line kernel is fetched into the instruction cache once per CTA
-    // instead of once per warp (ncu: 7 of 18 stall cycles per issue were instruction fetch).
-    const int SYNC = env_int("ORGYM_NET_JIT_SYNC", 0, 0, 1);
-    const int LDGSTS = env_int("ORGYM_NET_JIT_LDGSTS", 0, 0, 1);  // measured: 0.428 vs 0.418 ms without -- off by default
-    if (LDGSTS) {
-        // landing zone: [16 values][32 lanes] doubles inside this warp's rows of the action tile (4224 bytes per warp)
-        o("  __syncwarp();");
-        o("  double* const lz = (double*)(tile + wrow0 * 33) + ln;");
-        o("  const unsigned lz_s = (unsigned)__cvta_generic_to_shared(lz);");
-    }
     o("  double total = 0.0;");
     o("  if (do_step) {");
     // Nodes are independent of each other in this pass (every link has one purchaser, every market link one retailer;
-    // R_t / consumed are read-only here), so they are processed in groups: all loads of a group are issued first
-    // (dozens of independent loads in flight), then the group's arithmetic and stores.
-    for (int j0 = 0; j0 < J; j0 += GROUP) {
-        const int j1 = std::min(J, j0 + GROUP);
+    // R_t / consumed are read-only here): all loads of a node are issued first, then its arithmetic and stores.  One
+    // node at a time measured fastest with the 64-register budget (0.419 ms for the step pair on the 64-node graph;
+    // groups of 2 / 3 / 4 nodes: 0.433 / 0.449 / 0.470 ms) -- fewer live values, fewer spills.
+    for (int j = 0; j < J; j++) {
         o("    {");
-        if (PF >= 2)
-            for (int j = j0 + GROUP * (PF - 1); j < std::min(J, j0 + GROUP * PF); j++) emit_prefetch_node(j, "      ");
-        // load phase.  ORGYM_NET_JIT_LDGSTS=1: every value the group needs is fetched with an asynchronous
-        // global->shared copy (cp.async, SASS LDGSTS) into a per-lane landing zone -- the warp's own 4 KB of the action tile,
-        // free after pass A -- and read back once the group has landed.  Loads in flight then cost no registers: at the 64
-        // registers that keep the whole batch resident in one wave the compiler had been serialising a node's dozen loads
-        // into ~4 dependent round trips (ncu: long_scoreboard 27 of 38 stall cycles per issue).
         struct Ld { std::string decl, addr; };
         std::vector<Ld> lds;
         char nb[160], ab[160];
-        for (int j = j0; j < j1; j++) {
-            snprintf(nb, sizeof(nb), "double x%d", j);
-            snprintf(ab, sizeof(ab), "s_X + %d * NP + el", j);
+        snprintf(nb, sizeof(nb), "double x%d", j);
+        snprintf(ab, sizeof(ab), "s_X + %d * NP + el", j);
+        lds.push_back({nb, ab});
+        if (has_seg[j]) {
+            snprintf(nb, sizeof(nb), "const double c%d", j);
+            snprintf(ab, sizeof(ab), "sc_C + %d * NP + el", j);
             lds.push_back({nb, ab});
-            if (has_seg[j]) {
-                snprintf(nb, sizeof(nb), "const double c%d", j);
-                snprintf(ab, sizeof(ab), "sc_C + %d * NP + el", j);
+        }
+        for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
+            const int i = P.pred_idx[z], L = P.L[i];
+            snprintf(nb, sizeof(nb), "const double rt%d", i);
+            snprintf(ab, sizeof(ab), "sc_R + %d * NP + el", i);
+            lds.push_back({nb, ab});
+            snprintf(nb, sizeof(nb), "const double y%d", i);
+            snprintf(ab, sizeof(ab), "s_Y + %d * NP + el", i);
+            lds.push_back({nb, ab});
+            if (L > 0) {
+                o("      double* const slot%d = ring + (%d + t %% %d) * NP + el;", i, P.roff[i], L);
+                snprintf(nb, sizeof(nb), "const double ar%d", i);
+                snprintf(ab, sizeof(ab), "slot%d", i);
                 lds.push_back({nb, ab});
-            }
-            for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
-                const int i = P.pred_idx[z], L = P.L[i];
-                snprintf(nb, sizeof(nb), "const double rt%d", i);
-                snprintf(ab, sizeof(ab), "sc_R + %d * NP + el", i);
-                lds.push_back({nb, ab});
-                snprintf(nb, sizeof(nb), "const double y%d", i);
-                snprintf(ab, sizeof(ab), "s_Y + %d * NP + el", i);
-                lds.push_back({nb, ab});
-                if (L > 0) {
-                    o("      double* const slot%d = ring + (%d + t %% %d) * NP + el;", i, P.roff[i], L);
-                    snprintf(nb, sizeof(nb), "const double ar%d", i);
-                    snprintf(ab, sizeof(ab), "slot%d", i);
-                    lds.push_back({nb, ab});
-                }
-            }
-            for (int r = 0; r < M; r++)
-                if (P.rt_node[r] == j) {
-                    snprintf(nb, sizeof(nb), "const double u%d", r);
-                    snprintf(ab, sizeof(ab), "s_U + %d * NP + el", r);
-                    lds.push_back({nb, ab});
-                }
-            for (int z = P.succ_ptr[j]; z < P.succ_ptr[j + 1]; z++) {
-                const int l = P.succ_idx[z];
-                if (l < E) {
-                    snprintf(nb, sizeof(nb), "const double qs%d_%d", j, l);
-                    snprintf(ab, sizeof(ab), "sc_R + %d * NP + el", l);
-                    lds.push_back({nb, ab});
-                }
             }
         }
-        if (LDGSTS) {
-            for (size_t b0 = 0; b0 < lds.size(); b0 += 16) {  // the landing zone holds 16 values per lane
-                const size_t b1 = std::min(lds.size(), b0 + 16);
-                for (size_t k = b0; k < b1; k++)
-                    o("      asm volatile(\"cp.async.ca.shared.global [%%0], [%%1], 8;\" ::\"r\"(lz_s + %uu), \"l\"(%s) : \"memory\");",
-                      (unsigned)((k - b0) * 256), lds[k].addr.c_str());
-                o("      asm volatile(\"cp.async.commit_group;\" ::: \"memory\");");
-                o("      asm volatile(\"cp.async.wait_group 0;\" ::: \"memory\");");
-                for (size_t k = b0; k < b1; k++) o("      %s = lz[%u];", lds[k].decl.c_str(), (unsigned)((k - b0) * 32));
+        for (int r = 0; r < M; r++)
+            if (P.rt_node[r] == j) {
+                snprintf(nb, sizeof(nb), "const double u%d", r);
+                snprintf(ab, sizeof(ab), "s_U + %d * NP + el", r);
+                lds.push_back({nb, ab});
             }
-        } else {
-            for (const Ld& l : lds) o("      %s = *(%s);", l.decl.c_str(), l.addr.c_str());
+        for (int z = P.succ_ptr[j]; z < P.succ_ptr[j + 1]; z++) {
+            const int l = P.succ_idx[z];
+            if (l < E) {
+                snprintf(nb, sizeof(nb), "const double qs%d_%d", j, l);
+                snprintf(ab, sizeof(ab), "sc_R + %d * NP + el", l);
+                lds.push_back({nb, ab});
+            }
         }
-        for (int j = j0; j < j1; j++) {  // compute + store phase
-            o("      { double arr = 0.0, PC = 0.0, HCp = 0.0;");
-            for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
-                const int i = P.pred_idx[z], L = P.L[i];
-                link_done[i] = 1;
-                if (L == 0)
-                    o("        { const double ar = rt%d;", i);
-                else
-                    o("        { const double ar = ar%d; *slot%d = rt%d;%s", i, i, i,
-                      P.ring32 ? (std::string(" r32[slot") + std::to_string(i) + " - ring] = (float)rt" + std::to_string(i) + ";").c_str() : "");
-                o("          arr += ar; const double yn = (y%d - ar) + rt%d; s_Y[%d * NP + el] = yn;", i, i, i);
-                o("          PC += %s * rt%d; HCp += %s * (yn > 0.0 ? yn : 0.0); }", lit(P.p[i]).c_str(), i, lit(P.g[i]).c_str());
-            }
-            if (has_seg[j])
-                o("        double x = (x%d + arr) - c%d;", j, j);
+        for (const Ld& l : lds) o("      %s = *(%s);", l.decl.c_str(), l.addr.c_str());
+        o("      { double arr = 0.0, PC = 0.0, HCp = 0.0;");
+        for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
+            const int i = P.pred_idx[z], L = P.L[i];
+            link_done[i] = 1;
+            if (L == 0)
+                o("        { const double ar = rt%d;", i);
             else
-                o("        double x = (x%d + arr) - 0.0;", j);
-            o("        double SR = 0.0, sold = 0.0, UP = 0.0;");
-            for (int r = 0; r < M; r++) {
-                if (P.rt_node[r] != j) continue;
-                o("        double S%d, U%d;", r, r);
-                o("        { double d;");
-                o("          if (A.demand) d = rint(A.demand[e * A.d_se + %d]);", r);
-                o("          else d = (double)sample_fixed(dem[%d], dem[%d].table, key, episode, t, %du);", r, r, r);
-                o("          d = d > 0.0 ? d : 0.0;");
-                o("          const double fill = d + u%d; const double invr = x > 0.0 ? x : 0.0;", r);
-                o("          S%d = invr < fill ? invr : fill; x = x - S%d; const double un = fill - S%d; U%d = %s;", r, r, r, r,
-                  P.backlog ? "un" : "0.0");
-                o("          s_U[%d * NP + el] = U%d;", r, r);
-                o("          if (A.info_demand) A.info_demand[NET_IIDX(A, e, NM, %d)] = d;", r);
-                o("          if (A.info_sales) A.info_sales[NET_IIDX(A, e, NE + NM, %d)] = S%d; }", E + r, r);
-            }
-            o("        s_X[%d * NP + el] = x;", j);
-            for (int z = P.succ_ptr[j]; z < P.succ_ptr[j + 1]; z++) {
-                const int l = P.succ_idx[z];
-                if (l < E)
-                    o("        SR += %s * qs%d_%d; sold += qs%d_%d;", lit(P.p[l]).c_str(), j, l, j, l);
-                else {
-                    const int r = l - E;
-                    if (P.is_retail[j]) o("        UP += %s * U%d;", lit(P.rt_b[r]).c_str(), r);
-                    o("        SR += %s * S%d; sold += S%d;", lit(P.rt_p[r]).c_str(), r, r);
-                }
-            }
-            o("        const double xp = x > 0.0 ? x : 0.0; const double HC = %s * xp + HCp; double OC = 0.0;", lit(P.h[j]).c_str());
-            if (P.is_factory[j]) {
-                if (!(P.v[j] > 0.0))
-                    o("        OC = 0.0;");
-                else if (P.v[j] == 1.0)
-                    o("        OC = %s * sold;", lit(P.o[j]).c_str());
-                else
-                    o("        OC = %s * (sold / %s);", lit(P.o[j]).c_str(), lit(P.v[j]).c_str());
-            }
-            o("        (void)sold; const double pj = (((SR - PC) - OC) - HC) - UP; total += pj;");
-            o("        if (A.info_profit) A.info_profit[NET_IIDX(A, e, NJ, %d)] = pj; }", j);
+                o("        { const double ar = ar%d; *slot%d = rt%d;%s", i, i, i,
+                  P.ring32 ? (std::string(" r32[slot") + std::to_string(i) + " - ring] = (float)rt" + std::to_string(i) + ";").c_str() : "");
+            o("          arr += ar; const double yn = (y%d - ar) + rt%d; s_Y[%d * NP + el] = yn;", i, i, i);
+            o("          PC += %s * rt%d; HCp += %s * (yn > 0.0 ? yn : 0.0); }", lit(P.p[i]).c_str(), i, lit(P.g[i]).c_str());
         }
+        if (has_seg[j])
+            o("        double x = (x%d + arr) - c%d;", j, j);
+        else
+            o("        double x = (x%d + arr) - 0.0;", j);
+        o("        double SR = 0.0, sold = 0.0, UP = 0.0;");
+        for (int r = 0; r < M; r++) {
+            if (P.rt_node[r] != j) continue;
+            o("        double S%d, U%d;", r, r);
+            o("        { double d;");
+            o("          if (A.demand) d = rint(A.demand[e * A.d_se + %d]);", r);
+            o("          else d = (double)sample_fixed(dem[%d], dem[%d].table, key, episode, t, %du);", r, r, r);
+            o("          d = d > 0.0 ? d : 0.0;");
+            o("          const double fill = d + u%d; const double invr = x > 0.0 ? x : 0.0;", r);
+            o("          S%d = invr < fill ? invr : fill; x = x - S%d; const double un = fill - S%d; U%d = %s;", r, r, r, r,
+              P.backlog ? "un" : "0.0");
+            o("          s_U[%d * NP + el] = U%d;", r, r);
+            o("          if (A.info_demand) A.info_demand[NET_IIDX(A, e, NM, %d)] = d;", r);
+            o("          if (A.info_sales) A.info_sales[NET_IIDX(A, e, NE + NM, %d)] = S%d; }", E + r, r);
+        }
+        o("        s_X[%d * NP + el] = x;", j);
+        for (int z = P.succ_ptr[j]; z < P.succ_ptr[j + 1]; z++) {
+            const int l = P.succ_idx[z];
+            if (l < E)
+                o("        SR += %s * qs%d_%d; sold += qs%d_%d;", lit(P.p[l]).c_str(), j, l, j, l);
+            else {
+                const int r = l - E;
+                if (P.is_retail[j]) o("        UP += %s * U%d;", lit(P.rt_b[r]).c_str(), r);
+                o("        SR += %s * S%d; sold += S%d;", lit(P.rt_p[r]).c_str(), r, r);
+            }
+        }
+        o("        const double xp = x > 0.0 ? x : 0.0; const double HC = %s * xp + HCp; double OC = 0.0;", lit(P.h[j]).c_str());
+        if (P.is_factory[j]) {
+            if (!(P.v[j] > 0.0))
+                o("        OC = 0.0;");
+            else if (P.v[j] == 1.0)
+                o("        OC = %s * sold;", lit(P.o[j]).c_str());
+            else
+                o("        OC = %s * (sold / %s);", lit(P.o[j]).c_str(), lit(P.v[j]).c_str());
+        }
+        o("        (void)sold; const double pj = (((SR - PC) - OC) - HC) - UP; total += pj;");
+        o("        if (A.info_profit) A.info_profit[NET_IIDX(A, e, NJ, %d)] = pj; }", j);
         o("    }");
-        if (SYNC && j1 < J) {
-            o("  }");
-            o("  __syncthreads();");
-            o("  if (do_step) {");
-        }
     }
     }
     for (int i = 0; i < E; i++) {  // reorder links whose purchaser holds no inventory: pipeline bookkeeping only
@@ -926,63 +827,25 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
             }
             k += L;
         }
-        if (stream_async()) {
-            // Asynchronous staging: every thread copies the float64 sources of CW observation columns of its own
-            // instance straight into shared memory with cp.async (SASS LDGSTS: no destination registers, no
-            // scoreboard wait), NST chunks deep; the warp then converts and writes the rows of its 32 lanes with
-            // coalesced stores.  Every warp owns the rows of its lanes in every stage, so __syncwarp suffices.
-            const int CW = stream_cw(), NST = stream_nst(), RPI = 32 / CW;
-            const int nchunk = (W + CW - 1) / CW;
-            o("  __syncthreads();   // the action tile of pass A and the staging buffers share the dynamic shared memory");
-            o("  double* dt = (double*)smem_raw;   // [%d stages][NTHR][%d + 1]", NST, CW);
-            o("  const unsigned dt_me = (unsigned)__cvta_generic_to_shared(dt + tid * %d);", CW + 1);
-            o("  const int lc = ln %% %d, lr = ln / %d;", CW, CW);
-            auto emit_issue = [&](int ch) {
-                if (ch < nchunk) {
-                    const int c0 = ch * CW, c1 = std::min(W, c0 + CW), st = ch % NST;
-                    o("  if (valid) {");
-                    for (int c = c0; c < c1; c++)
-                        o("    asm volatile(\"cp.async.ca.shared.global [%%0], [%%1], 8;\" :: \"r\"(dt_me + %du * NTHR + %du), \"l\"(&%s) : \"memory\");",
-                          (unsigned)(st * (CW + 1) * 8), (unsigned)(8 * (c - c0)), col[(size_t)c].c_str());
-                    o("  }");
-                }
-                o("  asm volatile(\"cp.async.commit_group;\" ::: \"memory\");");
-            };
-            for (int ch = 0; ch < NST - 1; ch++) emit_issue(ch);
-            for (int ch = 0; ch < nchunk; ch++) {
-                const int c0 = ch * CW, st = ch % NST;
-                emit_issue(ch + NST - 1);
-                o("  asm volatile(\"cp.async.wait_group %d;\" ::: \"memory\");", NST - 1);
-                o("  __syncwarp();");
-                o("  { const double* sb_ = dt + %d * NTHR;", st * (CW + 1));
-                o("    for (int r = wrow0 + lr; r < wrow1; r += %d)", RPI);
-                o("      if (%d + lc < NOBS) __stcs(A.obs + (e0 + r) * NOBS + %d + lc, (float)sb_[r * %d + lc]); }", c0, c0, CW + 1);
-                o("  __syncwarp();");
-            }
-        } else {
-            // double-buffered: the loads of chunk c+1 are issued before chunk c is flushed, so their latency overlaps the flush
-            int dbuf = 1;
-            if (const char* dv = getenv("ORGYM_NET_JIT_DBUF")) dbuf = atoi(dv) ? 1 : 0;
-            o("  float v[32];");
-            if (dbuf) o("  float vn[32];");
-            auto emit_loads = [&](const char* dst, int c0) {
-                const int c1 = std::min(W, c0 + 32);
-                o("  if (valid) {");
-                for (int c = c0; c < c1; c++) o("    %s[%d] = (float)%s;", dst, c - c0, col[(size_t)c].c_str());
-                o("  }");
-            };
-            if (dbuf) emit_loads("v", 0);
-            for (int c0 = 0; c0 < W; c0 += 32) {
-                const int c1 = std::min(W, c0 + 32);
-                if (!dbuf) emit_loads("v", c0);
-                if (dbuf && c0 + 32 < W) emit_loads("vn", c0 + 32);
-                o("  _Pragma(\"unroll\") for (int c = 0; c < %d; c++) trow[c] = v[c];", c1 - c0);
-                o("  __syncwarp();");
-                o("  for (int r = wrow0; r < wrow1; r++)");
-                o("    if (%d + ln < NOBS) __stcs(A.obs + (e0 + r) * NOBS + %d + ln, tile[r * 33 + ln]);", c0, c0);
-                o("  __syncwarp();");
-                if (dbuf && c0 + 32 < W) o("  _Pragma(\"unroll\") for (int c = 0; c < 32; c++) v[c] = vn[c];");
-            }
+        // double-buffered: the loads of chunk c+1 are issued before chunk c is flushed, so their latency overlaps the flush
+        o("  float v[32];");
+        o("  float vn[32];");
+        auto emit_loads = [&](const char* dst, int c0) {
+            const int c1 = std::min(W, c0 + 32);
+            o("  if (valid) {");
+            for (int c = c0; c < c1; c++) o("    %s[%d] = (float)%s;", dst, c - c0, col[(size_t)c].c_str());
+            o("  }");
+        };
+        emit_loads("v", 0);
+        for (int c0 = 0; c0 < W; c0 += 32) {
+            const int c1 = std::min(W, c0 + 32);
+            if (c0 + 32 < W) emit_loads("vn", c0 + 32);
+            o("  _Pragma(\"unroll\") for (int c = 0; c < %d; c++) trow[c] = v[c];", c1 - c0);
+            o("  __syncwarp();");
+            o("  for (int r = wrow0; r < wrow1; r++)");
+            o("    if (%d + ln < NOBS) __stcs(A.obs + (e0 + r) * NOBS + %d + ln, tile[r * 33 + ln]);", c0, c0);
+            o("  __syncwarp();");
+            if (c0 + 32 < W) o("  _Pragma(\"unroll\") for (int c = 0; c < 32; c++) v[c] = vn[c];");
         }
     }
     o("}");
@@ -992,10 +855,6 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
 int net_jit_build(NetHandle* H, std::string* err) {
     const NetDev& P = H->dev;
     H->jit_threads = 128;
-    if (const char* tv = getenv("ORGYM_NET_JIT_THREADS")) {  // tuning knob: 64 / 128 / 256 threads per CTA
-        const int t = atoi(tv);
-        if (t == 64 || t == 128 || t == 256 || t == 512) H->jit_threads = t;
-    }
     std::string src = net_jit_source(P, H->jit_threads);
     H->jit_stream = net_jit_uses_stream(P);
     H->jit_obs_split = H->jit_stream && net_jit_obs_split(P);
@@ -1031,7 +890,8 @@ int net_jit_launch(const NetHandle* H, const NetSimArgs& A_in, cudaStream_t s) {
     size_t smem = 16;
     if (!A.rollout && H->jit_stream) {
         A.use_tile = 0;  // the streaming kernel stages through its own tiles
-        smem = H->jit_onepass && H->jit_obs_split ? 16 : net_jit_stream_smem(nthr);  // the single-pass form stages nothing
+        // [NTHR][33] float staging tile of pass A (two-pass form) and pass C; the single-pass form stages nothing
+        smem = H->jit_onepass && H->jit_obs_split ? 16 : (size_t)nthr * 33 * 4;
     } else if (!A.rollout) {
         A.use_tile = tile <= 160 * 1024 ? 1 : 0;
         if (A.use_tile) smem = tile;

@@ -100,13 +100,12 @@ def test_newsvendor_no_oob_writes(N):
     env.close()
 
 
-@pytest.mark.parametrize("mode", ["specialised", "stream", "stream_jit", "stream_jit_twopass", "generic"])
+@pytest.mark.parametrize("mode", ["specialised", "stream_jit", "stream_jit_twopass", "generic"])
 @pytest.mark.parametrize("N", [1, 127, 129, 600])
 def test_netinv_no_oob_writes(N, mode, monkeypatch):
     torch = _torch()
     monkeypatch.setenv("ORGYM_NET_JIT", "0" if mode == "generic" else "2")
     monkeypatch.setenv("ORGYM_NET_JIT_STREAM", "1" if mode.startswith("stream") else "0")
-    monkeypatch.setenv("ORGYM_NET_STREAM_AOT", "0" if mode.startswith("stream_jit") else "1")
     monkeypatch.setenv("ORGYM_NET_JIT_ONEPASS", "0" if mode == "stream_jit_twopass" else "1")
     env = pkg.NetInvMgmtBacklogEnv(num_envs=N, device="cuda:0", autoreset_mode="same_step", num_periods=5)
     g = Guard()

@@ -14,17 +14,16 @@ def _torch():
     return torch
 
 
-@pytest.fixture(params=["specialised", "stream_aot", "stream_jit", "stream_jit_twopass", "stream_jit_fused_obs", "generic"])
+@pytest.fixture(params=["specialised", "stream_jit", "stream_jit_twopass", "stream_jit_fused_obs", "generic"])
 def kernel_mode(request, monkeypatch):
     """Run the parity tests through all network kernels: the NVRTC-specialised register-resident one; the streaming
-    STEP path meant for large graphs, forced here, in its forms -- table-driven ahead-of-time kernel + observation
-    kernel, generated streaming kernel (single pass over the nodes: the default for large graphs; or two passes with
-    scratch rows, the form for graphs whose suppliers do not follow their purchasers in node order) + observation kernel,
-    generated kernel with its own fused observation pass --; and the generic constant-bank interpreter."""
+    STEP path meant for large graphs, forced here, in its forms -- generated streaming kernel (single pass over the
+    nodes: the default for large graphs; or two passes with scratch rows, the form for graphs whose suppliers do not
+    follow their purchasers in node order) + observation kernel, generated kernel with its own fused observation
+    pass --; and the generic constant-bank interpreter."""
     m = request.param
     monkeypatch.setenv("ORGYM_NET_JIT", "0" if m == "generic" else "2")
     monkeypatch.setenv("ORGYM_NET_JIT_STREAM", "1" if m.startswith("stream") else "0")
-    monkeypatch.setenv("ORGYM_NET_STREAM_AOT", "1" if m == "stream_aot" else "0")
     monkeypatch.setenv("ORGYM_NET_OBS_TMA", "0" if m == "stream_jit_fused_obs" else "1")
     monkeypatch.setenv("ORGYM_NET_JIT_ONEPASS", "0" if m == "stream_jit_twopass" else "1")
     return m

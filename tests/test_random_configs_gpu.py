@@ -135,14 +135,13 @@ def _random_graph(rng, ordered=False):
     return g
 
 
-@pytest.mark.parametrize("mode", ["specialised", "stream", "stream_jit", "stream_jit_twopass", "generic"])
+@pytest.mark.parametrize("mode", ["specialised", "stream_jit", "stream_jit_twopass", "generic"])
 @pytest.mark.parametrize("case", range(6 * STRESS))
 def test_netinv_random_graph(case, mode, monkeypatch):
     from oracle import oracle
     torch = _torch()
     monkeypatch.setenv("ORGYM_NET_JIT", "0" if mode == "generic" else "2")
     monkeypatch.setenv("ORGYM_NET_JIT_STREAM", "1" if mode.startswith("stream") else "0")
-    monkeypatch.setenv("ORGYM_NET_STREAM_AOT", "0" if mode.startswith("stream_jit") else "1")
     monkeypatch.setenv("ORGYM_NET_JIT_ONEPASS", "0" if mode == "stream_jit_twopass" else "1")
     rng = np.random.default_rng(3000 + case)
     g = _random_graph(rng, ordered=bool(case % 2))
