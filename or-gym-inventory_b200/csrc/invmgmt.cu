@@ -7,7 +7,11 @@
 //                       tile go through shared memory and the TMA engine (cp.async.bulk)
 //   inv_rollout_kernel  fused reset + `periods` steps with on-device policy and Philox demand; on-hand
 //                       inventory / backlog in registers, lead-time rings in shared memory; issue-bound
-//   inv_reduce_kernel   deterministic reduction of the per-CTA episode statistics
+//   inv_mlp_rollout_kernel  the same fused rollout with an MLP actor evaluated on the device every period
+//   inv_export_kernel   state export to int64 I / B / period arrays
+//
+// The rollout kernels write one row of partial sums per 128 envs; orgym_launch_reduce (api.cu) reduces them
+// deterministically into the episode summary.  invmgmt_jit.cu generates the specialised rollout kernels.
 //
 // Integer state is exact (int64, or int32 with a range guard); rewards are float64 evaluated in the reference's
 // operation order (no FMA contraction: the library is built with --fmad=false).
@@ -218,10 +222,8 @@ __global__ void __launch_bounds__(256) inv_reset_kernel(const __grid_constant__ 
 }
 
 // ---- step ------------------------------------------------------------------------------------------------------
-// t % d for 0 <= t < 2^20 and 1 <= d <= 64 without a division: q = mulhi(t, ceil(2^32 / d)) is exact in that range
-#ifndef ORGYM_STEP_MIN_BLOCKS
 #define ORGYM_STEP_MIN_BLOCKS 6
-#endif
+// t % d for 0 <= t < 2^20 and 1 <= d <= 64 without a division: q = mulhi(t, ceil(2^32 / d)) is exact in that range
 __device__ __forceinline__ int mod_small(int t, int d, uint32_t magic) {
     return magic ? t - (int)__umulhi((uint32_t)t, magic) * d : 0;  // magic == 0 encodes d == 1
 }
@@ -1009,6 +1011,57 @@ __global__ void __launch_bounds__(MLP_THREADS, (EXACT && NS <= 4 && sizeof(S) ==
 // ------------------------------------------------------------------------------------------------
 // host side of the C ABI
 // ------------------------------------------------------------------------------------------------
+// The fields of InvDev a configuration determines, without validation (orgym_invmgmt_create validates like the
+// reference first).  The price arrays may be absent (orgym_invmgmt_value_bounds without profit_mag): prices stay 0.
+static void inv_dev_from_config(const orgym_invmgmt_config_t* cfg, InvDev* P) {
+    const int n = cfg->num_stages - 1;
+    memset(P, 0, sizeof(*P));
+    P->n = n;
+    P->m = n + 1;
+    P->T = cfg->periods;
+    P->backlog = cfg->backlog ? 1 : 0;
+    for (int i = 0; i < n; i++) {
+        P->I0[i] = cfg->init_inv[i];
+        P->c[i] = cfg->capacity[i];
+        P->L[i] = (int)cfg->lead_time[i];
+        P->roff[i] = P->sumL;
+        P->sumL += P->L[i];
+        if (P->L[i] > P->lt_max) P->lt_max = P->L[i];
+    }
+    if (cfg->unit_price && cfg->unit_cost && cfg->demand_cost && cfg->holding_cost)
+        for (int j = 0; j <= n; j++) {
+            P->up[j] = cfg->unit_price[j];
+            P->uc[j] = cfg->unit_cost[j];
+            P->kc[j] = cfg->demand_cost[j];
+            P->hc[j] = cfg->holding_cost[j];
+        }
+    P->obs_dim = n * (P->lt_max + 1);
+    for (int i = 0; i < n; i++) P->Lmagic[i] = P->L[i] > 1 ? (uint32_t)((0x100000000ULL + P->L[i] - 1) / P->L[i]) : 0u;
+    P->Lm_magic = P->lt_max > 1 ? (uint32_t)((0x100000000ULL + P->lt_max - 1) / P->lt_max) : 0u;
+}
+
+// alpha**t for t = 0..T-1 with libm pow, like CPython's float ** int
+static std::vector<double> inv_discounts(double alpha, int T) {
+    std::vector<double> disc((size_t)T);
+    for (int t = 0; t < T; t++) disc[(size_t)t] = std::pow(alpha, (double)t);
+    return disc;
+}
+
+// log2 of the alias-table size and the support's base of a sampled demand distribution (as orgym_build_alias builds it)
+static int inv_demand_table(const orgym_dist_t* d, int* log2k, int64_t* base) {
+    std::vector<double> pmf;
+    if (int rc = orgym_dist_pmf(d, &pmf, base)) return rc;
+    *log2k = 0;
+    while ((size_t(1) << *log2k) < pmf.size()) ++*log2k;
+    return ORGYM_OK;
+}
+
+// shared memory of the demand's alias table staged by the step and rollout kernels (a user trace stages none)
+static size_t inv_alias_smem(const InvDev& P) { return P.dem.kind == ORGYM_DIST_USER ? 0 : (size_t(8) << P.dem.log2k); }
+// dynamic shared memory above which the step kernel writes observations directly and the rollout kernel keeps its
+// lead-time rings in global scratch (correct, not fast)
+#define INV_STAGING_SMEM_LIMIT (200 * 1024)
+
 template <typename S>
 static void launch_step(const InvHandle* H, const InvStepArgs& A, size_t smem, cudaStream_t s) {
     const InvDev& P = H->dev;
@@ -1103,7 +1156,7 @@ static int inv_mlp_plan(const InvDev& P, const orgym_mlp_t* mlp, int rslots, siz
         f += a4(l < L - 1 ? M->Np[l] : M->K[l + 1]);
     }
     const int wfloats = f;
-    const size_t tab = P.dem.kind == ORGYM_DIST_USER ? 0 : (size_t(8) << P.dem.log2k);
+    const size_t tab = inv_alias_smem(P);
     const int nbuf = L >= 3 ? 2 : (L == 2 ? 1 : 0);
     size_t smem = 0;
     for (int E = 64; E >= 32; E /= 2) {
@@ -1148,15 +1201,7 @@ extern "C" int orgym_invmgmt_create(const orgym_invmgmt_config_t* cfg, int64_t n
         orgym_set_error("%d inventory stages exceed this build's limit of %d", n, MAXN);
         return ORGYM_E_UNSUPPORTED;
     }
-    InvHandle* H = new InvHandle();
-    InvDev& P = H->dev;
-    memset(&P, 0, sizeof(P));
-    P.n = n;
-    P.m = m;
-    P.T = cfg->periods;
-    P.backlog = cfg->backlog ? 1 : 0;
     int rc = ORGYM_OK;
-    long long cmax = 0;
     for (int i = 0; i < n && rc == ORGYM_OK; i++) {
         if (cfg->init_inv[i] < 0) { orgym_set_error("Initial inventory cannot be negative"); rc = ORGYM_E_INVALID; }
         if (cfg->capacity[i] <= 0) { orgym_set_error("Supply capacities must be positive"); rc = ORGYM_E_INVALID; }
@@ -1165,21 +1210,9 @@ extern "C" int orgym_invmgmt_create(const orgym_invmgmt_config_t* cfg, int64_t n
             orgym_set_error("lead time %lld exceeds this build's limit of %d", (long long)cfg->lead_time[i], ORGYM_INV_MAX_LEAD);
             rc = ORGYM_E_UNSUPPORTED;
         }
-        P.I0[i] = cfg->init_inv[i];
-        P.c[i] = cfg->capacity[i];
-        P.L[i] = (int)cfg->lead_time[i];
-        P.roff[i] = P.sumL;
-        P.sumL += P.L[i];
-        if (P.L[i] > P.lt_max) P.lt_max = P.L[i];
-        if (P.c[i] > cmax) cmax = P.c[i];
-        if (P.I0[i] > cmax) cmax = P.I0[i];
     }
     for (int j = 0; j < m && rc == ORGYM_OK; j++) {
-        P.up[j] = cfg->unit_price[j];
-        P.uc[j] = cfg->unit_cost[j];
-        P.kc[j] = cfg->demand_cost[j];
-        P.hc[j] = cfg->holding_cost[j];
-        if (P.up[j] < 0 || P.uc[j] < 0 || P.kc[j] < 0 || P.hc[j] < 0) {
+        if (cfg->unit_price[j] < 0 || cfg->unit_cost[j] < 0 || cfg->demand_cost[j] < 0 || cfg->holding_cost[j] < 0) {
             orgym_set_error("prices and costs cannot be negative");
             rc = ORGYM_E_INVALID;
         }
@@ -1192,24 +1225,26 @@ extern "C" int orgym_invmgmt_create(const orgym_invmgmt_config_t* cfg, int64_t n
         orgym_set_error("User specified demand length != num periods");
         rc = ORGYM_E_INVALID;
     }
-    P.obs_dim = n * (P.lt_max + 1);
-    for (int i = 0; i < n; i++) P.Lmagic[i] = P.L[i] > 1 ? (uint32_t)((0x100000000ULL + P.L[i] - 1) / P.L[i]) : 0u;
-    P.Lm_magic = P.lt_max > 1 ? (uint32_t)((0x100000000ULL + P.lt_max - 1) / P.lt_max) : 0u;
     if (rc == ORGYM_OK && cfg->periods > (1 << 20)) {
         orgym_set_error("periods above 2^20 are not supported");
         rc = ORGYM_E_UNSUPPORTED;
     }
+    if (rc != ORGYM_OK) return rc;
+    InvHandle* H = new InvHandle();
+    InvDev& P = H->dev;
+    inv_dev_from_config(cfg, &P);
+    long long cmax = 0;
+    for (int i = 0; i < n; i++) cmax = std::max({cmax, P.c[i], P.I0[i]});
     H->wide = cfg->wide_state ? 1 : 0;
-    if (rc == ORGYM_OK && !H->wide && cmax > (INT32_GUARD >> 8)) H->wide = 1;  // compact int32 state cannot hold it
-    if (rc == ORGYM_OK) rc = orgym_handle_base_init(&H->base, FAM_INVMGMT, device, num_envs);
+    if (!H->wide && cmax > (INT32_GUARD >> 8)) H->wide = 1;  // compact int32 state cannot hold it
+    rc = orgym_handle_base_init(&H->base, FAM_INVMGMT, device, num_envs);
     if (rc != ORGYM_OK) {
         delete H;
         return rc;
     }
     DeviceGuard g(device);
     H->npad = round_up(num_envs, 32);
-    std::vector<double> disc((size_t)P.T);
-    for (int t = 0; t < P.T; t++) disc[(size_t)t] = std::pow(cfg->alpha, (double)t);  // CPython float ** int == libm pow
+    const std::vector<double> disc = inv_discounts(cfg->alpha, P.T);
     double* disc_dev = nullptr;
     cudaError_t ce = cudaMalloc(&disc_dev, sizeof(double) * (size_t)P.T);
     if (ce == cudaSuccess) {
@@ -1296,15 +1331,6 @@ extern "C" int orgym_invmgmt_reset(orgym_handle_t h, void* state_dev, int reseed
     return ORGYM_OK;
 }
 
-static int g_use_bulk = -1;
-static int use_bulk() {
-    if (g_use_bulk < 0) {
-        const char* v = getenv("ORGYM_NO_BULK");
-        g_use_bulk = (v && v[0] == '1') ? 0 : 1;
-    }
-    return g_use_bulk;
-}
-
 extern "C" int orgym_invmgmt_step(orgym_handle_t h, void* state_dev, const void* actions_dev, int action_is_f64,
                                   const int64_t* demand_override_dev, int autoreset_mode, int64_t* obs_dev,
                                   double* reward_dev, uint8_t* terminated_dev, uint8_t* truncated_dev,
@@ -1347,13 +1373,13 @@ extern "C" int orgym_invmgmt_step(orgym_handle_t h, void* state_dev, const void*
         else
             H->hint_t = (t + 1 >= P.T && autoreset_mode == ORGYM_AUTORESET_SAME_STEP) ? 0 : t + 1;
     }
-    A.use_bulk = use_bulk() && ((uintptr_t)actions_dev % 16 == 0) && ((uintptr_t)obs_dev % 16 == 0);
+    A.use_bulk = ((uintptr_t)actions_dev % 16 == 0) && ((uintptr_t)obs_dev % 16 == 0);
     int ostride = (P.obs_dim & 1) ? P.obs_dim : P.obs_dim + 1;
-    size_t smem = (((size_t)ORGYM_TILE * ostride * (H->wide ? 8 : 4) + 15) & ~(size_t)15) + (size_t)ORGYM_TILE * P.n * 8 + 16 +
-                  (P.dem.kind == ORGYM_DIST_USER ? 0 : (size_t(8) << P.dem.log2k));
-    if (smem > 200 * 1024) {  // rows too long to stage: the generic kernel writes them directly (correct, not fast)
+    const size_t rest = (size_t)ORGYM_TILE * P.n * 8 + 16 + inv_alias_smem(P);  // action tile, mbarrier, alias table
+    size_t smem = (((size_t)ORGYM_TILE * ostride * (H->wide ? 8 : 4) + 15) & ~(size_t)15) + rest;
+    if (smem > INV_STAGING_SMEM_LIMIT) {  // rows too long to stage: the generic kernel writes them directly
         A.direct_obs = 1;
-        smem = (size_t)ORGYM_TILE * P.n * 8 + 16 + (P.dem.kind == ORGYM_DIST_USER ? 0 : (size_t(8) << P.dem.log2k));
+        smem = rest;
     }
     if (H->wide)
         launch_step<long long>(H, A, smem, (cudaStream_t)stream);
@@ -1425,12 +1451,12 @@ static void inv_value_bounds(const InvDev& P, double dmax, double* xvar, double*
 }
 
 // ---- run-time specialised rollout (invmgmt_jit.cu) ------------------------------------------------------------------
-static void inv_jit_spec(const InvDev& P, const std::vector<double>& disc, int log2k, int base, int policy,
-                         const long long* target, InvJitSpec* S) {
+static void inv_jit_spec(const InvDev& P, const std::vector<double>& disc, int policy, const long long* target,
+                         InvJitSpec* S) {
     {
         double xv = 0.0, xs = 0.0;
         InvTermBounds tb;
-        inv_value_bounds(P, (double)base + (double)(1LL << log2k), &xv, &xs, &tb);
+        inv_value_bounds(P, (double)P.dem.base + (double)(1LL << P.dem.log2k), &xv, &xs, &tb);
         S->xbound = xv < 9.0e15 ? (long long)xv + 1 : 0;
         for (int j = 0; j <= P.n; j++) {
             S->sale_bound[j] = tb.sale[j];
@@ -1454,9 +1480,23 @@ static void inv_jit_spec(const InvDev& P, const std::vector<double>& disc, int l
         S->hc[j] = P.hc[j];
     }
     S->disc = disc;
-    S->log2k = log2k;
-    S->base = base;
+    S->log2k = P.dem.log2k;
+    S->base = P.dem.base;
     S->policy = policy;
+}
+
+// The specialiser's range: ORGYM_E_UNSUPPORTED, with the reason, for a user-trace demand (checked alone when S is null)
+// and for a kernel spec outside inv_jit_eligible.
+static int inv_jit_check(const InvDev& P, const InvJitSpec* S) {
+    if (P.dem.kind == ORGYM_DIST_USER) {
+        orgym_set_error("user-trace demand runs the ahead-of-time kernel");
+        return ORGYM_E_UNSUPPORTED;
+    }
+    if (S && !inv_jit_eligible(*S)) {
+        orgym_set_error("configuration outside the specialiser's range (1..6 stages, <= 64 periods, sum of lead times <= 40)");
+        return ORGYM_E_UNSUPPORTED;
+    }
+    return ORGYM_OK;
 }
 
 // base-stock levels (lead_times + 1) * mu * sf (benchmark_InvManagementBacklogEnv.py:186); *all_int = they are integers
@@ -1487,33 +1527,12 @@ extern "C" int orgym_invmgmt_codegen(const orgym_invmgmt_config_t* cfg, const or
     const int n = cfg->num_stages - 1;
     ORGYM_REQUIRE(n >= 1 && n <= MAXN && cfg->periods > 0, "bad stage count / horizon");
     InvDev Pb;
-    memset(&Pb, 0, sizeof(Pb));
-    Pb.n = n;
-    Pb.m = n + 1;
-    Pb.T = cfg->periods;
-    Pb.backlog = cfg->backlog ? 1 : 0;
-    for (int i = 0; i < n; i++) {
-        Pb.L[i] = (int)cfg->lead_time[i];
-        Pb.c[i] = cfg->capacity[i];
-        Pb.I0[i] = cfg->init_inv[i];
-    }
-    for (int j = 0; j <= n; j++) {
-        Pb.up[j] = cfg->unit_price[j];
-        Pb.uc[j] = cfg->unit_cost[j];
-        Pb.kc[j] = cfg->demand_cost[j];
-        Pb.hc[j] = cfg->holding_cost[j];
-    }
-    std::vector<double> disc((size_t)Pb.T);
-    for (int t = 0; t < Pb.T; t++) disc[(size_t)t] = std::pow(cfg->alpha, (double)t);
-    if (cfg->dist.kind == ORGYM_DIST_USER) {
-        orgym_set_error("user-trace demand runs the ahead-of-time kernel");
-        return ORGYM_E_UNSUPPORTED;
-    }
-    std::vector<double> pmf;
+    inv_dev_from_config(cfg, &Pb);
+    Pb.dem.kind = cfg->dist.kind;
+    if (int rc = inv_jit_check(Pb, nullptr)) return rc;  // a user trace has no demand table to specialise on
     int64_t base = 0;
-    if (int rc = orgym_dist_pmf(&cfg->dist, &pmf, &base)) return rc;
-    int log2k = 0;
-    while ((size_t(1) << log2k) < pmf.size()) log2k++;
+    if (int rc = inv_demand_table(&cfg->dist, &Pb.dem.log2k, &base)) return rc;
+    Pb.dem.base = (int32_t)base;
     // policy to bake in: the caller's, or the benchmark's default base-stock (levels (L+1) * p0, SF = 1)
     int policy = 0;
     double param[4] = {1.0, cfg->dist.p0, 0.0, 0.0};
@@ -1536,11 +1555,8 @@ extern "C" int orgym_invmgmt_codegen(const orgym_invmgmt_config_t* cfg, const or
         return ORGYM_E_UNSUPPORTED;
     }
     InvJitSpec S;
-    inv_jit_spec(Pb, disc, log2k, (int)base, policy, target_int, &S);
-    if (!inv_jit_eligible(S)) {
-        orgym_set_error("configuration outside the specialiser's range (1..6 stages, <= 64 periods, sum of lead times <= 40)");
-        return ORGYM_E_UNSUPPORTED;
-    }
+    inv_jit_spec(Pb, inv_discounts(cfg->alpha, Pb.T), policy, target_int, &S);
+    if (int rc = inv_jit_check(Pb, &S)) return rc;
     std::string src = inv_jit_source(S);
     if (needed) *needed = (int64_t)src.size();
     if (buf && buflen > 0) {
@@ -1568,24 +1584,14 @@ extern "C" int orgym_invmgmt_value_bounds(const orgym_invmgmt_config_t* cfg, dou
     const int n = cfg->num_stages - 1;
     ORGYM_REQUIRE(n >= 1 && n <= MAXN && cfg->periods > 0, "bad stage count / horizon");
     InvDev Pb;
-    memset(&Pb, 0, sizeof(Pb));
-    Pb.n = n;
-    Pb.T = cfg->periods;
-    Pb.backlog = cfg->backlog ? 1 : 0;
-    for (int i = 0; i < n; i++) {
-        Pb.L[i] = (int)cfg->lead_time[i];
-        Pb.c[i] = cfg->capacity[i];
-        Pb.I0[i] = cfg->init_inv[i];
-    }
+    inv_dev_from_config(cfg, &Pb);
     double dmax = 0.0;
     if (cfg->dist.kind == ORGYM_DIST_USER) {
         for (int t = 0; t < cfg->dist.user_D_len; t++) dmax = std::max(dmax, std::fabs((double)cfg->dist.user_D[t]));
     } else {
-        std::vector<double> pmf;
-        int64_t base = 0;
-        if (int rc = orgym_dist_pmf(&cfg->dist, &pmf, &base)) return rc;
         int log2k = 0;
-        while ((size_t(1) << log2k) < pmf.size()) log2k++;
+        int64_t base = 0;
+        if (int rc = inv_demand_table(&cfg->dist, &log2k, &base)) return rc;
         dmax = (double)base + (double)(1LL << log2k);
     }
     InvTermBounds tb;
@@ -1593,9 +1599,7 @@ extern "C" int orgym_invmgmt_value_bounds(const orgym_invmgmt_config_t* cfg, dou
     if (profit_mag) {  // bound on the sum of |terms| of one period's profit (the specialiser's exactness proof)
         ORGYM_REQUIRE(cfg->unit_price && cfg->unit_cost && cfg->demand_cost && cfg->holding_cost, "null argument");
         double mag = 0.0;
-        for (int j = 0; j <= n; j++)
-            mag += (cfg->unit_price[j] + cfg->unit_cost[j]) * tb.sale[j] + cfg->holding_cost[j] * tb.inv[j] +
-                   cfg->demand_cost[j] * tb.unf[j];
+        for (int j = 0; j <= n; j++) mag += (Pb.up[j] + Pb.uc[j]) * tb.sale[j] + Pb.hc[j] * tb.inv[j] + Pb.kc[j] * tb.unf[j];
         *profit_mag = mag;
     }
     return ORGYM_OK;
@@ -1625,16 +1629,9 @@ static int inv_jit_get(InvHandle* H, int policy, const long long* target_int, cu
         *fn = v.k.fn;
         return ORGYM_OK;
     }
-    if (P.dem.kind == ORGYM_DIST_USER) {
-        orgym_set_error("user-trace demand runs the ahead-of-time kernel");
-        return ORGYM_E_UNSUPPORTED;
-    }
     InvJitSpec S;
-    inv_jit_spec(P, H->disc_host, P.dem.log2k, P.dem.base, policy, target_int, &S);
-    if (!inv_jit_eligible(S)) {
-        orgym_set_error("configuration outside the specialiser's range (1..6 stages, <= 64 periods, sum of lead times <= 40)");
-        return ORGYM_E_UNSUPPORTED;
-    }
+    inv_jit_spec(P, H->disc_host, policy, target_int, &S);
+    if (int rc = inv_jit_check(P, &S)) return rc;
     if (H->jit_variants.size() >= 16) {  // bounded: drop the oldest variant (e.g. a sweep over safety factors)
         if (H->jit_variants.front().k.lib) orgym_jit_release(&H->jit_variants.front().k);
         H->jit_variants.erase(H->jit_variants.begin());
@@ -1693,8 +1690,7 @@ extern "C" int64_t orgym_invmgmt_rollout_scratch_bytes(orgym_handle_t h) {
     const InvDev& P = H->dev;
     int64_t rslots = 0;
     for (int i = 0; i < P.n; i++) rslots += P.L[i] > 0 ? P.L[i] : 1;
-    const size_t tab = P.dem.kind == ORGYM_DIST_USER ? 0 : (size_t(8) << P.dem.log2k);
-    if (tab + (size_t)rslots * ROLL_THREADS * 8 * 2 <= 200 * 1024) return 0;
+    if (inv_alias_smem(P) + (size_t)rslots * ROLL_THREADS * 8 * 2 <= INV_STAGING_SMEM_LIMIT) return 0;
     return rslots * round_up(H->base.num_envs, ROLL_THREADS) * 8 * 2;
 }
 
@@ -1738,25 +1734,51 @@ extern "C" int orgym_invmgmt_rollout(orgym_handle_t h, uint64_t seed, int64_t en
     A.stats32 = out->stats32_dev;
     A.action_traj = out->action_traj_dev;
     A.partials = out->summary_dev ? H->partials : nullptr;
-    // int32 arithmetic only when every state value and per-episode sum is provably below 2^31: on-device policy
-    // (requests within [0, c]), sampled demand (bounded support) and (T+1) * n * (c_max + I0_max + d_max) * 4 < 2^31;
-    // pre-staged actions / replayed demand may be arbitrary int64 -> exact wide arithmetic
-    long long vmax = 0;
-    for (int i = 0; i < P.n; i++) vmax = std::max(vmax, std::max(P.c[i], P.I0[i]));
-    long long dmax = P.dem.kind == ORGYM_DIST_USER ? (1LL << 40) : (long long)P.dem.base + (1LL << P.dem.log2k);
-    if (P.dem.kind == ORGYM_DIST_USER && !in->demand_dev) {
-        dmax = 0;  // trace values were copied to the device at create; bound them through the config-time maximum
-        dmax = H->user_dmax;
-    }
+    // int32 arithmetic only when inv_value_bounds proves every state value below 2^30 and every per-episode sum below
+    // 2^31: on-device policy (requests within [0, c]) and bounded demand -- the sampler's support, or a trace whose
+    // values were copied to the device at create and are bounded by their config-time maximum.  Pre-staged actions /
+    // replayed demand may be arbitrary int64 -> exact wide arithmetic
+    const long long dmax = P.dem.kind != ORGYM_DIST_USER ? (long long)P.dem.base + (1LL << P.dem.log2k)
+                           : in->demand_dev          ? (1LL << 40)
+                                                     : H->user_dmax;
     double xvar = 0.0, xsum = 0.0;
     inv_value_bounds(P, (double)dmax, &xvar, &xsum);
-    (void)vmax;
     const bool bounded = xvar < 1073741824.0 && xsum < 2147483648.0;
     const bool wide = H->wide || in->policy == ORGYM_POLICY_ACTIONS || in->demand_dev != nullptr || !bounded;
-    // fast path: kernels specialised for this configuration (register-resident rings, straight-line periods)
+    // fast path: kernels specialised for this configuration (register-resident rings, straight-line periods); the MLP
+    // policy and the outputs they do not produce run the ahead-of-time kernels
     H->last_rollout_jit = 0;
     const int jit_mode = inv_jit_mode();
-    if (in->policy == ORGYM_POLICY_MLP) {
+    cudaKernel_t jit_fn = nullptr;
+    if (jit_mode && !wide && inv_jit_policy_ok(in, A.target_is_int) && !A.reward_traj && !A.final_I && !A.final_B &&
+        !A.action_traj) {
+        const int jrc = inv_jit_get(H, in->policy == ORGYM_POLICY_BASE_STOCK ? 0 : 1, A.target_int, &jit_fn);
+        if (jrc != ORGYM_OK && jit_mode == 2) return jrc;  // strict: the reason is in orgym_last_error()
+    }
+    // every kernel writes one partial-sum row per ROLL_THREADS envs, so one reduction serves all three
+    static_assert(INV_JIT_THREADS == ROLL_THREADS, "the specialised kernel's CTAs must match the partial-sum rows");
+    if (jit_fn) {
+        InvJitArgs J;
+        memset(&J, 0, sizeof(J));
+        J.N = A.N;
+        J.env_offset = A.env_offset;
+        J.seed = A.seed;
+        J.episode = A.episode;
+        for (int i = 0; i < P.n; i++) J.target[i] = (int32_t)A.target_int[i];
+        J.table = P.dem.table;
+        J.ep_return = A.ep_return;
+        J.stats = A.stats;
+        J.stats32 = A.stats32;
+        J.partials = A.partials;
+        void* args[] = {(void*)&J};
+        const unsigned grid = (unsigned)((A.N + INV_JIT_THREADS - 1) / INV_JIT_THREADS);
+        cudaError_t le = cudaLaunchKernel((const void*)jit_fn, dim3(grid), dim3(INV_JIT_THREADS), args, 0, (cudaStream_t)stream);
+        if (le != cudaSuccess) {
+            orgym_set_error("specialised rollout kernel launch failed: %s", cudaGetErrorString(le));
+            return ORGYM_E_CUDA;
+        }
+        H->last_rollout_jit = 1;
+    } else if (in->policy == ORGYM_POLICY_MLP) {
         InvMlpPlan M;
         size_t smem = 0;
         if (int rc = inv_mlp_plan(P, in->mlp, A.rslots, wide ? 8 : 4, &M, &smem)) return rc;
@@ -1765,70 +1787,29 @@ extern "C" int orgym_invmgmt_rollout(orgym_handle_t h, uint64_t seed, int64_t en
         else
             launch_mlp_rollout<int>(H, A, M, smem, (cudaStream_t)stream);
         ORGYM_CUDA(cudaGetLastError());
-        if (out->summary_dev) {
-            int rr = orgym_launch_reduce(H->partials, (int)((A.N + ROLL_THREADS - 1) / ROLL_THREADS), out->summary_dev,
-                                         (cudaStream_t)stream);
-            if (rr != ORGYM_OK) return rr;
-        }
-        return ORGYM_OK;
-    }
-    if (jit_mode && !wide && inv_jit_policy_ok(in, A.target_is_int) && !A.reward_traj && !A.final_I && !A.final_B &&
-        !A.action_traj) {
-        cudaKernel_t fn = nullptr;
-        const int jrc = inv_jit_get(H, in->policy == ORGYM_POLICY_BASE_STOCK ? 0 : 1, A.target_int, &fn);
-        if (jrc != ORGYM_OK && jit_mode == 2) return jrc;  // strict: the reason is in orgym_last_error()
-        if (jrc == ORGYM_OK) {
-            InvJitArgs J;
-            memset(&J, 0, sizeof(J));
-            J.N = A.N;
-            J.env_offset = A.env_offset;
-            J.seed = A.seed;
-            J.episode = A.episode;
-            for (int i = 0; i < P.n; i++) J.target[i] = (int32_t)A.target_int[i];
-            J.table = P.dem.table;
-            J.ep_return = A.ep_return;
-            J.stats = A.stats;
-            J.stats32 = A.stats32;
-            J.partials = A.partials;
-            void* args[] = {(void*)&J};
-            const unsigned grid = (unsigned)((A.N + INV_JIT_THREADS - 1) / INV_JIT_THREADS);
-            cudaError_t le = cudaLaunchKernel((const void*)fn, dim3(grid), dim3(INV_JIT_THREADS), args, 0, (cudaStream_t)stream);
-            if (le != cudaSuccess) {
-                orgym_set_error("specialised rollout kernel launch failed: %s", cudaGetErrorString(le));
-                return ORGYM_E_CUDA;
+    } else {
+        const size_t ring = (size_t)A.rslots * ROLL_THREADS * (wide ? 8 : 4);
+        size_t smem = inv_alias_smem(P) + ring * (in->policy == ORGYM_POLICY_BASE_STOCK ? 2 : 1);
+        if (smem > INV_STAGING_SMEM_LIMIT) {  // rings too long for shared memory: caller-owned global scratch, generic kernel
+            if (!in->scratch_dev) {
+                orgym_set_error("lead-time rings (sum of lead times = %d) do not fit in shared memory: pass a scratch_dev buffer "
+                                "of orgym_invmgmt_rollout_scratch_bytes() = %lld bytes", P.sumL,
+                                (long long)orgym_invmgmt_rollout_scratch_bytes(h));
+                return ORGYM_E_INVALID;
             }
-            H->last_rollout_jit = 1;
-            if (out->summary_dev) {
-                int nblocks = (int)grid;
-                int rrc = orgym_launch_reduce(H->partials, nblocks, out->summary_dev, (cudaStream_t)stream);
-                if (rrc != ORGYM_OK) return rrc;
-            }
-            return ORGYM_OK;
+            A.ring_scratch = in->scratch_dev;
+            A.ring_stride = round_up(A.N, ROLL_THREADS);
+            smem = inv_alias_smem(P);
         }
+        if (wide)
+            launch_rollout<long long>(H, A, smem, (cudaStream_t)stream);
+        else
+            launch_rollout<int>(H, A, smem, (cudaStream_t)stream);
+        ORGYM_CUDA(cudaGetLastError());
     }
-    size_t ring = (size_t)A.rslots * ROLL_THREADS * (wide ? 8 : 4);
-    size_t smem = (P.dem.kind == ORGYM_DIST_USER ? 0 : (size_t(8) << P.dem.log2k)) +
-                  ring * (in->policy == ORGYM_POLICY_BASE_STOCK ? 2 : 1);
-    if (smem > 200 * 1024) {  // rings too long for shared memory: caller-owned global scratch, generic kernel (correct, not fast)
-        const int64_t stride = round_up(A.N, ROLL_THREADS);
-        if (!in->scratch_dev) {
-            orgym_set_error("lead-time rings (sum of lead times = %d) do not fit in shared memory: pass a scratch_dev buffer of "
-                            "orgym_invmgmt_rollout_scratch_bytes() = %lld bytes", P.sumL,
-                            (long long)orgym_invmgmt_rollout_scratch_bytes(h));
-            return ORGYM_E_INVALID;
-        }
-        A.ring_scratch = in->scratch_dev;
-        A.ring_stride = stride;
-        smem = P.dem.kind == ORGYM_DIST_USER ? 0 : (size_t(8) << P.dem.log2k);
-    }
-    if (wide)
-        launch_rollout<long long>(H, A, smem, (cudaStream_t)stream);
-    else
-        launch_rollout<int>(H, A, smem, (cudaStream_t)stream);
-    ORGYM_CUDA(cudaGetLastError());
     if (out->summary_dev) {
-        int nblocks = (int)((A.N + ROLL_THREADS - 1) / ROLL_THREADS);
-        int rr = orgym_launch_reduce(H->partials, nblocks, out->summary_dev, (cudaStream_t)stream);
+        int rr = orgym_launch_reduce(H->partials, (int)((A.N + ROLL_THREADS - 1) / ROLL_THREADS), out->summary_dev,
+                                     (cudaStream_t)stream);
         if (rr != ORGYM_OK) return rr;
     }
     return ORGYM_OK;

@@ -37,12 +37,6 @@ std::string lit(double v) {
     snprintf(buf, sizeof(buf), "%a", v);
     return buf;
 }
-int env_int(const char* name, int dflt, int lo, int hi) {
-    const char* v = getenv(name);
-    if (!v) return dflt;
-    const int x = atoi(v);
-    return x < lo || x > hi ? dflt : x;
-}
 
 // integer form of a coefficient: c / 2^qexp (exact by construction of qexp)
 long long coef_int(double c, int qexp) { return (long long)std::ldexp(c, -qexp); }
@@ -54,8 +48,7 @@ void emit_kernel(Src& o, const InvJitSpec& S, const char* name, int policy, int 
     const int n = S.n, T = S.T, K = 1 << S.log2k;
     const bool bs = policy == 0, bl = S.backlog != 0;
     int qexp = 0;
-    const bool fma_ok = env_int("ORGYM_INV_JIT_FMA", 1, 0, 1) != 0;
-    const bool exact = fma_ok && inv_jit_profit_is_exact(S) && inv_jit_quantum(S, &qexp);
+    const bool exact = inv_jit_profit_is_exact(S) && inv_jit_quantum(S, &qexp);
     // integer profit (exact only): sum_j (c_j / Q) * x_j in int64, one conversion per period -- or, when the rewards
     // are undiscounted and even the running sum over all periods provably never rounds, one conversion per episode
     bool disc_ok = true, undiscounted = true;
@@ -64,23 +57,18 @@ void emit_kernel(Src& o, const InvJitSpec& S, const char* name, int policy, int 
         if (S.disc[(size_t)t] != 1.0) undiscounted = false;
         if (!(dq == 0.0 || std::fabs(dq) > 1e-290)) disc_ok = false;  // scaling by Q must stay exact (no subnormals)
     }
-    const bool iprofit = exact && disc_ok && env_int("ORGYM_INV_JIT_INT", 1, 0, 1) != 0;
+    const bool iprofit = exact && disc_ok;
     const bool episode_sum = iprofit && undiscounted && inv_jit_profit_is_exact(S, T);
     const char* W4[4] = {"w.x", "w.y", "w.z", "w.w"};
     const char* A4[4] = {"a4.x", "a4.y", "a4.z", "a4.w"};
     // (random policy) periods re-rolled into a loop over blocks of UNR periods -- see below; the per-period discount
     // factors then come from a constant-memory table (uniform loads)
-    // Block length 8 (4 for short horizons; ORGYM_INV_JIT_RND_UNROLL overrides, 0 = straight-line).  A ring whose lead time
-    // divides the block length keeps compile-time slot indices ((tb + u) mod L = u mod L), the others are shifted by L - 1
-    // register moves per period; a block length that is not a multiple of 4 picks the period's Philox word at run time.
-    // Measured on the default configuration (lead times 3, 5, 10; 2^24 x 30): straight-line 2.78-3.0 ms, blocks of 4
-    // 2.57, 8 2.55, 12 2.56, 10 (two rings static, run-time word) 2.78, 15 3.01 -- the block has to stay small.
-    int UNR = 0;
-    if (!bs) {
-        UNR = T >= 16 ? 8 : (T >= 8 ? 4 : 0);
-        const int forced = env_int("ORGYM_INV_JIT_RND_UNROLL", -1, 0, 32);
-        if (forced >= 0) UNR = (forced > 0 && T >= 2 * forced) ? forced : 0;
-    }
+    // Block length 8 (4 for short horizons, straight-line below 8 periods).  A ring whose lead time divides the block
+    // length keeps compile-time slot indices ((tb + u) mod L = u mod L), the others are shifted by L - 1 register moves
+    // per period.  Measured on the default configuration (lead times 3, 5, 10; 2^24 x 30): straight-line 2.78-3.0 ms,
+    // blocks of 4 2.57, 8 2.55, 12 2.56, 10 (two rings static, run-time Philox word) 2.78, 15 3.01 -- the block has to
+    // stay small.
+    const int UNR = bs ? 0 : (T >= 16 ? 8 : (T >= 8 ? 4 : 0));
     if (UNR > 0 && !(iprofit && episode_sum)) {
         o("__constant__ double c_disc[%d] = {", T);
         for (int t = 0; t < T; t++)
@@ -127,7 +115,6 @@ void emit_kernel(Src& o, const InvJitSpec& S, const char* name, int policy, int 
     bool shift[ORGYM_INV_MAX_STAGES];
     for (int i = 0; i < n; i++) shift[i] = UNR > 0 && S.L[i] > 0 && UNR % S.L[i] != 0;
     const int Tloop = UNR > 0 ? T - T % UNR : 0;
-    const bool dyn_word = UNR > 0 && UNR % 4 != 0;   // the demand word of a period inside the loop is picked at run time
     // emits period t; inside the loop t = tb + u is symbolic and only u is known here
     auto emit_period = [&](int t, int u, bool in_loop) {
         char tx[32], bx[32], dx[48];
@@ -161,13 +148,8 @@ void emit_kernel(Src& o, const InvJitSpec& S, const char* name, int policy, int 
         }
         // demand
         if (S.log2k > 0) {
-            if (in_loop && dyn_word) {
-                o("    if (((tb + %d) & 3) == 0) w = philox_block(key, (unsigned)((tb + %d) >> 2), ep, STREAM_DEMAND, 0u);", u, u);
-                o("    int dl; { const unsigned int wv = pick_word(w, (tb + %d) & 3), pe = tab[wv >> %d];", u, 32 - S.log2k);
-            } else {
-                if (w4 == 0) o("    w = philox_block(key, %s, ep, STREAM_DEMAND, 0u);", bx);
-                o("    int dl; { const unsigned int wv = %s, pe = tab[wv >> %d];", W4[w4], 32 - S.log2k);
-            }
+            if (w4 == 0) o("    w = philox_block(key, %s, ep, STREAM_DEMAND, 0u);", bx);
+            o("    int dl; { const unsigned int wv = %s, pe = tab[wv >> %d];", W4[w4], 32 - S.log2k);
             o("      dl = %d + (int)((((wv << %d) | %uu) < pe) ? (wv >> %d) : (pe & %uu)); }", S.base, S.log2k, (unsigned)(K - 1),
               32 - S.log2k, (unsigned)(K - 1));
         } else {
@@ -407,7 +389,7 @@ std::string inv_jit_source(const InvJitSpec& S) {
     o.s += orgym_jit_inv_args_src();
     o("#define NTHR %d", INV_JIT_THREADS);
     // base-stock keeps only the retailer's state per thread (the rest is folded): room for more resident CTAs
-    const int mb = env_int("ORGYM_INV_JIT_MINBLOCKS", S.policy == 0 ? 8 : 4, 1, 12);
-    emit_kernel(o, S, inv_jit_kernel_name(S.policy), S.policy, mb);
+    // (minimum-CTA sweep in profiles/r02_sweeps.txt)
+    emit_kernel(o, S, inv_jit_kernel_name(S.policy), S.policy, S.policy == 0 ? 8 : 4);
     return o.s;
 }

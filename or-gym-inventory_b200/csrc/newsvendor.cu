@@ -13,12 +13,8 @@
 #include "poisson_mu.cuh"
 
 #define NV_MAXL ORGYM_NV_MAX_LEAD
-#ifndef NV_STEP_MINB
 #define NV_STEP_MINB 8
-#endif
-#ifndef NV_ROLL_MINB
 #define NV_ROLL_MINB 5
-#endif
 
 struct NvDev {
     const double* rcp;  // reciprocal table (orgym_rcp_table)
@@ -875,11 +871,6 @@ extern "C" int orgym_newsvendor_reset(orgym_handle_t h, void* state_dev, int res
     return ORGYM_OK;
 }
 
-static int nv_use_bulk() {
-    const char* v = getenv("ORGYM_NO_BULK");
-    return (v && v[0] == '1') ? 0 : 1;
-}
-
 extern "C" int orgym_newsvendor_step(orgym_handle_t h, void* state_dev, const float* actions_dev,
                                      const int64_t* demand_override_dev, int autoreset_mode, float* obs_dev,
                                      double* reward_dev, uint8_t* terminated_dev, uint8_t* truncated_dev,
@@ -910,7 +901,7 @@ extern "C" int orgym_newsvendor_step(orgym_handle_t h, void* state_dev, const fl
         A.final_obs = info->final_obs_dev;
     }
     A.err = H->base.err_dev;
-    A.use_bulk = nv_use_bulk() && ((uintptr_t)obs_dev % 16 == 0);
+    A.use_bulk = (uintptr_t)obs_dev % 16 == 0;
     size_t smem = (size_t)ORGYM_TILE * (H->dev.obs_dim + 1) * 4;
     orgym_ensure_dyn_smem<nv_step_kernel>(smem);
     nv_step_kernel<<<(unsigned)((A.N + ORGYM_TILE - 1) / ORGYM_TILE), ORGYM_TILE, smem, (cudaStream_t)stream>>>(H->dev, A);

@@ -254,12 +254,14 @@ def test_c_host_example_matches_the_python_host(lib, tmp_path):
     e.close()
 
 
-def test_serial_rollout_specialiser_uses_integer_profit_only_when_provably_exact(lib, monkeypatch):
+def test_serial_rollout_specialiser_uses_integer_profit_only_when_provably_exact_and_scalable(lib):
     """Defaults: float32 coefficients on a 2^-29 grid and small integers -> no float64 operation of the reference's profit
     can round -> the generator emits integer multiply-adds on coefficient / 2^-29 (and, the rewards being undiscounted
     and the 30-period running sum exact as well, converts once per episode).  With discounting: one conversion per
-    period.  Capacities of a million push the bound past 2^52 * quantum -> it must keep the reference's operation order
-    (4 products + 3 subtractions per stage, sequential sum)."""
+    period.  A discount so small that alpha**29 * 2^-29 is below the generator's 1e-290 guard keeps the exact profit
+    but not the integer scaling: one fused multiply-add chain.  Capacities of a million push the bound past
+    2^52 * quantum -> it must keep the reference's operation order (4 products + 3 subtractions per stage, sequential
+    sum)."""
     rin = None
 
     def source(backlog=True, **kw):
@@ -277,10 +279,8 @@ def test_serial_rollout_specialiser_uses_integer_profit_only_when_provably_exact
     disc = source()                                                                                # default alpha = 0.97
     assert "long long acc" not in disc and "(__longlong_as_double(pa + 0x4338000000000000LL) - 0x1.8p52);" in disc
     assert "tm_0" not in disc
-    monkeypatch.setenv("ORGYM_INV_JIT_INT", "0")
-    fused = source()
+    fused = source(alpha=1e-10)
     assert "fma(" in fused and "tm_0" not in fused and "long long pa" not in fused
-    monkeypatch.delenv("ORGYM_INV_JIT_INT")
     big = source(c=[1_000_000, 2_000_000, 2_300_000])
     assert "fma(" not in big and "long long pa" not in big and "tm_0" in big and "pr = pr + tm_3;" in big
 
