@@ -299,6 +299,19 @@ int orgym_newsvendor_export_params(orgym_handle_t h, const void* state_dev, doub
 #define ORGYM_NV_POLICY_ORDER_UP_TO 1 /* benchmark_newsvendor.py:97-111;   param[0] = safety factor */
 #define ORGYM_NV_POLICY_CLASSIC 2     /* benchmark_newsvendor.py:113-161 (k_vs_h); param[0] = safety factor */
 #define ORGYM_NV_POLICY_SS 3          /* benchmark_newsvendor_sb3_rllib.py:363-371; param[0] = S buffer factor */
+#define ORGYM_NV_POLICY_MLP 4         /* actor network evaluated on the device, in->mlp */
+
+/* ORGYM_NV_POLICY_MLP: a trained actor network (orgym_mlp_t, width[0] = lead_time + 5, width[num_layers] = 1), e.g. a
+ * stable-baselines3 MlpPolicy as benchmark_newsvendor.py:164 wraps it, evaluated inside the fused rollout.  Per period,
+ * for each env:
+ *   x    = the float32 observation step() returns: price, cost, h, k, mu, then the pipeline oldest first (:206-208)
+ *   h_l, y = exactly the serial env's contract (orgym_mlp_t above): acc = b, then fmaf ascending in k; accurate tanhf
+ *          or NaN-keeping ReLU; no activation after the last Linear
+ *   a    = NaN if y is NaN, else min(max(y, 0f), (float)max_order_quantity)   (SB3 predict's np.clip to the Box, float32)
+ * a then takes the env's own action rule, exactly like an ORGYM_NV_POLICY_ACTIONS action (.item(), np.clip in float64,
+ * :131-132); action_traj_dev records a.  A NaN action places no order when lead_time > 0; with lead_time = 0 it is also
+ * the stock on hand (:136-139), so the reward is NaN, as in the reference.  Results are a pure function of (weights,
+ * seed, global env id, episode): independent of batch size and env_offset sharding. */
 
 typedef struct {
     int32_t policy;
@@ -308,6 +321,11 @@ typedef struct {
     const int64_t* demand_dev;
     int64_t dem_stride_env, dem_stride_t;
     const double* fixed_params_dev; /* float64[N,5] or NULL */
+    /* HOST pointer, read only when policy == ORGYM_NV_POLICY_MLP.  ORGYM_E_INVALID for a missing or malformed network
+     * (layer count, widths outside 1..ORGYM_MLP_MAX_WIDTH, width[0] != lead_time + 5, width[num_layers] != 1, null
+     * weights); ORGYM_E_UNSUPPORTED when the weights, activations, observation tile and Poisson CDF tile of one CTA do
+     * not fit in shared memory. */
+    const orgym_mlp_t* mlp;
 } orgym_newsvendor_rollout_in_t;
 
 typedef struct {

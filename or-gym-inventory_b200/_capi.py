@@ -75,7 +75,8 @@ class NvInfo(C.Structure):
 class NvRolloutIn(C.Structure):
     _fields_ = [("policy", C.c_int32), ("param", C.c_double * 4), ("actions", C.c_void_p),
                 ("act_stride_env", C.c_int64), ("act_stride_t", C.c_int64), ("demand", C.c_void_p),
-                ("dem_stride_env", C.c_int64), ("dem_stride_t", C.c_int64), ("fixed_params", C.c_void_p)]
+                ("dem_stride_env", C.c_int64), ("dem_stride_t", C.c_int64), ("fixed_params", C.c_void_p),
+                ("mlp", C.POINTER(Mlp))]
 
 
 class NvRolloutOut(C.Structure):

@@ -20,6 +20,7 @@
 
 #include "common.cuh"
 #include "launch_util.cuh"
+#include "mlp.cuh"
 #include <type_traits>
 
 #include "invmgmt_jit.cuh"
@@ -811,13 +812,8 @@ __global__ void __launch_bounds__(ROLL_THREADS) inv_rollout_kernel(const __grid_
 // One CTA = 128 consecutive envs (one row of the partial sums, like inv_rollout_kernel), run as 128/E sub-tiles of E
 // envs one after the other; weights and biases are staged in shared memory once per CTA.  Thread tid < E owns env
 // e0 + tid of the current sub-tile (integer state in registers, lead-time ring in shared memory).  Per period the whole
-// CTA evaluates the network on the sub-tile's observations as a register-tiled SGEMM: activations are feature-major
-// [feature][env] float32 tiles, each thread computes blocks of MLP_TE envs x MLP_TN neurons, so one 16-byte load of
-// activations and one of weights feed 16 FMAs.  The observation tile itself is the request window (shifted in place).
-#define MLP_THREADS 256
-#define MLP_TE 4
-#define MLP_TN 4
-
+// CTA evaluates the network on the sub-tile's observations (mlp.cuh: register-tiled SGEMM on feature-major tiles).  The
+// observation tile itself is the request window (shifted in place).
 struct InvMlpPlan {
     int L, act, E, log2E;
     int K[ORGYM_MLP_MAX_LAYERS + 1];   // widths
@@ -828,48 +824,6 @@ struct InvMlpPlan {
     int w_off[ORGYM_MLP_MAX_LAYERS], b_off[ORGYM_MLP_MAX_LAYERS], obs_off, buf_off[2], y_off;
     int fbase, ring_off;
 };
-
-__device__ __forceinline__ float mlp_act(float x, int act) {
-    // accurate tanhf (tanh.approx.f32 has ~2^-11 relative error: far more truncated actions would flip); ReLU keeps NaN
-    return act == ORGYM_MLP_TANH ? tanhf(x) : (x < 0.f ? 0.f : x);
-}
-
-// out[n][e] = act(b[n] + sum_k Wt[k][n] in[k][e]) for the E envs of the tile; each output accumulates in k order
-__device__ __forceinline__ void mlp_hidden_layer(const float* __restrict__ in, float* __restrict__ out,
-                                                 const float* __restrict__ Wt, const float* __restrict__ bias, int K,
-                                                 int Np, int E, int log2E, int act) {
-    const int egs = E / MLP_TE, log2egs = log2E - 2;
-    const int ntile = egs * (Np / MLP_TN);
-    for (int tile = threadIdx.x; tile < ntile; tile += MLP_THREADS) {
-        const int eg = tile & (egs - 1), ng = tile >> log2egs;
-        const float* xp = in + eg * MLP_TE;
-        const float* wp = Wt + ng * MLP_TN;
-        const float4 bv = *reinterpret_cast<const float4*>(bias + ng * MLP_TN);
-        float acc[MLP_TE][MLP_TN];
-#pragma unroll
-        for (int i = 0; i < MLP_TE; i++) {
-            acc[i][0] = bv.x;
-            acc[i][1] = bv.y;
-            acc[i][2] = bv.z;
-            acc[i][3] = bv.w;
-        }
-#pragma unroll 4
-        for (int k = 0; k < K; k++) {
-            const float4 x4 = *reinterpret_cast<const float4*>(xp + k * E);
-            const float4 w4 = *reinterpret_cast<const float4*>(wp + k * Np);
-            const float x[4] = {x4.x, x4.y, x4.z, x4.w}, w[4] = {w4.x, w4.y, w4.z, w4.w};
-#pragma unroll
-            for (int i = 0; i < MLP_TE; i++)
-#pragma unroll
-                for (int j = 0; j < MLP_TN; j++) acc[i][j] = __fmaf_rn(w[j], x[i], acc[i][j]);
-        }
-#pragma unroll
-        for (int j = 0; j < MLP_TN; j++)
-            *reinterpret_cast<float4*>(out + (ng * MLP_TN + j) * E + eg * MLP_TE) =
-                make_float4(mlp_act(acc[0][j], act), mlp_act(acc[1][j], act), mlp_act(acc[2][j], act),
-                            mlp_act(acc[3][j], act));
-    }
-}
 
 template <int NS, bool EXACT, typename S>
 __global__ void __launch_bounds__(MLP_THREADS, (EXACT && NS <= 4 && sizeof(S) == 4) ? 3 : 2) inv_mlp_rollout_kernel(const __grid_constant__ InvDev P,
@@ -888,24 +842,7 @@ __global__ void __launch_bounds__(MLP_THREADS, (EXACT && NS <= 4 && sizeof(S) ==
     const int K = (P.dem.kind == ORGYM_DIST_USER) ? 0 : (1 << P.dem.log2k);
     for (int i = tid; i < K; i += MLP_THREADS) tab[i] = P.dem.table[i];
     // weights: hidden layers transposed to [k][Np] (zero-padded columns), the last layer as given ([n][K] row-major)
-    for (int l = 0; l < L; l++) {
-        const int Kl = M.K[l], Nl = M.K[l + 1];
-        const float* Wg = M.W[l];
-        const float* bg = M.b[l];
-        float* Ws = fs + M.w_off[l];
-        float* bs = fs + M.b_off[l];
-        if (l < L - 1) {
-            const int Np = M.Np[l];
-            for (int idx = tid; idx < Kl * Np; idx += MLP_THREADS) {
-                const int k = idx / Np, j = idx - k * Np;
-                Ws[idx] = j < Nl ? Wg[(size_t)j * Kl + k] : 0.f;
-            }
-            for (int j = tid; j < Np; j += MLP_THREADS) bs[j] = (j < Nl && bg) ? bg[j] : 0.f;
-        } else {
-            for (int idx = tid; idx < Kl * Nl; idx += MLP_THREADS) Ws[idx] = Wg[idx];
-            for (int j = tid; j < Nl; j += MLP_THREADS) bs[j] = bg ? bg[j] : 0.f;
-        }
-    }
+    mlp_stage_weights(M, fs);
     const int Lm = P.lt_max, od = P.obs_dim;
     const int Klast = M.K[L - 1];
     const float* Wlast = fs + M.w_off[L - 1];
@@ -1119,43 +1056,25 @@ static void launch_mlp_rollout(const InvHandle* H, const InvRolloutArgs& A, cons
 
 // Checks an orgym_mlp_t against the handle (ORGYM_E_INVALID) and lays out one CTA's shared memory for it: the largest
 // sub-tile of E in {64, 32} envs whose working set fits (ORGYM_E_UNSUPPORTED, with the sizes, when none does).
-#define MLP_SMEM_BUDGET (227 * 1024 - 1024)  // sm_100 opt-in limit per block, less the static partial-sum rows
 static int inv_mlp_plan(const InvDev& P, const orgym_mlp_t* mlp, int rslots, size_t ring_elem, InvMlpPlan* M,
                         size_t* smem_out) {
     ORGYM_REQUIRE(mlp, "policy ORGYM_POLICY_MLP needs in->mlp");
-    const int L = mlp->num_layers;
-    ORGYM_REQUIRE(L >= 1 && L <= ORGYM_MLP_MAX_LAYERS, "mlp: num_layers = %d, must be 1..%d", L, ORGYM_MLP_MAX_LAYERS);
-    ORGYM_REQUIRE(L == 1 || mlp->activation == ORGYM_MLP_TANH || mlp->activation == ORGYM_MLP_RELU,
-                  "mlp: activation %d is neither ORGYM_MLP_TANH nor ORGYM_MLP_RELU", mlp->activation);
-    for (int l = 0; l <= L; l++)
-        ORGYM_REQUIRE(mlp->width[l] >= 1 && mlp->width[l] <= ORGYM_MLP_MAX_WIDTH, "mlp: width[%d] = %d outside 1..%d", l,
-                      mlp->width[l], ORGYM_MLP_MAX_WIDTH);
-    ORGYM_REQUIRE(mlp->width[0] == P.obs_dim, "mlp: width[0] = %d differs from obs_dim = %d", mlp->width[0], P.obs_dim);
-    ORGYM_REQUIRE(mlp->width[L] == P.n, "mlp: width[%d] = %d differs from the action dimension m-1 = %d", L, mlp->width[L],
-                  P.n);
-    for (int l = 0; l < L; l++) ORGYM_REQUIRE(mlp->weight_dev[l], "mlp: weight_dev[%d] is NULL", l);
+    MlpNet net;
+    if (int rc = mlp_net_plan(mlp, P.obs_dim, P.n, "the action dimension m-1", &net)) return rc;
+    const int L = net.L;
     memset(M, 0, sizeof(*M));
     M->L = L;
-    M->act = L > 1 ? mlp->activation : ORGYM_MLP_TANH;
-    int hmax = 0;
-    for (int l = 0; l <= L; l++) M->K[l] = mlp->width[l];
+    M->act = net.act;
+    for (int l = 0; l <= L; l++) M->K[l] = net.K[l];
     for (int l = 0; l < L; l++) {
-        M->W[l] = mlp->weight_dev[l];
-        M->b[l] = mlp->bias_dev[l];
-        if (l < L - 1) {
-            M->Np[l] = (int)round_up(M->K[l + 1], MLP_TN);
-            hmax = std::max(hmax, M->Np[l]);
-        }
+        M->W[l] = net.W[l];
+        M->b[l] = net.b[l];
+        M->Np[l] = net.Np[l];
+        M->w_off[l] = net.w_off[l];
+        M->b_off[l] = net.b_off[l];
     }
     auto a4 = [](int x) { return (int)round_up(x, 4); };  // float offsets stay 16-byte aligned
-    int f = 0;
-    for (int l = 0; l < L; l++) {
-        M->w_off[l] = f;
-        f += a4(M->K[l] * (l < L - 1 ? M->Np[l] : M->K[l + 1]));
-        M->b_off[l] = f;
-        f += a4(l < L - 1 ? M->Np[l] : M->K[l + 1]);
-    }
-    const int wfloats = f;
+    const int wfloats = net.wfloats, hmax = net.hmax;
     const size_t tab = inv_alias_smem(P);
     const int nbuf = L >= 3 ? 2 : (L == 2 ? 1 : 0);
     size_t smem = 0;

@@ -4,12 +4,14 @@
 //   nv_step_kernel     one period (:125-204) + observation (:206-208)
 //   nv_rollout_kernel  fused reset + step_limit periods with on-device drivers (order-up-to, classic newsvendor,
 //                      (s,S)) and per-env Poisson demand (PTRS / inversion)
+//   nv_mlp_rollout_kernel  the same fused rollout with an MLP actor evaluated on the device every period
 //
 // The reward is a chain of mixed float32 / float64 / Python-float operations whose precision depends on which
 // branch produced each operand (NumPy >= 2 promotion rules); `Sc` carries the operand kind so the chain is
 // reproduced bit for bit.  Pipeline state is float32 like the reference's `state` vector.
 #include "common.cuh"
 #include "launch_util.cuh"
+#include "mlp.cuh"
 #include "poisson_mu.cuh"
 
 #define NV_MAXL ORGYM_NV_MAX_LEAD
@@ -601,6 +603,20 @@ __device__ __forceinline__ double nv_policy_level(const NvDev& P, int policy, do
     return nv_level_finish(policy, poisson_ppf_dev(q, mu, P.rcp));
 }
 
+// demand of period t of one env in a fused rollout: replayed, PTRS (large means), or the alias table plus the small-table
+// inversion of the Poisson remainder with one Philox block per two periods (the same words as poisson_mu).  pcdf is the
+// env's column of the remainder's CDF tile ([k][env], stride pstride); dw carries the block from even to odd periods.
+__device__ __forceinline__ long long nv_roll_demand(const NvDev& P, const NvRolloutArgs& A, const NvParams& q,
+                                                    const PoisSplit& ps, uint64_t key, int64_t e, bool valid, int t,
+                                                    uint4& dw, const double* pcdf, int pstride) {
+    if (A.demand) return valid ? A.demand[e * A.d_se + (int64_t)t * A.d_st] : 0;
+    if (ps.i0 < 0) return poisson_ptrs(q.mu, key, A.episode, t);
+    if ((t & 1) == 0) dw = philox_block(key, (uint32_t)t >> 1, A.episode, STREAM_POISSON_TAB, 0);
+    const uint32_t wa = (t & 1) ? dw.z : dw.x, wi = (t & 1) ? dw.w : dw.y;
+    return poisson_tab_alias(P.pt, ps, wa) +
+           poisson_small_lookup(((double)wi + 0.5) * (1.0 / 4294967296.0), pcdf, pstride, ps.r, ps.p0, P.rcp);
+}
+
 __device__ __forceinline__ float clipf(float q, float hi) { return q < 0.0f ? 0.0f : (q > hi ? hi : q); }
 
 // LT > 0: the lead time is the compile-time constant LT (1..7): the pipeline lives in LT registers, summed and shifted
@@ -665,17 +681,7 @@ __global__ void __launch_bounds__(NV_ROLL_THREADS, NV_ROLL_MINB) nv_rollout_kern
             x = x > (double)hi ? (double)hi : x;
             act = (float)x;
         }
-        long long d;
-        if (A.demand)
-            d = valid ? A.demand[e * A.d_se + (int64_t)t * A.d_st] : 0;
-        else if (ps.i0 < 0)
-            d = poisson_ptrs(q.mu, key, A.episode, t);
-        else {  // one Philox block per two periods (same words as poisson_mu)
-            if ((t & 1) == 0) dw = philox_block(key, (uint32_t)t >> 1, A.episode, STREAM_POISSON_TAB, 0);
-            const uint32_t wa = (t & 1) ? dw.z : dw.x, wi = (t & 1) ? dw.w : dw.y;
-            d = poisson_tab_alias(P.pt, ps, wa) +
-                poisson_small_lookup(((double)wi + 0.5) * (1.0 / 4294967296.0), pcdf + tid, NV_ROLL_THREADS, ps.r, ps.p0, P.rcp);
-        }
+        const long long d = nv_roll_demand(P, A, q, ps, key, e, valid, t, dw, pcdf + tid, NV_ROLL_THREADS);
         float oq;
         double su, ex, sh;
         double r;
@@ -788,6 +794,167 @@ __global__ void __launch_bounds__(256, 4) nv_level_kernel(const __grid_constant_
     } else
         q = nv_draw_params(P, A.seed + (uint64_t)(A.env_offset + e), A.episode);
     A.level_out[e] = nv_policy_level(P, A.policy, A.param0, P.L, (float)q.h, (float)q.k, (float)q.mu);
+}
+
+// ---- fused rollout driven by an MLP actor (ORGYM_NV_POLICY_MLP) -----------------------------------------------------
+// One CTA of MLP_THREADS threads = 128 consecutive envs (one row of the partial sums, like nv_rollout_kernel), run as 128/E
+// sub-tiles of E envs one after the other; weights and biases are staged in shared memory once per CTA (mlp.cuh).
+// Thread tid < E owns env e0 + tid of the current sub-tile: its parameters, demand sampler constants, Philox words and
+// accumulators live in its registers, the CDF of its Poisson remainder in column tid of a [ORGYM_PT_CDF][E] tile.
+// The float32 observation tile [obs_dim][E] is the network's input and the env's pipeline at once: rows 0-4 hold
+// price, cost, h, k, mu for the episode, rows 5.. the pipeline oldest first, shifted left and appended in place.
+// Per period the whole CTA runs the hidden layers (one barrier each); the owner threads then evaluate the single output
+// (K ascending FMAs on their own column), take the period through the env's own device functions and append the order.
+struct NvMlpPlan {
+    MlpNet net;
+    int E, log2E;
+    int obs_off, buf_off[2];  // float offsets in dynamic shared memory (the weights start at 0)
+    int pcdf_off;             // byte offset of the Poisson-remainder CDF tile
+};
+
+__global__ void __launch_bounds__(MLP_THREADS, 2) nv_mlp_rollout_kernel(const __grid_constant__ NvDev P,
+                                                                       const __grid_constant__ NvRolloutArgs A,
+                                                                       const __grid_constant__ NvMlpPlan M) {
+    static_assert(MLP_THREADS >= NV_ROLL_THREADS, "one CTA covers a partial-sum row");
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ double red[NV_ROLL_THREADS / 32][7];
+    const int tid = threadIdx.x, E = M.E, NL = M.net.L, L = P.L, od = P.obs_dim;
+    float* fs = (float*)smem;
+    float* obs = fs + M.obs_off;
+    double* pcdf = (double*)(smem + M.pcdf_off) + tid;
+    mlp_stage_weights(M.net, fs);
+    const int Klast = M.net.K[NL - 1];
+    const float* Wlast = fs + M.net.w_off[NL - 1];
+    const float* blast = fs + M.net.b_off[NL - 1];
+    const float* hin = NL == 1 ? obs : fs + M.buf_off[(NL - 2) & 1];  // input of the last layer
+    const float hi = (float)P.max_q;
+    const bool owner = tid < E;
+    const int nsub = NV_ROLL_THREADS / E;
+    for (int sub = 0; sub < nsub; sub++) {
+        const int64_t e0 = (int64_t)blockIdx.x * NV_ROLL_THREADS + (int64_t)sub * E;
+        const int64_t e = e0 + tid;
+        const bool valid = owner && e < A.N;
+        if (e0 >= A.N) {  // CTA-uniform: the sums of the missing warps are zero, like idle lanes of nv_rollout_kernel
+            if (tid < 7 * (E / 32)) red[sub * (E / 32) + tid / 7][tid % 7] = 0.0;
+            continue;
+        }
+        const uint64_t key = A.seed + (uint64_t)(A.env_offset + e);
+        NvParams q = {0.0, 0.0, 0.0, 0.0, 0.0};
+        NvPar32 qf = {0.f, 0.f, 0.f, 0.f};
+        PoisSplit ps;
+        uint4 dw = make_uint4(0, 0, 0, 0);
+        double ret = 0.0, s_sales = 0.0, s_dem = 0.0, s_lost = 0.0, s_ex = 0.0;
+        if (owner) {
+            if (A.fixed && valid) {
+                q.price = A.fixed[e * 5 + 0]; q.cost = A.fixed[e * 5 + 1]; q.h = A.fixed[e * 5 + 2];
+                q.k = A.fixed[e * 5 + 3]; q.mu = A.fixed[e * 5 + 4];
+            } else
+                q = nv_draw_params(P, key, A.episode);
+            qf = {(float)q.price, (float)q.cost, (float)q.h, (float)q.k};
+            ps = poisson_split(P.pt, q.mu);
+            if (ps.i0 >= 0 && !A.demand) poisson_small_table(ps.r, ps.p0, P.rcp, pcdf, E);
+            // first observation [price, cost, h, k, mu, 0 ...] (:115, :122)
+            obs[0 * E + tid] = (float)q.price; obs[1 * E + tid] = (float)q.cost; obs[2 * E + tid] = (float)q.h;
+            obs[3 * E + tid] = (float)q.k; obs[4 * E + tid] = (float)q.mu;
+            for (int j = 0; j < L; j++) obs[(5 + j) * E + tid] = 0.0f;
+        }
+        __syncthreads();
+        for (int t = 0; t < P.T; t++) {
+            const float* in = obs;
+            for (int l = 0; l < NL - 1; l++) {
+                float* out = fs + M.buf_off[l & 1];
+                mlp_hidden_layer(in, out, fs + M.net.w_off[l], fs + M.net.b_off[l], M.net.K[l], M.net.Np[l], E, M.log2E,
+                                 M.net.act);
+                __syncthreads();
+                in = out;
+            }
+            if (owner) {
+                float y = blast[0];  // last layer: acc = b, then K ascending FMAs, no activation
+                for (int k = 0; k < Klast; k++) y = __fmaf_rn(Wlast[k], hin[k * E + tid], y);
+                float act = y > 0.0f ? y : 0.0f;  // np.clip to the action Box in float32, NaN kept
+                act = act < hi ? act : hi;
+                act = y != y ? y : act;
+                const long long d = nv_roll_demand(P, A, q, ps, key, e, valid, t, dw, pcdf, E);
+                const float psum = nv_pipe_sum(L, [&](int j) { return obs[(5 + j) * E + tid]; });
+                const float pipe0 = L > 0 ? obs[5 * E + tid] : 0.0f;
+                float oq;
+                double su, ex, sh;
+                double r;
+                if (L > 0)
+                    r = nv_period_lt(P, q, qf, act, d, pipe0, psum, &oq, nullptr, &su, &ex, &sh);
+                else
+                    r = nv_period(P, q, act, d, pipe0, psum, &oq, nullptr, &su, &ex, &sh);
+                ret += r;
+                s_sales += su; s_dem += (double)d; s_lost += sh; s_ex += ex;
+                if (valid && A.reward_traj) A.reward_traj[e * P.T + t] = r;
+                if (valid && A.action_traj) A.action_traj[e * P.T + t] = act;
+                for (int j = 0; j < L; j++)  // shift left, append the order placed (:177-179)
+                    obs[(5 + j) * E + tid] = j + 1 < L ? obs[(6 + j) * E + tid] : oq;
+            }
+            __syncthreads();
+        }
+        if (valid) {
+            if (A.ep_return) A.ep_return[e] = ret;
+            if (A.stats) {
+                A.stats[e * 4 + 0] = s_sales; A.stats[e * 4 + 1] = s_dem; A.stats[e * 4 + 2] = s_lost; A.stats[e * 4 + 3] = s_ex;
+            }
+            if (A.final_obs)
+                for (int z = 0; z < od; z++) A.final_obs[e * od + z] = obs[z * E + tid];
+        }
+        if (A.partials && owner) {  // warp of 32 consecutive envs: the xor tree of nv_rollout_kernel
+            const double v[7] = {valid ? 1.0 : 0.0, valid ? ret : 0.0, valid ? ret * ret : 0.0, valid ? s_sales : 0.0,
+                                 valid ? s_dem : 0.0, valid ? s_lost : 0.0, valid ? s_ex : 0.0};
+#pragma unroll
+            for (int z = 0; z < 7; z++) {
+                double x = v[z];
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+                if ((tid & 31) == 0) red[sub * (E / 32) + (tid >> 5)][z] = x;
+            }
+        }
+    }
+    if (A.partials) {
+        __syncthreads();
+        if (tid < 7) {  // the four warps in order, as nv_rollout_kernel
+            double x = 0.0;
+            for (int wv = 0; wv < NV_ROLL_THREADS / 32; wv++) x += red[wv][tid];
+            A.partials[(size_t)blockIdx.x * 8 + tid] = x;
+        }
+    }
+}
+
+// Checks an orgym_mlp_t against the handle (ORGYM_E_INVALID) and lays out one CTA's shared memory for it: the largest
+// sub-tile of E in {64, 32} envs whose working set fits (ORGYM_E_UNSUPPORTED, with the sizes, when none does).
+static int nv_mlp_plan(const NvDev& P, const orgym_mlp_t* mlp, NvMlpPlan* M, size_t* smem_out) {
+    ORGYM_REQUIRE(mlp, "policy ORGYM_NV_POLICY_MLP needs in->mlp");
+    memset(M, 0, sizeof(*M));
+    if (int rc = mlp_net_plan(mlp, P.obs_dim, 1, "the action dimension", &M->net)) return rc;
+    const int L = M->net.L, hmax = M->net.hmax;
+    const int nbuf = L >= 3 ? 2 : (L == 2 ? 1 : 0);
+    size_t smem = 0;
+    for (int E = 64; E >= 32; E /= 2) {
+        int g = M->net.wfloats;
+        M->obs_off = g;
+        g += P.obs_dim * E;
+        M->buf_off[0] = g;
+        g += nbuf >= 1 ? hmax * E : 0;
+        M->buf_off[1] = g;
+        g += nbuf >= 2 ? hmax * E : 0;
+        M->pcdf_off = (int)round_up((int64_t)g * 4, 16);
+        smem = (size_t)M->pcdf_off + (size_t)ORGYM_PT_CDF * E * sizeof(double);
+        M->E = E;
+        M->log2E = E == 64 ? 6 : 5;
+        if (smem <= MLP_SMEM_BUDGET) break;
+    }
+    if (smem > MLP_SMEM_BUDGET) {
+        orgym_set_error("mlp: one CTA of 32 envs needs %zu bytes of shared memory (weights and biases %d floats, observation "
+                        "tile %d x 32, %d activation tile(s) %d x 32, Poisson CDF tile %d x 32 doubles); this build's limit "
+                        "is %d",
+                        smem, M->net.wfloats, P.obs_dim, nbuf, hmax, ORGYM_PT_CDF, MLP_SMEM_BUDGET);
+        return ORGYM_E_UNSUPPORTED;
+    }
+    *smem_out = smem;
+    return ORGYM_OK;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -927,7 +1094,7 @@ extern "C" int orgym_newsvendor_rollout(orgym_handle_t h, uint64_t seed, int64_t
     if (orgym_check_handle(h, FAM_NEWSVENDOR)) return ORGYM_E_INVALID;
     NvHandle* H = (NvHandle*)h;
     ORGYM_REQUIRE(in && out, "null argument");
-    ORGYM_REQUIRE(in->policy >= 0 && in->policy <= 3, "unknown policy %d", in->policy);
+    ORGYM_REQUIRE(in->policy >= 0 && in->policy <= ORGYM_NV_POLICY_MLP, "unknown policy %d", in->policy);
     ORGYM_REQUIRE(in->policy != ORGYM_NV_POLICY_ACTIONS || in->actions_dev, "policy ACTIONS needs actions_dev");
     DeviceGuard g(H->base.device);
     NvRolloutArgs A;
@@ -966,12 +1133,18 @@ extern "C" int orgym_newsvendor_rollout(orgym_handle_t h, uint64_t seed, int64_t
         orgym_ensure_dyn_smem<nv_rollout_kernel<LTV>>(16);                                         \
         nv_rollout_kernel<LTV><<<nblocks, NV_ROLL_THREADS, 16, (cudaStream_t)stream>>>(H->dev, A); \
         break;
-    switch (H->dev.L) {  // lead times 1..7: register-resident pipeline (see the kernel)
-        NV_ROLL_CASE(1) NV_ROLL_CASE(2) NV_ROLL_CASE(3) NV_ROLL_CASE(4) NV_ROLL_CASE(5) NV_ROLL_CASE(6) NV_ROLL_CASE(7)
-        default:
-            orgym_ensure_dyn_smem<nv_rollout_kernel<0>>(smem);  // + 17 KB static
-            nv_rollout_kernel<0><<<nblocks, NV_ROLL_THREADS, smem, (cudaStream_t)stream>>>(H->dev, A);
-    }
+    if (in->policy == ORGYM_NV_POLICY_MLP) {
+        NvMlpPlan M;
+        if (int rc = nv_mlp_plan(H->dev, in->mlp, &M, &smem)) return rc;
+        orgym_ensure_dyn_smem<nv_mlp_rollout_kernel>(smem);
+        nv_mlp_rollout_kernel<<<nblocks, MLP_THREADS, smem, (cudaStream_t)stream>>>(H->dev, A, M);
+    } else
+        switch (H->dev.L) {  // lead times 1..7: register-resident pipeline (see the kernel)
+            NV_ROLL_CASE(1) NV_ROLL_CASE(2) NV_ROLL_CASE(3) NV_ROLL_CASE(4) NV_ROLL_CASE(5) NV_ROLL_CASE(6) NV_ROLL_CASE(7)
+            default:
+                orgym_ensure_dyn_smem<nv_rollout_kernel<0>>(smem);  // + 17 KB static
+                nv_rollout_kernel<0><<<nblocks, NV_ROLL_THREADS, smem, (cudaStream_t)stream>>>(H->dev, A);
+        }
 #undef NV_ROLL_CASE
     ORGYM_CUDA(cudaGetLastError());
     if (out->summary_dev) {

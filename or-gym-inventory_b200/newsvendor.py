@@ -9,10 +9,12 @@ from typing import Dict, Optional
 import numpy as np
 
 from . import _capi
+from .mlp import pack_mlp
 from .spaces import Box
 from .vector import BatchedEnv, _AUTORESET, _torch
 
 POLICIES = {"actions": 0, "order_up_to": 1, "classic": 2, "sS": 3}
+POLICY_MLP = 4
 
 
 class NewsvendorParams:
@@ -152,15 +154,24 @@ class NewsvendorEnv(BatchedEnv):
     def rollout(self, policy="classic", *, seed=None, episode=0, safety_factor=1.0, S_factor=1.2, actions=None,
                 demand=None, fixed_params=None, time_major=False, want=("ep_return", "stats", "summary"), buffer_set=0):
         """Fused reset + step_limit periods (K1/K2).  policy: 'order_up_to' | 'classic' | 'sS' | 'actions'
-        (float32 [N,T] or [T,N]).  Returns device tensors: ep_return f64[N], stats f64[N,4] (sum sales units,
-        demand, lost units, excess units), summary f64[8]; on request reward_traj, action_traj, final_obs."""
+        (float32 [N,T] or [T,N]) | an actor network -- a torch.nn.Sequential (Linear, Tanh|ReLU, ..., Linear) or an
+        SB3 ActorCriticPolicy (e.g. `model.policy` of a trained PPO) -- evaluated on the device every period on the
+        observation step() would return, its output clipped to [0, max_order_quantity] like SB3's deterministic
+        predict.  Returns device tensors: ep_return f64[N], stats f64[N,4] (sum sales units, demand, lost units,
+        excess units), summary f64[8]; on request reward_traj, action_traj, final_obs."""
         torch = _torch()
         P = self.params
         N, T = self.num_envs, int(P.step_limit)
         rin = _capi.NvRolloutIn()
         keep = []
-        rin.policy = POLICIES[policy]
-        rin.param[0] = float(S_factor if policy == "sS" else safety_factor)
+        if isinstance(policy, str):
+            rin.policy = POLICIES[policy]
+            rin.param[0] = float(S_factor if policy == "sS" else safety_factor)
+        else:
+            mlp, tensors = pack_mlp(policy, P.obs_dim, 1, self.device)
+            keep += [mlp, tensors]
+            rin.policy = POLICY_MLP
+            rin.mlp = C.pointer(mlp)
         if policy == "actions":
             a = self._to_dev(actions, torch.float32, (T, N) if time_major else (N, T))
             keep.append(a)
