@@ -368,10 +368,21 @@ __global__ void __launch_bounds__(256) orgym_reduce_partials_kernel(const double
     const int rpb = (nrows + nb - 1) / nb;
     const int r0 = blockIdx.x * rpb, r1 = min(nrows, r0 + rpb);
     double v[7] = {0, 0, 0, 0, 0, 0, 0};
-    for (int r = r0 + tid; r < r1; r += 256) {
-        const double4 a = *reinterpret_cast<const double4*>(partials + (size_t)r * 8);
-        const double4 b = *reinterpret_cast<const double4*>(partials + (size_t)r * 8 + 4);
-        v[0] += a.x; v[1] += a.y; v[2] += a.z; v[3] += a.w; v[4] += b.x; v[5] += b.y; v[6] += b.z;
+    // a thread's rows r, r + 256, ... are summed in that order; the loads of 4 of them are issued before the first add
+    for (int r = r0 + tid; r < r1; r += 4 * 256) {
+        double4 a[4], b[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++)
+            if (r + k * 256 < r1) {
+                a[k] = *reinterpret_cast<const double4*>(partials + (size_t)(r + k * 256) * 8);
+                b[k] = *reinterpret_cast<const double4*>(partials + (size_t)(r + k * 256) * 8 + 4);
+            }
+#pragma unroll
+        for (int k = 0; k < 4; k++)
+            if (r + k * 256 < r1) {
+                v[0] += a[k].x; v[1] += a[k].y; v[2] += a[k].z; v[3] += a[k].w;
+                v[4] += b[k].x; v[5] += b[k].y; v[6] += b[k].z;
+            }
     }
     __shared__ double red[8][7];
     __shared__ int is_last;
@@ -392,12 +403,16 @@ __global__ void __launch_bounds__(256) orgym_reduce_partials_kernel(const double
     __syncthreads();
     if (tid == 0) is_last = (atomicInc(ticket, (unsigned)nb - 1u) == (unsigned)nb - 1u);
     __syncthreads();
-    if (is_last) {
+    if (is_last) {  // block-uniform: the barrier below is reached by every thread of the last CTA
         __threadfence();
+        // the CTA sums are staged in shared memory by all threads at once, then added in block order as before
+        __shared__ double fin[ORGYM_REDUCE_CTAS][7];
+        for (int i = tid; i < nb * 7; i += 256) fin[i / 7][i % 7] = __ldcg(scratch + (size_t)(i / 7) * 8 + i % 7);
+        __syncthreads();
         if (tid < 8) {
             double x = 0.0;
             if (tid < 7)
-                for (int b = 0; b < nb; b++) x += __ldcg(scratch + (size_t)b * 8 + tid);
+                for (int b = 0; b < nb; b++) x += fin[b][tid];
             out[tid] = x;
         }
     }

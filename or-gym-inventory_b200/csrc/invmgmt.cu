@@ -1332,10 +1332,13 @@ extern "C" int orgym_invmgmt_export_state(orgym_handle_t h, const void* state_de
 //   I_i(t) = I0_i - sum of the <= min(L_i, T) orders of stage i still in transit          (i >= 1)
 // so with  Rhi_i = c_i,  Rlo_i = min(0, Ilo_{i+1})  (Rlo_{n-1} = 0: no supplier constraint):
 //   Ilo_i = I0_i - min(L_i,T) * Rhi_i,   Ihi_i = I0_i - min(L_i,T) * Rlo_i,   and for the retailer 0 <= I_0 <= I0_0 + T * c_0.
-// Backlogs grow by at most (request - fulfilled) <= c_i - Rlo_i per period.  *xvar bounds every state value, order, sale
-// and unfulfilled quantity of any period; *xsum bounds the per-episode statistics (sums over periods and stages).
+// The retailer's lower bound holds whatever it receives (a negative fulfilled order included): it sells min(on-hand,
+// fill), so it keeps max(on-hand - fill, 0).  Backlogs grow by at most (request - fulfilled) <= c_i - Rlo_i per period.
+// *xvar bounds every state value, order, sale and unfulfilled quantity of any period; *xsum bounds the per-episode
+// statistics (sums over periods and stages).
 struct InvTermBounds {  // per stage j = 0..n: |units sold|, on-hand inventory above zero, unfulfilled quantity
     double sale[MAXN + 1], inv[MAXN + 1], unf[MAXN + 1];
+    bool nonneg[MAXN];  // sign fact: Ilo_j >= 0, stage j's on-hand inventory is never negative after a period
 };
 static void inv_value_bounds(const InvDev& P, double dmax, double* xvar, double* xsum, InvTermBounds* tb = nullptr) {
     const int n = P.n, T = P.T;
@@ -1360,6 +1363,7 @@ static void inv_value_bounds(const InvDev& P, double dmax, double* xvar, double*
             tb->sale[i + 1] = std::max((double)P.c[i], std::fabs(Rlo[i]));  // fulfilled order r_i in [Rlo_i, c_i]
             tb->unf[i + 1] = Umax;
             tb->inv[i] = std::max(0.0, Ihi[i]);
+            tb->nonneg[i] = Ilo[i] >= 0.0;
         }
     }
     const double B0 = P.backlog ? (double)T * (dmax - Rlo[0]) : 0.0;   // retail backlog
@@ -1382,6 +1386,7 @@ static void inv_jit_spec(const InvDev& P, const std::vector<double>& disc, int p
             S->inv_bound[j] = tb.inv[j];
             S->unf_bound[j] = tb.unf[j];
         }
+        for (int i = 0; i < P.n; i++) S->inv_nonneg[i] = tb.nonneg[i];
     }
     S->n = P.n;
     S->T = P.T;

@@ -5,10 +5,10 @@
 // (ring address arithmetic, LDS/STS, position wrap-around, the policy switch, the period loop, Philox word selection).
 // For a given configuration all of it is static: lead times, capacities, prices and the horizon are known at create
 // time, and the ring position of period t is t mod L_i.  This generator therefore emits the T periods as straight-line
-// CUDA -- every ring slot a named register, every index a literal, prices / discount factors as hexadecimal float
-// literals -- and compiles it for sm_100a with NVRTC (jit.cu).  The arithmetic (integer dynamics, float64 reward terms
-// in the reference's order, numpy's summation order, Philox streams) is the ahead-of-time kernel's statement by
-// statement; tests/test_invmgmt_gpu.py checks the two kernels bit for bit against each other.
+// CUDA -- every ring slot a named register, every index a literal, prices as hexadecimal float literals, discount
+// factors from a constant-memory table -- and compiles it for sm_100a with NVRTC (jit.cu).  The arithmetic (integer
+// dynamics, float64 reward terms in the reference's order, numpy's summation order, Philox streams) is the ahead-of-time
+// kernel's statement by statement; tests/test_invmgmt_gpu.py checks the two kernels bit for bit against each other.
 //
 // Reference: inventory_management.py:224-352 (step), benchmark_InvManagementBacklogEnv.py:142-198 (BaseStockAgent).
 #include "invmgmt_jit.cuh"
@@ -61,15 +61,17 @@ void emit_kernel(Src& o, const InvJitSpec& S, const char* name, int policy, int 
     const bool episode_sum = iprofit && undiscounted && inv_jit_profit_is_exact(S, T);
     const char* W4[4] = {"w.x", "w.y", "w.z", "w.w"};
     const char* A4[4] = {"a4.x", "a4.y", "a4.z", "a4.w"};
-    // (random policy) periods re-rolled into a loop over blocks of UNR periods -- see below; the per-period discount
-    // factors then come from a constant-memory table (uniform loads)
+    // (random policy) periods re-rolled into a loop over blocks of UNR periods -- see below.
     // Block length 8 (4 for short horizons, straight-line below 8 periods).  A ring whose lead time divides the block
     // length keeps compile-time slot indices ((tb + u) mod L = u mod L), the others are shifted by L - 1 register moves
     // per period.  Measured on the default configuration (lead times 3, 5, 10; 2^24 x 30): straight-line 2.78-3.0 ms,
     // blocks of 4 2.57, 8 2.55, 12 2.56, 10 (two rings static, run-time Philox word) 2.78, 15 3.01 -- the block has to
     // stay small.
     const int UNR = bs ? 0 : (T >= 16 ? 8 : (T >= 8 ? 4 : 0));
-    if (UNR > 0 && !(iprofit && episode_sum)) {
+    // The per-period discount factors (times 1/Q under the integer profit) come from a constant-memory table, in the
+    // loop and in the straight-line periods alike: DMUL takes a constant-bank operand, whereas a float64 literal costs
+    // two uniform-register moves every period.
+    if (!episode_sum) {
         o("__constant__ double c_disc[%d] = {", T);
         for (int t = 0; t < T; t++)
             o("    %s,", lit(iprofit ? std::ldexp(S.disc[(size_t)t], qexp) : S.disc[(size_t)t]).c_str());
@@ -115,6 +117,15 @@ void emit_kernel(Src& o, const InvJitSpec& S, const char* name, int policy, int 
     bool shift[ORGYM_INV_MAX_STAGES];
     for (int i = 0; i < n; i++) shift[i] = UNR > 0 && S.L[i] > 0 && UNR % S.L[i] != 0;
     const int Tloop = UNR > 0 ? T - T % UNR : 0;
+    // max(on-hand of stage j after the period, 0); the clamp is left out where inv_value_bounds proves on-hand >= 0
+    auto onhand = [&](int j) {
+        char b[48];
+        if (S.inv_nonneg[j])
+            snprintf(b, sizeof(b), "Ic_%d", j);
+        else
+            snprintf(b, sizeof(b), "(Ic_%d > 0 ? Ic_%d : 0)", j, j);
+        return std::string(b);
+    };
     // emits period t; inside the loop t = tb + u is symbolic and only u is known here
     auto emit_period = [&](int t, int u, bool in_loop) {
         char tx[32], bx[32], dx[48];
@@ -125,7 +136,7 @@ void emit_kernel(Src& o, const InvJitSpec& S, const char* name, int policy, int 
         } else {
             snprintf(tx, sizeof(tx), "%uu", (unsigned)t);
             snprintf(bx, sizeof(bx), "%uu", (unsigned)(t >> 2));
-            snprintf(dx, sizeof(dx), "%s", lit(iprofit ? std::ldexp(S.disc[(size_t)t], qexp) : S.disc[(size_t)t]).c_str());
+            snprintf(dx, sizeof(dx), "c_disc[%d]", t);
         }
         const int w4 = (in_loop ? u : t) & 3;
         const int tq = in_loop ? u : t;               // ring slots of the non-shifted rings: (tb + u) mod L = u mod L
@@ -188,32 +199,38 @@ void emit_kernel(Src& o, const InvJitSpec& S, const char* name, int policy, int 
             // every float64 operation of the reference's expression is exact (inv_jit_profit_is_exact), so the profit
             // equals Q * sum_j (c_j / Q) * x_j with integer coefficients c_j / Q: IMADs instead of I2F + DFMA
             o("    long long pa = %s;", episode_sum ? "acc" : "0");
-            // terms with the same integer coefficient are summed first (int32, bounded by the sum of their bounds)
-            struct Term { long long c; std::string x; double bound; };
+            // terms with the same integer coefficient are summed first (int32, bounded by the sum of their bounds) -- but
+            // only within one class.  Under base-stock every quantity of the stages above the retailer is a compile-time
+            // constant (reference quirk :300: a stage's on-hand never sees the order it ships downstream), so the
+            // retailer's orders, sales, on-hand and unfulfilled quantities (class 0) are kept apart from those of the
+            // upstream stages (class 1), which the compiler then folds into one constant per period.
+            struct Term { long long c; std::string x; double bound; int cls; };
             std::vector<Term> terms;
-            auto add = [&](long long c, const std::string& x, double bound) {
+            auto add = [&](long long c, const std::string& x, double bound, int cls) {
                 if (c == 0) return;
                 for (auto& tm : terms)
-                    if (tm.c == c && tm.bound + bound < 2147483647.0) {
+                    if (tm.c == c && tm.cls == cls && tm.bound + bound < 2147483647.0) {
                         tm.x += " + " + x;
                         tm.bound += bound;
                         return;
                     }
-                terms.push_back({c, x, bound});
+                terms.push_back({c, x, bound, cls});
             };
+            // class of the quantities of stage i: its on-hand Ic_i, its fulfilled order r_i (the units stage i + 1 sells)
+            // and its unfulfilled request U_{i+1}; i = -1 stands for the retail sale s0 and the unmet demand U_0
+            auto cls_of = [&](int i) { return bs && i >= 1 ? 1 : 0; };
             char nm[64];
             for (int j = 0; j <= n; j++) {
                 snprintf(nm, sizeof(nm), "U_%d", j);
-                add(-coef_int(S.kc[j], qexp), nm, S.unf_bound[j]);
+                add(-coef_int(S.kc[j], qexp), nm, S.unf_bound[j], cls_of(j - 1));
                 if (j < n) {
-                    snprintf(nm, sizeof(nm), "(Ic_%d > 0 ? Ic_%d : 0)", j, j);
-                    add(-coef_int(S.hc[j], qexp), nm, S.inv_bound[j]);
+                    add(-coef_int(S.hc[j], qexp), onhand(j), S.inv_bound[j], cls_of(j));
                 }
                 if (j == 0)
                     snprintf(nm, sizeof(nm), "s0");
                 else
                     snprintf(nm, sizeof(nm), "r_%d", j - 1);
-                add(coef_int(S.up[j], qexp) - coef_int(S.uc[j], qexp), nm, S.sale_bound[j]);
+                add(coef_int(S.up[j], qexp) - coef_int(S.uc[j], qexp), nm, S.sale_bound[j], cls_of(j - 1));
             }
             for (const auto& tm : terms) {
                 const long long ac = tm.c < 0 ? -tm.c : tm.c;
@@ -241,7 +258,7 @@ void emit_kernel(Src& o, const InvJitSpec& S, const char* name, int policy, int 
             o("    double pr = 0.0;");
             for (int j = n; j >= 0; j--) {
                 o("    pr = fma(%s, (double)U_%d, pr);", lit(-S.kc[j]).c_str(), j);
-                if (j < n) o("    { const int inv = Ic_%d > 0 ? Ic_%d : 0; pr = fma(%s, (double)inv, pr); }", j, j, lit(-S.hc[j]).c_str());
+                if (j < n) o("    { const int inv = %s; pr = fma(%s, (double)inv, pr); }", onhand(j).c_str(), lit(-S.hc[j]).c_str());
                 if (j == 0)
                     o("    pr = fma(%s, (double)s0, pr);", lit(S.up[j] - S.uc[j]).c_str());
                 else
@@ -259,8 +276,8 @@ void emit_kernel(Src& o, const InvJitSpec& S, const char* name, int policy, int 
                 if (j == n)
                     o("      tm_%d = (rev - pc) - pen; }", j);
                 else
-                    o("      const int inv = Ic_%d > 0 ? Ic_%d : 0; const double hold = %s * (double)inv; tm_%d = ((rev - pc) - hold) - pen; }",
-                      j, j, lit(S.hc[j]).c_str(), j);
+                    o("      const int inv = %s; const double hold = %s * (double)inv; tm_%d = ((rev - pc) - hold) - pen; }",
+                      onhand(j).c_str(), lit(S.hc[j]).c_str(), j);
             }
             o("    double pr = 0.0;");
             for (int j = 0; j <= n; j++) o("    pr = pr + tm_%d;", j);
@@ -268,7 +285,7 @@ void emit_kernel(Src& o, const InvJitSpec& S, const char* name, int policy, int 
         }
         // statistics and state
         o("    s_sales += s0; s_dem += d; s_stock += U_0;");
-        for (int i = 0; i < n; i++) o("    I_%d = Ic_%d; s_inv += I_%d > 0 ? I_%d : 0;", i, i, i, i);
+        for (int i = 0; i < n; i++) o("    I_%d = Ic_%d; s_inv += %s;", i, i, onhand(i).c_str());
         if (bl)
             for (int j = 0; j <= n; j++) o("    B_%d = U_%d;", j, j);
         // rings: slot t mod L_i held R[t - L_i] / the request of period t - L_i

@@ -18,6 +18,8 @@ struct InvJitSpec {  // host-side copy of everything the generator bakes into th
     // per-term bounds behind the exactness proof (0 <= j <= n): |units sold by stage j| (retail sales, fulfilled order
     // of stage j-1), on-hand inventory above zero, unfulfilled quantity.  profit_mag() = sum_j coefficient x bound.
     double sale_bound[ORGYM_INV_MAX_STAGES + 1], inv_bound[ORGYM_INV_MAX_STAGES + 1], unf_bound[ORGYM_INV_MAX_STAGES + 1];
+    // sign facts from the same proof: stage i's on-hand inventory after any period is >= 0 (its clamp at 0 is dropped)
+    bool inv_nonneg[ORGYM_INV_MAX_STAGES];
     // policy baked into the kernel: 0 = base-stock with the integer levels `target`, 1 = uniform random orders
     int policy;
     long long target[ORGYM_INV_MAX_STAGES];
