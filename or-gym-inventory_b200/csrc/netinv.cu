@@ -401,7 +401,37 @@ __global__ void net_export_kernel(const __grid_constant__ NetDev P, int64_t N, c
 static size_t net_obs_smem(const NetDev& P) {
     return 128 + (((size_t)P.obs_dim * 2 + 127) & ~(size_t)127) + (((size_t)NET_OBS_ROWS * P.obs_dim * 4 + 127) & ~(size_t)127);
 }
-int net_obs_kernel_fits(const NetDev& P) { return net_jit_uses_stream(P) && net_obs_smem(P) <= 200 * 1024; }
+
+NetPlan net_plan(const NetDev& P) {
+    NetPlan plan;
+    // auto: specialise graphs of up to 128 reorder links (the 64-node / 88-link synthetic graph compiles in 10-15 s,
+    // once: cubins are cached on disk); ORGYM_NET_JIT=0 never, =1 always, =2 always and fail loudly
+    const char* jv = getenv("ORGYM_NET_JIT");
+    plan.jit = !jv ? (P.E <= 128 ? 1 : 0) : jv[0] == '0' ? 0 : jv[0] == '2' ? 2 : 1;
+    // graph size selects the streaming STEP form; ORGYM_NET_JIT_STREAM=1 / 0 forces it on / off, so that small graphs
+    // can test it
+    const char* sv = getenv("ORGYM_NET_JIT_STREAM");
+    plan.stream = sv ? (atoi(sv) ? 1 : 0) : (net_large_graph(P) ? 1 : 0);
+    // Single-pass streaming form: usable when every inventory-holding supplier comes after its purchasers in node order
+    // (true of the reference's graphs, which number nodes market -> raw material), so that a purchaser still finds its
+    // suppliers' start-of-period inventory in the state tile.  ORGYM_NET_JIT_ONEPASS=0 forces the two-pass form, so
+    // that graphs in the reference's numbering can test it.
+    const char* ov = getenv("ORGYM_NET_JIT_ONEPASS");
+    plan.onepass = !(ov && atoi(ov) == 0);
+    for (int j = 0; j < P.J; j++)
+        for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
+            const int s = P.sup[P.pred_idx[z]];
+            if (s >= 0 && s <= j) plan.onepass = 0;
+        }
+    // The streaming kernel stops after the state update and the TMA-staged net_obs_kernel writes the observation from
+    // the float32 ring copy, unless 32 observation rows do not fit that kernel's shared memory: then the kernel's own
+    // pass C writes it (ORGYM_NET_OBS_TMA=0 forces pass C, so that small graphs can test it; the ring copy stays).
+    plan.ring32 = plan.stream && net_obs_smem(P) <= 200 * 1024;
+    const char* tv = getenv("ORGYM_NET_OBS_TMA");
+    plan.obs_kernel = plan.ring32 && !(tv && atoi(tv) == 0);
+    return plan;
+}
+
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 
 __global__ void __launch_bounds__(NET_OBS_THREADS) net_obs_kernel(const __grid_constant__ NetDev P, int64_t N,
@@ -659,19 +689,15 @@ extern "C" int orgym_netinv_create(const orgym_netinv_config_t* c, int64_t num_e
             cudaFuncSetAttribute(net_sim_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(220 * 1024));
             cudaFuncSetAttribute(net_sim_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(220 * 1024));
             cudaFuncSetAttribute(net_obs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(220 * 1024));
-            // large graphs whose observation is assembled by net_obs_kernel keep a float32 copy of the rings in the tile
-            P.ring32 = net_obs_kernel_fits(P);
-            // kernel specialised for this topology (NVRTC); any failure falls back to the generic kernel above
-            H->jit_threads = 0;
+            H->plan = net_plan(P);
+            P.ring32 = H->plan.ring32;
+            // kernel specialised for this topology (NVRTC); unless it is required, a failure falls back to the generic
+            // kernel above
             H->dem_dev = nullptr;
-            // auto: specialise graphs of up to 128 reorder links (the 64-node / 88-link synthetic graph compiles in
-            // 10-15 s, once: cubins are cached on disk); ORGYM_NET_JIT=0 never, =1 always, =2 always and fail loudly
-            const char* jv = getenv("ORGYM_NET_JIT");
-            const bool want_jit = jv ? jv[0] != '0' : (P.E <= 128);
-            if (want_jit) {
+            if (H->plan.jit) {
                 std::string jerr;
                 if (net_jit_build(H, &jerr) != 0) {
-                    if (jv && jv[0] == '2') FAIL(ORGYM_E_CUDA, "ORGYM_NET_JIT=2 but specialisation failed: %s", jerr.c_str());
+                    if (H->plan.jit == 2) FAIL(ORGYM_E_CUDA, "ORGYM_NET_JIT=2 but specialisation failed: %s", jerr.c_str());
                     fprintf(stderr, "[orgym_b200] network kernel specialisation unavailable (%s); using the generic kernel\n",
                             jerr.substr(0, 600).c_str());
                 }
@@ -771,7 +797,7 @@ extern "C" int orgym_netinv_step(orgym_handle_t h, void* state_dev, const float*
         int jrc = net_jit_launch(H, A, (cudaStream_t)stream);
         if (jrc != ORGYM_OK) return jrc;
         // large graphs: the streaming kernel leaves the state in HBM; the observation is assembled by the TMA-staged kernel
-        if (H->jit_stream && H->jit_obs_split) return net_obs_launch(H, state_dev, obs_dev, (cudaStream_t)stream);
+        if (H->plan.obs_kernel) return net_obs_launch(H, state_dev, obs_dev, (cudaStream_t)stream);
         return ORGYM_OK;
     }
     size_t tile = (size_t)H->threads * (P.obs_dim | 1) * 4;
@@ -826,7 +852,7 @@ extern "C" int orgym_netinv_rollout(orgym_handle_t h, void* scratch_dev, uint64_
     A.final_Y = out->final_Y_dev;
     A.final_U = out->final_U_dev;
     A.partials = out->summary_dev ? H->partials : nullptr;
-    const int thr = H->jit.fn ? H->jit_threads : H->threads;
+    const int thr = H->jit.fn ? NET_JIT_THREADS : H->threads;
     int nblocks = (int)((A.N + thr - 1) / thr);
     if (H->jit.fn) {
         int rc = net_jit_launch(H, A, (cudaStream_t)stream);
@@ -851,8 +877,9 @@ extern "C" int orgym_netinv_codegen(const orgym_netinv_config_t* cfg, int compil
         delete P;
         return rc;
     }
-    P->ring32 = net_obs_kernel_fits(*P);
-    std::string src = net_jit_source(*P, 128);
+    const NetPlan plan = net_plan(*P);
+    P->ring32 = plan.ring32;
+    std::string src = net_jit_source(*P, plan);
     delete P;
     if (needed) *needed = (int64_t)src.size();
     if (buf && buflen > 0) {

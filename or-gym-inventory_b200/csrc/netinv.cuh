@@ -10,7 +10,7 @@
 
 struct NetDev {
     int T, backlog, J, E, M, obs_dim, sumL;
-    int ring32;  // the state tile carries a float32 copy of the lead-time rings for net_obs_kernel (large graphs)
+    int ring32;  // the state tile carries a float32 copy of the lead-time rings for net_obs_kernel (NetPlan::ring32)
     const double* disc;  // [T] alpha**t
     double I0[NJ], h[NJ], C[NJ], v[NJ], o[NJ];
     uint8_t is_factory[NJ], is_retail[NJ];
@@ -26,22 +26,36 @@ struct NetDev {
     AliasDev dem[NM];
 };
 
+// Which kernels a handle runs, decided once per graph by net_plan (netinv.cu).  The state layout (NetDev::ring32), the
+// generated source and the launches all read this one decision.
+struct NetPlan {
+    int jit;         // NVRTC specialisation: 0 never (generic kernel), 1 when it compiles, 2 required (failure is an error)
+    int stream;      // the specialised STEP kernel is the streaming form: state stays in HBM (large graphs)
+    int onepass;     // streaming form in its single-pass variant: suppliers follow their purchasers in node order
+    int ring32;      // state tiles carry the float32 ring copy: stream, and net_obs_kernel's shared memory fits the rows
+    int obs_kernel;  // net_obs_kernel writes the STEP observation instead of the streaming kernel's pass C (ring32)
+};
+
+// threads per CTA of the specialised kernels
+#define NET_JIT_THREADS 128
+
 struct NetHandle {
     HandleBase base;
     NetDev dev;
-    int threads;  // threads per CTA that fit the shared-memory work vectors
+    NetPlan plan;
+    int threads;  // threads per CTA of the generic kernel that fit the shared-memory work vectors
     size_t smem;
     std::vector<void*> allocs;
     double* partials;
     // run-time specialised kernel (netinv_jit.cu); jit.fn == nullptr -> generic kernel
     JitKernel jit;             // module + STEP kernel
     cudaKernel_t jit_rollout;  // ROLLOUT kernel of the same module
-    int jit_threads;
-    int jit_stream;            // STEP kernel is the streaming variant (large graphs)
-    int jit_obs_split;         // streaming variant without its observation pass: net_obs_kernel (TMA-staged) follows it
-    int jit_onepass;           // streaming variant in its single-pass form (no scratch rows, no action tile)
     AliasDev* dem_dev;  // device copy of dev.dem[] for the specialised kernel
 };
+
+// Hundreds of live float64 values per instance: the register-resident specialised kernels spill.  Such graphs get the
+// streaming STEP form and launch bounds for 255 registers.
+static inline bool net_large_graph(const NetDev& P) { return 2 * P.J + 3 * P.E + 2 * P.M > 128; }
 
 // State layout: tiles of NET_TILE = 128 instances; inside a tile every field is slot-major,
 //   [key u64][X J][Y E][U M][ring sumL] f64, [period i32][episode u32], [scratch: R_t E, consumed J] f64
@@ -87,13 +101,10 @@ static inline int64_t net_state_bytes(const NetDev& P, int64_t num_envs) {
 }
 
 
+// netinv.cu: the kernel plan of a graph, from its size and node order; the only reader of ORGYM_NET_JIT and of the test
+// hooks ORGYM_NET_JIT_STREAM, ORGYM_NET_JIT_ONEPASS and ORGYM_NET_OBS_TMA
+NetPlan net_plan(const NetDev& P);
 // netinv_jit.cu: generate + compile the kernel specialised for this topology (returns 0 on success)
 int net_jit_build(NetHandle* H, std::string* err);
 int net_jit_launch(const NetHandle* H, const struct NetSimArgs& A, cudaStream_t s);
-std::string net_jit_source(const NetDev& P, int nthr);
-int net_jit_uses_stream(const NetDev& P);
-// netinv.cu: the streaming STEP form is used and 32 observation rows fit net_obs_kernel's shared memory.  Such handles
-// keep the float32 ring copy (NetDev::ring32) that net_obs_kernel reads.
-int net_obs_kernel_fits(const NetDev& P);
-int net_jit_onepass(const NetDev& P);    // suppliers follow their purchasers in node order (test hook: ORGYM_NET_JIT_ONEPASS=0)
-int net_jit_obs_split(const NetDev& P);  // net_obs_kernel_fits (test hook: ORGYM_NET_OBS_TMA=0 keeps the fused observation pass)
+std::string net_jit_source(const NetDev& P, const NetPlan& plan);  // P.ring32 == plan.ring32

@@ -33,51 +33,32 @@ std::string lit(double v) {
     snprintf(buf, sizeof(buf), "%a", v);
     return buf;
 }
-void emit_step_stream(Src& o, const NetDev& P, int min_blocks);
+// One allocation step of supplier s (network_management.py:459-485): what its on-hand inventory x leaves after the
+// consumption `cons` of its earlier links, capped by a factory's capacity, fills the request `req` into f.  `head`
+// starts the first line, `ind` indents the others.
+void emit_alloc(Src& o, const NetDev& P, int s, const std::string& head, const std::string& ind, const std::string& x,
+                const std::string& cons, const std::string& f) {
+    o("%sdouble avail = %s - %s; avail = avail > 0.0 ? avail : 0.0; double oa = avail;", head.c_str(), x.c_str(), cons.c_str());
+    if (P.is_factory[s])
+        o("%s{ double mp = %s * avail; double lim = mp < %s ? mp : %s; oa = lim < oa ? lim : oa; }", ind.c_str(),
+          lit(P.v[s]).c_str(), lit(P.C[s]).c_str(), lit(P.C[s]).c_str());
+    o("%s%s = oa < req ? oa : req;", ind.c_str(), f.c_str());
+}
+// what the fill f of one of its links takes from supplier s: f / v (x / 1.0 == x, so yield 1 divides by nothing)
+std::string consumed(const NetDev& P, int s, const std::string& f) { return P.v[s] == 1.0 ? f : f + " / " + lit(P.v[s]); }
+// ring commit of the streaming kernel: `v` goes into the ring slot `slot` and into its float32 copy
+std::string ring_commit(const NetDev& P, const std::string& slot, const std::string& v) {
+    return "*" + slot + " = " + v + ";" + (P.ring32 ? " r32[" + slot + " - ring] = (float)" + v + ";" : "");
+}
+void emit_step_stream(Src& o, const NetDev& P, const NetPlan& plan, int min_blocks);
 }  // namespace
 
-// graph size selects the streaming STEP form; ORGYM_NET_JIT_STREAM=1 / 0 forces it on / off, so that small graphs can
-// test it
-int net_jit_uses_stream(const NetDev& P) {
-    int stream = 2 * P.J + 3 * P.E + 2 * P.M > 128 ? 1 : 0;
-    if (const char* sv = getenv("ORGYM_NET_JIT_STREAM")) stream = atoi(sv) ? 1 : 0;
-    return stream;
-}
-
-static int env_int(const char* name, int dflt, int lo, int hi) {
-    const char* v = getenv(name);
-    if (!v) return dflt;
-    const int x = atoi(v);
-    return x < lo || x > hi ? dflt : x;
-}
-// The streaming STEP kernel stops after the state update and netinv.cu's TMA-staged net_obs_kernel writes the
-// observation, unless the observation rows are too wide for that kernel: then the kernel's own pass C writes it
-// (ORGYM_NET_OBS_TMA=0 forces pass C, so that small graphs can test it).
-int net_jit_obs_split(const NetDev& P) {
-    return env_int("ORGYM_NET_OBS_TMA", 1, 0, 1) && net_obs_kernel_fits(P);
-}
-// Single-pass form of the streaming STEP kernel (see emit_step_stream): usable when every inventory-holding supplier comes
-// after its purchasers in main-node order (true of the reference's graphs, which number nodes market -> raw material),
-// so that a purchaser still finds its suppliers' start-of-period inventory in the state tile.  ORGYM_NET_JIT_ONEPASS=0
-// forces the two-pass form, so that graphs in the reference's numbering can test it.
-int net_jit_onepass(const NetDev& P) {
-    if (!env_int("ORGYM_NET_JIT_ONEPASS", 1, 0, 1)) return 0;
-    for (int j = 0; j < P.J; j++)
-        for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
-            const int s = P.sup[P.pred_idx[z]];
-            if (s >= 0 && s <= j) return 0;
-        }
-    for (int i = 0; i + 1 < P.E; i++)  // a supplier's links must be one contiguous run of the sorted link list
-        for (int k = i + 2; k < P.E; k++)
-            if (P.sup[i] >= 0 && P.sup[k] == P.sup[i] && P.sup[i + 1] != P.sup[i]) return 0;
-    return 1;
-}
-std::string net_jit_source(const NetDev& P, int nthr) {
+std::string net_jit_source(const NetDev& P, const NetPlan& plan) {
     const int J = P.J, E = P.E, M = P.M;
     Src o;
     o.s += orgym_jit_device_rng_src();
     o.s += orgym_jit_net_args_src();
-    o("#define NTHR %d", nthr);
+    o("#define NTHR %d", NET_JIT_THREADS);
     o("#define NJ %d\n#define NE %d\n#define NM %d\n#define NOBS %d\n#define NSUML %d\n#define NT %d", J, E, M, P.obs_dim,
       P.sumL, P.T);
     o("#define OSTRIDE %d", P.obs_dim | 1);
@@ -187,16 +168,8 @@ std::string net_jit_source(const NetDev& P, int nthr) {
             o("      R[%d] = 0.0; (void)req; }", i);
         else {
             if (i == 0 || P.sup[i - 1] != s) o("      cons = 0.0;");
-            o("      double avail = X[%d] - cons; avail = avail > 0.0 ? avail : 0.0; double oa = avail;", s);
-            if (P.is_factory[s]) {
-                o("      { double mp = %s * avail; double lim = mp < %s ? mp : %s; oa = lim < oa ? lim : oa; }", lit(P.v[s]).c_str(),
-                  lit(P.C[s]).c_str(), lit(P.C[s]).c_str());
-            }
-            o("      double f = oa < req ? oa : req;");
-            if (P.v[s] == 1.0)
-                o("      cons += f;");
-            else
-                o("      cons += f / %s;", lit(P.v[s]).c_str());
+            emit_alloc(o, P, s, "      ", "      ", "X[" + std::to_string(s) + "]", "cons", "double f");
+            o("      cons += %s;", consumed(P, s, "f").c_str());
             o("      R[%d] = f;", i);
             if (i == E - 1 || P.sup[i + 1] != s) o("      Cn[%d] = cons;", s);
             o("    }");
@@ -331,17 +304,16 @@ std::string net_jit_source(const NetDev& P, int nthr) {
     };
     // small graphs: STEP 5 CTAs/SM (<= 102 registers), ROLLOUT 3; large graphs (hundreds of live float64 values per
     // instance) spill either way and run best with all 255 registers (measured on the 64-node synthetic graph)
-    const bool big = 2 * J + 3 * E + 2 * M > 128;
-    const int stream = net_jit_uses_stream(P);  // large graphs: state stays in HBM, coalesced 32-column tiles
-    if (stream)
+    const bool big = net_large_graph(P);
+    if (plan.stream)  // large graphs: state stays in HBM, coalesced 32-column tiles
         // 64 registers per thread: a launch of 2^17 instances is 28 warps per SM, so with 8 CTAs of 128 threads per SM the
         // whole batch is resident in one wave (measured on the 64-node graph: 0.470 vs 0.486 ms for the step pair at 128
         // registers)
-        emit_step_stream(o, P, 8);
+        emit_step_stream(o, P, plan, 8);
     else
         emit_kernel("net_jit_step", 0, big ? 2 : 5);
     emit_kernel("net_jit_rollout", 1, big ? 1 : 3);
-    o("// step_kernel_kind=%s", stream ? "stream" : "register");
+    o("// step_kernel_kind=%s", plan.stream ? "stream" : "register");
     return o.s;
 }
 
@@ -357,11 +329,16 @@ std::string net_jit_source(const NetDev& P, int nthr) {
 // and observation blocks move through 32-column shared-memory tiles, so every global access is coalesced whatever
 // the observation length.
 namespace {
-void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
+void emit_step_stream(Src& o, const NetDev& P, const NetPlan& plan, int min_blocks) {
     const int J = P.J, E = P.E, M = P.M, W = P.obs_dim;
-    std::vector<int> has_seg(J, 0);
-    for (int i = 0; i < E; i++)
-        if (P.sup[i] >= 0) has_seg[P.sup[i]] = 1;
+    auto emit_reset = [&](const char* ind) {  // the instance's initial state, stored to its tile
+        for (int j = 0; j < J; j++) o("%ss_X[%d * NP + el] = %s;", ind, j, lit(P.I0[j]).c_str());
+        o("%sfor (int i = 0; i < NE; i++) s_Y[i * NP + el] = 0.0;", ind);
+        o("%sfor (int r = 0; r < NM; r++) s_U[r * NP + el] = 0.0;", ind);
+        o("%sfor (int k = 0; k < NSUML; k++) ring[k * NP + el] = 0.0;", ind);
+        if (P.ring32) o("%sfor (int k = 0; k < NSUML; k++) r32[k * NP + el] = 0.0f;", ind);
+        o("%ss_period[el] = 0; s_episode[el] = episode + 1;", ind);
+    };
     o("extern \"C\" __global__ void __launch_bounds__(NTHR, %d) net_jit_step(const NetSimArgs A, const double* __restrict__ disc,", min_blocks);
     o("    const AliasDev* __restrict__ dem) {");
     o("  extern __shared__ __align__(16) unsigned char smem_raw[];");
@@ -390,12 +367,7 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
     o("    if (t >= NT) {");
     o("      do_step = false;");
     o("      if (A.autoreset == ORGYM_AUTORESET_NEXT_STEP) {");
-    for (int j = 0; j < J; j++) o("        s_X[%d * NP + el] = %s;", j, lit(P.I0[j]).c_str());
-    o("        for (int i = 0; i < NE; i++) s_Y[i * NP + el] = 0.0;");
-    o("        for (int r = 0; r < NM; r++) s_U[r * NP + el] = 0.0;");
-    o("        for (int k = 0; k < NSUML; k++) ring[k * NP + el] = 0.0;");
-    if (P.ring32) o("        for (int k = 0; k < NSUML; k++) r32[k * NP + el] = 0.0f;");
-    o("        s_period[el] = 0; s_episode[el] = episode + 1;");
+    emit_reset("        ");
     o("        A.reward[e] = 0.0; A.terminated[e] = 0; A.truncated[e] = 0;");
     o("      } else {");
     o("        atomicOr(A.err, ORGYM_ERR_STEP_PAST_END);");
@@ -403,10 +375,66 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
     o("      }");
     o("    }");
     o("  }");
-    const int ONEPASS = net_jit_onepass(P);
-    o("  // stream_form=%s", ONEPASS ? "onepass" : "twopass");
-    std::vector<int> link_done(E, 0);
-    if (ONEPASS) {
+    // Visit of main node j once the R_t of its links are known, the same in both forms: arrivals, pipeline update and
+    // ring commit of its inbound links, its on-hand inventory less the consumption `cons`, its market links, its
+    // profit.  In scope: the loaded rows x<j>, y<i>, ar<i>, u<r>, the ring slots slot<i> and R_t rt<i> of its inbound
+    // links, and the R_t of each outbound link l as <succ><l>.
+    auto emit_visit = [&](int j, const std::string& cons, const std::string& succ) {
+        o("      { double arr = 0.0, PC = 0.0, HCp = 0.0;");
+        for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
+            const int i = P.pred_idx[z];
+            if (P.L[i] == 0)
+                o("        { const double ar = rt%d;", i);
+            else
+                o("        { const double ar = ar%d; %s", i,
+                  ring_commit(P, "slot" + std::to_string(i), "rt" + std::to_string(i)).c_str());
+            o("          arr += ar; const double yn = (y%d - ar) + rt%d; s_Y[%d * NP + el] = yn;", i, i, i);
+            o("          PC += %s * rt%d; HCp += %s * (yn > 0.0 ? yn : 0.0); }", lit(P.p[i]).c_str(), i, lit(P.g[i]).c_str());
+        }
+        o("        double x = (x%d + arr) - %s;", j, cons.c_str());
+        o("        double SR = 0.0, sold = 0.0, UP = 0.0;");
+        for (int r = 0; r < M; r++) {
+            if (P.rt_node[r] != j) continue;
+            o("        double S%d, U%d;", r, r);
+            o("        { double d;");
+            o("          if (A.demand) d = rint(A.demand[e * A.d_se + %d]);", r);
+            o("          else d = (double)sample_fixed(dem[%d], dem[%d].table, key, episode, t, %du);", r, r, r);
+            o("          d = d > 0.0 ? d : 0.0;");
+            o("          const double fill = d + u%d; const double invr = x > 0.0 ? x : 0.0;", r);
+            o("          S%d = invr < fill ? invr : fill; x = x - S%d; const double un = fill - S%d; U%d = %s;", r, r, r, r,
+              P.backlog ? "un" : "0.0");
+            o("          s_U[%d * NP + el] = U%d;", r, r);
+            o("          if (A.info_demand) A.info_demand[NET_IIDX(A, e, NM, %d)] = d;", r);
+            o("          if (A.info_sales) A.info_sales[NET_IIDX(A, e, NE + NM, %d)] = S%d; }", E + r, r);
+        }
+        o("        s_X[%d * NP + el] = x;", j);
+        for (int z = P.succ_ptr[j]; z < P.succ_ptr[j + 1]; z++) {
+            const int l = P.succ_idx[z];
+            if (l < E)
+                o("        SR += %s * %s%d; sold += %s%d;", lit(P.p[l]).c_str(), succ.c_str(), l, succ.c_str(), l);
+            else {
+                const int r = l - E;
+                if (P.is_retail[j]) o("        UP += %s * U%d;", lit(P.rt_b[r]).c_str(), r);
+                o("        SR += %s * S%d; sold += S%d;", lit(P.rt_p[r]).c_str(), r, r);
+            }
+        }
+        o("        const double xp = x > 0.0 ? x : 0.0; const double HC = %s * xp + HCp; double OC = 0.0;", lit(P.h[j]).c_str());
+        if (P.is_factory[j]) {
+            if (!(P.v[j] > 0.0))
+                o("        OC = 0.0;");
+            else if (P.v[j] == 1.0)
+                o("        OC = %s * sold;", lit(P.o[j]).c_str());
+            else
+                o("        OC = %s * (sold / %s);", lit(P.o[j]).c_str(), lit(P.v[j]).c_str());
+        }
+        o("        (void)sold; const double pj = (((SR - PC) - OC) - HC) - UP; total += pj;");
+        o("        if (A.info_profit) A.info_profit[NET_IIDX(A, e, NJ, %d)] = pj; }", j);
+    };
+    std::vector<int> has_pur(E, 0);  // the link's purchaser holds inventory (it is visited with that node)
+    for (int j = 0; j < J; j++)
+        for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) has_pur[P.pred_idx[z]] = 1;
+    o("  // stream_form=%s", plan.onepass ? "onepass" : "twopass");
+    if (plan.onepass) {
         // ---- single pass over the main nodes.  The two-pass form below parks every R_t and every supplier's consumption in
         // scratch rows of the state tile between its passes: with the whole batch resident that is 1 KB per instance
         // written and read back through DRAM (the scratch of 2^17 instances exceeds the L2).  Here a node recomputes what
@@ -424,36 +452,28 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
         o("  const float* const arow = A.actions + ec * NE;");
         o("#define REQ(i) net_req(arow + (i))");
         // allocation chain of supplier s from its first link to link i1; f of link i lands in variable <pfx><i>
-        auto emit_chain = [&](int s, int i1, const char* xvar, const char* pfx, const char* ind, bool keep_cons) {
-            o("%sdouble cons_%s = 0.0;", ind, pfx);
+        auto emit_chain = [&](int s, int i1, const std::string& xvar, const std::string& pfx, const std::string& ind,
+                              bool keep_cons) {
+            o("%sdouble cons_%s = 0.0;", ind.c_str(), pfx.c_str());
             for (int i = seg0[s]; i <= i1; i++) {
-                o("%sdouble %s%d;", ind, pfx, i);
-                o("%s{ const double req = rq%d; double avail = %s - cons_%s; avail = avail > 0.0 ? avail : 0.0; double oa = avail;",
-                  ind, i, xvar, pfx);
-                if (P.is_factory[s])
-                    o("%s  { double mp = %s * avail; double lim = mp < %s ? mp : %s; oa = lim < oa ? lim : oa; }", ind,
-                      lit(P.v[s]).c_str(), lit(P.C[s]).c_str(), lit(P.C[s]).c_str());
-                o("%s  %s%d = oa < req ? oa : req;", ind, pfx, i);
-                if (i < i1 || keep_cons) {
-                    if (P.v[s] == 1.0)
-                        o("%s  cons_%s += %s%d; }", ind, pfx, pfx, i);
-                    else
-                        o("%s  cons_%s += %s%d / %s; }", ind, pfx, pfx, i, lit(P.v[s]).c_str());
-                } else
-                    o("%s  }", ind);
+                const std::string f = pfx + std::to_string(i);
+                o("%sdouble %s;", ind.c_str(), f.c_str());
+                emit_alloc(o, P, s, ind + "{ const double req = rq" + std::to_string(i) + "; ", ind + "  ", xvar, "cons_" + pfx, f);
+                if (i < i1 || keep_cons)
+                    o("%s  cons_%s += %s; }", ind.c_str(), pfx.c_str(), consumed(P, s, f).c_str());
+                else
+                    o("%s  }", ind.c_str());
             }
         };
-        auto emit_rt = [&](int i, const char* xvar, const char* ind) {  // declares rt<i>
+        auto emit_rt = [&](int i, const std::string& xvar, const char* ind) {  // declares rt<i>
             const int s = P.sup[i];
-            char pfx[32];
-            snprintf(pfx, sizeof(pfx), "g%d_", i);
             if (s == -1)
                 o("%sconst double rt%d = rq%d;", ind, i, i);
             else if (s < 0)
                 o("%sconst double rt%d = 0.0;", ind, i);
             else {
-                emit_chain(s, i, xvar, pfx, ind, false);
-                o("%sconst double rt%d = %s%d;", ind, i, pfx, i);
+                emit_chain(s, i, xvar, "g" + std::to_string(i) + "_", ind, false);
+                o("%sconst double rt%d = g%d_%d;", ind, i, i, i);
             }
             o("%sif (A.info_sales) A.info_sales[NET_IIDX(A, e, NE + NM, %d)] = rt%d;", ind, i, i);
         };
@@ -505,32 +525,27 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
                     snprintf(ab, sizeof(ab), "s_U + %d * NP + el", r);
                     n.d8.push_back({nb, ab});
                 }
-            if (has_seg[j])
+            if (P.has_seg[j])
                 for (int l = seg0[j]; l <= seg1[j]; l++) need[(size_t)l] = 1;
             for (int l = 0; l < E; l++)
                 if (need[(size_t)l]) n.acts.push_back(l);
         }
         o("  double total = 0.0;");
         o("  if (do_step) {");
-        {  // reorder links whose purchaser holds no inventory: pipeline bookkeeping only (before any X row changes)
-            std::vector<int> has_pur(E, 0);
-            for (int j = 0; j < J; j++)
-                for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) has_pur[P.pred_idx[z]] = 1;
-            for (int i = 0; i < E; i++) {
-                if (has_pur[i]) continue;
-                link_done[i] = 1;
-                const int s = P.sup[i], L = P.L[i];
-                o("    {");
-                if (s >= 0) o("      const double xq = s_X[%d * NP + el];", s);
-                for (int l : req_links(i)) o("      const double rq%d = REQ(%d);", l, l);
-                emit_rt(i, "xq", "      ");
-                if (L == 0)
-                    o("      const double ar = rt%d;", i);
-                else
-                    o("      double* slot = ring + (%d + t %% %d) * NP + el; const double ar = *slot; *slot = rt%d;%s", P.roff[i], L, i,
-                      P.ring32 ? (std::string(" r32[slot - ring] = (float)rt") + std::to_string(i) + ";").c_str() : "");
-                o("      s_Y[%d * NP + el] = (s_Y[%d * NP + el] - ar) + rt%d; }", i, i, i);
-            }
+        // reorder links whose purchaser holds no inventory: pipeline bookkeeping only (before any X row changes)
+        for (int i = 0; i < E; i++) {
+            if (has_pur[i]) continue;
+            const int s = P.sup[i], L = P.L[i];
+            o("    {");
+            if (s >= 0) o("      const double xq = s_X[%d * NP + el];", s);
+            for (int l : req_links(i)) o("      const double rq%d = REQ(%d);", l, l);
+            emit_rt(i, "xq", "      ");
+            if (L == 0)
+                o("      const double ar = rt%d;", i);
+            else
+                o("      double* slot = ring + (%d + t %% %d) * NP + el; const double ar = *slot; %s", P.roff[i], L,
+                  ring_commit(P, "slot", "rt" + std::to_string(i)).c_str());
+            o("      s_Y[%d * NP + el] = (s_Y[%d * NP + el] - ar) + rt%d; }", i, i, i);
         }
         // Each node ends in stores and (uniform) branches around the optional info outputs, basic-block boundaries the
         // compiler does not hoist loads across, so a warp pays one memory round trip per node.  Writing the loads of node
@@ -550,68 +565,10 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
             // R_t of the inbound links, own allocation chain
             for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
                 const int i = P.pred_idx[z];
-                char xv[32];
-                snprintf(xv, sizeof(xv), "xq%d", i);
-                emit_rt(i, xv, "      ");
-                link_done[i] = 1;
+                emit_rt(i, "xq" + std::to_string(i), "      ");
             }
-            if (has_seg[j]) {
-                char xv[32];
-                snprintf(xv, sizeof(xv), "x%d", j);
-                emit_chain(j, seg1[j], xv, "qs", "      ", true);
-            }
-            o("      { double arr = 0.0, PC = 0.0, HCp = 0.0;");
-            for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
-                const int i = P.pred_idx[z], L = P.L[i];
-                if (L == 0)
-                    o("        { const double ar = rt%d;", i);
-                else
-                    o("        { const double ar = ar%d; *slot%d = rt%d;%s", i, i, i,
-                      P.ring32 ? (std::string(" r32[slot") + std::to_string(i) + " - ring] = (float)rt" + std::to_string(i) + ";").c_str() : "");
-                o("          arr += ar; const double yn = (y%d - ar) + rt%d; s_Y[%d * NP + el] = yn;", i, i, i);
-                o("          PC += %s * rt%d; HCp += %s * (yn > 0.0 ? yn : 0.0); }", lit(P.p[i]).c_str(), i, lit(P.g[i]).c_str());
-            }
-            if (has_seg[j])
-                o("        double x = (x%d + arr) - cons_qs;", j);
-            else
-                o("        double x = (x%d + arr) - 0.0;", j);
-            o("        double SR = 0.0, sold = 0.0, UP = 0.0;");
-            for (int r = 0; r < M; r++) {
-                if (P.rt_node[r] != j) continue;
-                o("        double S%d, U%d;", r, r);
-                o("        { double d;");
-                o("          if (A.demand) d = rint(A.demand[e * A.d_se + %d]);", r);
-                o("          else d = (double)sample_fixed(dem[%d], dem[%d].table, key, episode, t, %du);", r, r, r);
-                o("          d = d > 0.0 ? d : 0.0;");
-                o("          const double fill = d + u%d; const double invr = x > 0.0 ? x : 0.0;", r);
-                o("          S%d = invr < fill ? invr : fill; x = x - S%d; const double un = fill - S%d; U%d = %s;", r, r, r, r,
-                  P.backlog ? "un" : "0.0");
-                o("          s_U[%d * NP + el] = U%d;", r, r);
-                o("          if (A.info_demand) A.info_demand[NET_IIDX(A, e, NM, %d)] = d;", r);
-                o("          if (A.info_sales) A.info_sales[NET_IIDX(A, e, NE + NM, %d)] = S%d; }", E + r, r);
-            }
-            o("        s_X[%d * NP + el] = x;", j);
-            for (int z = P.succ_ptr[j]; z < P.succ_ptr[j + 1]; z++) {
-                const int l = P.succ_idx[z];
-                if (l < E)
-                    o("        SR += %s * qs%d; sold += qs%d;", lit(P.p[l]).c_str(), l, l);
-                else {
-                    const int r = l - E;
-                    if (P.is_retail[j]) o("        UP += %s * U%d;", lit(P.rt_b[r]).c_str(), r);
-                    o("        SR += %s * S%d; sold += S%d;", lit(P.rt_p[r]).c_str(), r, r);
-                }
-            }
-            o("        const double xp = x > 0.0 ? x : 0.0; const double HC = %s * xp + HCp; double OC = 0.0;", lit(P.h[j]).c_str());
-            if (P.is_factory[j]) {
-                if (!(P.v[j] > 0.0))
-                    o("        OC = 0.0;");
-                else if (P.v[j] == 1.0)
-                    o("        OC = %s * sold;", lit(P.o[j]).c_str());
-                else
-                    o("        OC = %s * (sold / %s);", lit(P.o[j]).c_str(), lit(P.v[j]).c_str());
-            }
-            o("        (void)sold; const double pj = (((SR - PC) - OC) - HC) - UP; total += pj;");
-            o("        if (A.info_profit) A.info_profit[NET_IIDX(A, e, NJ, %d)] = pj; }", j);
+            if (P.has_seg[j]) emit_chain(j, seg1[j], "x" + std::to_string(j), "qs", "      ", true);
+            emit_visit(j, P.has_seg[j] ? "cons_qs" : "0.0", "qs");
             o("    }");
             // a CTA-wide barrier after every 4th node keeps the warps of a CTA within the same stretch of this long
             // straight-line kernel, so an instruction line is fetched once per CTA rather than once per warp (measured:
@@ -626,7 +583,7 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
     // ---- pass A: orders, 32 links per action chunk
     o("  double cons = 0.0;");
     for (int j = 0; j < J; j++)
-        if (has_seg[j]) o("  double xs%d = 0.0;", j);
+        if (P.has_seg[j]) o("  double xs%d = 0.0;", j);
     for (int c0 = 0; c0 < E; c0 += 32) {
         const int c1 = std::min(E, c0 + 32);
         o("  __syncwarp();");
@@ -648,15 +605,8 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
                 o("      f = 0.0; (void)req;");
             else {
                 if (i == 0 || P.sup[i - 1] != s) o("      cons = 0.0;");
-                o("      double avail = xs%d - cons; avail = avail > 0.0 ? avail : 0.0; double oa = avail;", s);
-                if (P.is_factory[s])
-                    o("      { double mp = %s * avail; double lim = mp < %s ? mp : %s; oa = lim < oa ? lim : oa; }",
-                      lit(P.v[s]).c_str(), lit(P.C[s]).c_str(), lit(P.C[s]).c_str());
-                o("      f = oa < req ? oa : req;");
-                if (P.v[s] == 1.0)
-                    o("      cons += f;");
-                else
-                    o("      cons += f / %s;", lit(P.v[s]).c_str());
+                emit_alloc(o, P, s, "      ", "      ", "xs" + std::to_string(s), "cons", "f");
+                o("      cons += %s;", consumed(P, s, "f").c_str());
                 if (i == E - 1 || P.sup[i + 1] != s) o("      sc_C[%d * NP + el] = cons;", s);
             }
             o("      sc_R[%d * NP + el] = f;", i);
@@ -679,7 +629,7 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
         snprintf(nb, sizeof(nb), "double x%d", j);
         snprintf(ab, sizeof(ab), "s_X + %d * NP + el", j);
         lds.push_back({nb, ab});
-        if (has_seg[j]) {
+        if (P.has_seg[j]) {
             snprintf(nb, sizeof(nb), "const double c%d", j);
             snprintf(ab, sizeof(ab), "sc_C + %d * NP + el", j);
             lds.push_back({nb, ab});
@@ -714,72 +664,20 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
             }
         }
         for (const Ld& l : lds) o("      %s = *(%s);", l.decl.c_str(), l.addr.c_str());
-        o("      { double arr = 0.0, PC = 0.0, HCp = 0.0;");
-        for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
-            const int i = P.pred_idx[z], L = P.L[i];
-            link_done[i] = 1;
-            if (L == 0)
-                o("        { const double ar = rt%d;", i);
-            else
-                o("        { const double ar = ar%d; *slot%d = rt%d;%s", i, i, i,
-                  P.ring32 ? (std::string(" r32[slot") + std::to_string(i) + " - ring] = (float)rt" + std::to_string(i) + ";").c_str() : "");
-            o("          arr += ar; const double yn = (y%d - ar) + rt%d; s_Y[%d * NP + el] = yn;", i, i, i);
-            o("          PC += %s * rt%d; HCp += %s * (yn > 0.0 ? yn : 0.0); }", lit(P.p[i]).c_str(), i, lit(P.g[i]).c_str());
-        }
-        if (has_seg[j])
-            o("        double x = (x%d + arr) - c%d;", j, j);
-        else
-            o("        double x = (x%d + arr) - 0.0;", j);
-        o("        double SR = 0.0, sold = 0.0, UP = 0.0;");
-        for (int r = 0; r < M; r++) {
-            if (P.rt_node[r] != j) continue;
-            o("        double S%d, U%d;", r, r);
-            o("        { double d;");
-            o("          if (A.demand) d = rint(A.demand[e * A.d_se + %d]);", r);
-            o("          else d = (double)sample_fixed(dem[%d], dem[%d].table, key, episode, t, %du);", r, r, r);
-            o("          d = d > 0.0 ? d : 0.0;");
-            o("          const double fill = d + u%d; const double invr = x > 0.0 ? x : 0.0;", r);
-            o("          S%d = invr < fill ? invr : fill; x = x - S%d; const double un = fill - S%d; U%d = %s;", r, r, r, r,
-              P.backlog ? "un" : "0.0");
-            o("          s_U[%d * NP + el] = U%d;", r, r);
-            o("          if (A.info_demand) A.info_demand[NET_IIDX(A, e, NM, %d)] = d;", r);
-            o("          if (A.info_sales) A.info_sales[NET_IIDX(A, e, NE + NM, %d)] = S%d; }", E + r, r);
-        }
-        o("        s_X[%d * NP + el] = x;", j);
-        for (int z = P.succ_ptr[j]; z < P.succ_ptr[j + 1]; z++) {
-            const int l = P.succ_idx[z];
-            if (l < E)
-                o("        SR += %s * qs%d_%d; sold += qs%d_%d;", lit(P.p[l]).c_str(), j, l, j, l);
-            else {
-                const int r = l - E;
-                if (P.is_retail[j]) o("        UP += %s * U%d;", lit(P.rt_b[r]).c_str(), r);
-                o("        SR += %s * S%d; sold += S%d;", lit(P.rt_p[r]).c_str(), r, r);
-            }
-        }
-        o("        const double xp = x > 0.0 ? x : 0.0; const double HC = %s * xp + HCp; double OC = 0.0;", lit(P.h[j]).c_str());
-        if (P.is_factory[j]) {
-            if (!(P.v[j] > 0.0))
-                o("        OC = 0.0;");
-            else if (P.v[j] == 1.0)
-                o("        OC = %s * sold;", lit(P.o[j]).c_str());
-            else
-                o("        OC = %s * (sold / %s);", lit(P.o[j]).c_str(), lit(P.v[j]).c_str());
-        }
-        o("        (void)sold; const double pj = (((SR - PC) - OC) - HC) - UP; total += pj;");
-        o("        if (A.info_profit) A.info_profit[NET_IIDX(A, e, NJ, %d)] = pj; }", j);
+        emit_visit(j, P.has_seg[j] ? "c" + std::to_string(j) : "0.0", "qs" + std::to_string(j) + "_");
         o("    }");
     }
-    }
     for (int i = 0; i < E; i++) {  // reorder links whose purchaser holds no inventory: pipeline bookkeeping only
-        if (link_done[i]) continue;
+        if (has_pur[i]) continue;
         const int L = P.L[i];
         o("    { const double rt = sc_R[%d * NP + el];", i);
         if (L == 0)
             o("      const double ar = rt;");
         else
-            o("      double* slot = ring + (%d + t %% %d) * NP + el; const double ar = *slot; *slot = rt;%s", P.roff[i], L,
-              P.ring32 ? " r32[slot - ring] = (float)rt;" : "");
+            o("      double* slot = ring + (%d + t %% %d) * NP + el; const double ar = *slot; %s", P.roff[i], L,
+              ring_commit(P, "slot", "rt").c_str());
         o("      s_Y[%d * NP + el] = (s_Y[%d * NP + el] - ar) + rt; }", i, i);
+    }
     }
     o("    const int tn = t + 1; const bool trunc = tn >= NT;");
     o("    if (A.info_profit_total) A.info_profit_total[e] = total;");
@@ -789,16 +687,11 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
     o("        for (int j = 0; j < NJ; j++) X[j] = s_X[j * NP + el];");
     o("        for (int r = 0; r < NM; r++) U[r] = s_U[r * NP + el];");
     o("        write_obs(X, U, ring, el, tn, A.final_obs + e * NOBS); }");
-    for (int j = 0; j < J; j++) o("      s_X[%d * NP + el] = %s;", j, lit(P.I0[j]).c_str());
-    o("      for (int i = 0; i < NE; i++) s_Y[i * NP + el] = 0.0;");
-    o("      for (int r = 0; r < NM; r++) s_U[r * NP + el] = 0.0;");
-    o("      for (int k = 0; k < NSUML; k++) ring[k * NP + el] = 0.0;");
-    if (P.ring32) o("      for (int k = 0; k < NSUML; k++) r32[k * NP + el] = 0.0f;");
-    o("      s_period[el] = 0; s_episode[el] = episode + 1;");
+    emit_reset("      ");
     o("    } else s_period[el] = tn;");
     o("  }");
     // ---- pass C: observation of the final state, 32 columns at a time (only when net_obs_kernel does not follow)
-    if (net_jit_obs_split(P)) {
+    if (plan.obs_kernel) {
         o("}");
         return;
     }
@@ -854,11 +747,7 @@ void emit_step_stream(Src& o, const NetDev& P, int min_blocks) {
 
 int net_jit_build(NetHandle* H, std::string* err) {
     const NetDev& P = H->dev;
-    H->jit_threads = 128;
-    std::string src = net_jit_source(P, H->jit_threads);
-    H->jit_stream = net_jit_uses_stream(P);
-    H->jit_obs_split = H->jit_stream && net_jit_obs_split(P);
-    H->jit_onepass = H->jit_stream && net_jit_onepass(P);
+    std::string src = net_jit_source(P, H->plan);
     int rc = orgym_jit_compile(src, "net_jit_step", &H->jit, err);
     if (rc != 0) return rc;
     if (cudaLibraryGetKernel(&H->jit_rollout, H->jit.lib, "net_jit_rollout") != cudaSuccess) {
@@ -885,13 +774,13 @@ int net_jit_build(NetHandle* H, std::string* err) {
 int net_jit_launch(const NetHandle* H, const NetSimArgs& A_in, cudaStream_t s) {
     const NetDev& P = H->dev;
     NetSimArgs A = A_in;
-    const int nthr = H->jit_threads;
+    const int nthr = NET_JIT_THREADS;
     size_t tile = (size_t)nthr * (P.obs_dim | 1) * 4;
     size_t smem = 16;
-    if (!A.rollout && H->jit_stream) {
+    if (!A.rollout && H->plan.stream) {
         A.use_tile = 0;  // the streaming kernel stages through its own tiles
         // [NTHR][33] float staging tile of pass A (two-pass form) and pass C; the single-pass form stages nothing
-        smem = H->jit_onepass && H->jit_obs_split ? 16 : (size_t)nthr * 33 * 4;
+        smem = H->plan.onepass && H->plan.obs_kernel ? 16 : (size_t)nthr * 33 * 4;
     } else if (!A.rollout) {
         A.use_tile = tile <= 160 * 1024 ? 1 : 0;
         if (A.use_tile) smem = tile;

@@ -46,6 +46,17 @@ def net_params(meta, pkg):
     return pkg.NetInvMgmtParams(**net_kwargs(meta))
 
 
+def set_net_kernel_mode(monkeypatch, mode):
+    """Route the network envs created next through one kernel path: "generic" (constant-bank interpreter),
+    "specialised" (NVRTC, register-resident), or the streaming STEP form forced on a small graph -- "stream_jit"
+    (single pass + observation kernel), "stream_jit_twopass" (two passes with scratch rows), "stream_jit_fused_obs"
+    (the kernel's own observation pass)."""
+    monkeypatch.setenv("ORGYM_NET_JIT", "0" if mode == "generic" else "2")
+    monkeypatch.setenv("ORGYM_NET_JIT_STREAM", "1" if mode.startswith("stream") else "0")
+    monkeypatch.setenv("ORGYM_NET_OBS_TMA", "0" if mode == "stream_jit_fused_obs" else "1")
+    monkeypatch.setenv("ORGYM_NET_JIT_ONEPASS", "0" if mode == "stream_jit_twopass" else "1")
+
+
 def net_S_columns(meta):
     """The reference's S frame is ordered by sorted network_links; ours is reorder links then retail links."""
     nl = [tuple(x) for x in meta["network_links"]]

@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 
 import or_gym_inventory_b200 as pkg
+from helpers import set_net_kernel_mode
 
 pytestmark = pytest.mark.gpu
 PAD = 4096  # bytes on each side
@@ -104,10 +105,8 @@ def test_newsvendor_no_oob_writes(N):
 @pytest.mark.parametrize("N", [1, 127, 129, 600])
 def test_netinv_no_oob_writes(N, mode, monkeypatch):
     torch = _torch()
-    monkeypatch.setenv("ORGYM_NET_JIT", "0" if mode == "generic" else "2")
-    monkeypatch.setenv("ORGYM_NET_JIT_STREAM", "1" if mode.startswith("stream") else "0")
-    monkeypatch.setenv("ORGYM_NET_JIT_ONEPASS", "0" if mode == "stream_jit_twopass" else "1")
-    env = pkg.NetInvMgmtBacklogEnv(num_envs=N, device="cuda:0", autoreset_mode="same_step", num_periods=5)
+    set_net_kernel_mode(monkeypatch, mode)
+    env =pkg.NetInvMgmtBacklogEnv(num_envs=N, device="cuda:0", autoreset_mode="same_step", num_periods=5)
     g = Guard()
     T, J, E, M = 5, 6, 11, 1
     shapes = dict(ep_return=((N,), torch.float64), stats=((N, 4), torch.float64), reward_traj=((N, T), torch.float64),

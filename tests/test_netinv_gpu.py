@@ -3,7 +3,7 @@ import numpy as np
 import pytest
 
 import or_gym_inventory_b200 as pkg
-from helpers import golden_files, ids, load_golden, net_kwargs, net_S_columns, seq_sum
+from helpers import golden_files, ids, load_golden, net_kwargs, net_S_columns, seq_sum, set_net_kernel_mode
 
 pytestmark = pytest.mark.gpu
 NET = golden_files("net_")
@@ -21,12 +21,8 @@ def kernel_mode(request, monkeypatch):
     nodes: the default for large graphs; or two passes with scratch rows, the form for graphs whose suppliers do not
     follow their purchasers in node order) + observation kernel, generated kernel with its own fused observation
     pass --; and the generic constant-bank interpreter."""
-    m = request.param
-    monkeypatch.setenv("ORGYM_NET_JIT", "0" if m == "generic" else "2")
-    monkeypatch.setenv("ORGYM_NET_JIT_STREAM", "1" if m.startswith("stream") else "0")
-    monkeypatch.setenv("ORGYM_NET_OBS_TMA", "0" if m == "stream_jit_fused_obs" else "1")
-    monkeypatch.setenv("ORGYM_NET_JIT_ONEPASS", "0" if m == "stream_jit_twopass" else "1")
-    return m
+    set_net_kernel_mode(monkeypatch, request.param)
+    return request.param
 
 
 def _mk(meta, n, **kw):

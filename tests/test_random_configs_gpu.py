@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 import or_gym_inventory_b200 as pkg
-from helpers import seq_sum
+from helpers import seq_sum, set_net_kernel_mode
 
 pytestmark = pytest.mark.gpu
 # ORGYM_STRESS=k multiplies the number of random cases (one-off soak runs; the default suite stays short)
@@ -140,9 +140,7 @@ def _random_graph(rng, ordered=False):
 def test_netinv_random_graph(case, mode, monkeypatch):
     from oracle import oracle
     torch = _torch()
-    monkeypatch.setenv("ORGYM_NET_JIT", "0" if mode == "generic" else "2")
-    monkeypatch.setenv("ORGYM_NET_JIT_STREAM", "1" if mode.startswith("stream") else "0")
-    monkeypatch.setenv("ORGYM_NET_JIT_ONEPASS", "0" if mode == "stream_jit_twopass" else "1")
+    set_net_kernel_mode(monkeypatch, mode)
     rng = np.random.default_rng(3000 + case)
     g = _random_graph(rng, ordered=bool(case % 2))
     T = int(rng.integers(4, 26))
