@@ -380,9 +380,11 @@ __global__ void __launch_bounds__(ORGYM_TILE, (NS <= 4 && sizeof(S) == 4) ? ORGY
     const int Lm = P.lt_max;
     // The ring / window addresses depend on the env's period, which itself has to be loaded: two dependent round trips
     // to HBM.  When the batch runs in lock-step the host-side handle knows the period (A.t_hint), so the second group
-    // of loads is issued speculatively together with the first; an env whose period differs simply reloads.
+    // of loads is issued speculatively together with the first; an env whose period differs simply reloads.  Rows in
+    // direct mode are not speculated: there the window lands in the caller's row itself, which an env already past
+    // the end (autoreset disabled) has to return unchanged.
     const int t_spec = A.t_hint;
-    const bool spec = valid && t_spec >= 0 && t_spec < P.T;
+    const bool spec = valid && !direct && t_spec >= 0 && t_spec < P.T;
     if (valid) {  // loads that do not depend on the period
         t = st.period[e];
         episode = st.episode[e];
