@@ -415,6 +415,20 @@ int orgym_netinv_export_state(orgym_handle_t h, const void* state_dev, double* X
 
 #define ORGYM_NET_POLICY_ACTIONS 0
 #define ORGYM_NET_POLICY_CONSTANT 1 /* benchmark_NetInvMgmtBacklogEnv.py:119-136: same float32 action vector every period */
+#define ORGYM_NET_POLICY_MLP 2      /* actor network evaluated on the device, in->mlp */
+
+/* ORGYM_NET_POLICY_MLP: a trained actor network (orgym_mlp_t, width[0] = obs_dim, width[num_layers] = E), e.g. the
+ * stable-baselines3 MlpPolicy that benchmark_NetInvMgmtLostSalesEnv_sb3_rllib.py trains, evaluated inside the fused
+ * rollout.  Per period, for each env:
+ *   x    = the float32 observation step() returns: U (M), then X (J), then for each link with L > 0 its pipeline, oldest
+ *          first (:334-413); at t = 0 the reset observation
+ *   h_l, y = exactly the serial env's contract (orgym_mlp_t above): acc = b, then fmaf ascending in k; accurate tanhf
+ *          or NaN-keeping ReLU; no activation after the last Linear
+ *   a_i  = NaN if y_i is NaN, else min(max(y_i, 0f), action_high[i])   (SB3 predict's np.clip to the Box, float32)
+ * a then takes the env's own action rule, exactly like an ORGYM_NET_POLICY_ACTIONS action: rint((double)a), then
+ * max(., 0), so a NaN action orders 0; action_traj_dev records a.  Results are a pure function of (weights, seed, global
+ * env id, episode): independent of batch size and env_offset sharding.  MLP rollouts always run the ahead-of-time kernel,
+ * whatever ORGYM_NET_JIT says (also under ORGYM_NET_JIT=2). */
 
 typedef struct {
     int32_t policy;
@@ -422,6 +436,13 @@ typedef struct {
     int64_t act_stride_env, act_stride_t;
     const double* demand_dev; /* (e,t,r) at [e*stride_env + t*stride_t + r] or NULL */
     int64_t dem_stride_env, dem_stride_t;
+    /* HOST pointers, read at the call only when policy == ORGYM_NET_POLICY_MLP.  mlp: ORGYM_E_INVALID for a missing or
+     * malformed network (layer count, widths outside 1..ORGYM_MLP_MAX_WIDTH, width[0] != obs_dim, width[num_layers] !=
+     * E, null weights); ORGYM_E_UNSUPPORTED, with the sizes in the message, when the weights, activations, observation
+     * and action tiles and work vectors of one CTA do not fit in shared memory even for 32 envs.  action_high:
+     * float32[E], the upper bound of the action Box (single_action_space.high); ORGYM_E_INVALID when NULL. */
+    const orgym_mlp_t* mlp;
+    const float* action_high;
 } orgym_netinv_rollout_in_t;
 
 typedef struct {
@@ -432,6 +453,7 @@ typedef struct {
     double* final_Y_dev;     /* [N,E] */
     double* final_U_dev;     /* [N,M] */
     double* summary_dev;     /* [8] */
+    float* action_traj_dev;  /* [N,T,E] actions the policy took; ORGYM_NET_POLICY_MLP only (ORGYM_E_INVALID otherwise) */
 } orgym_netinv_rollout_out_t;
 
 /* fused reset + num_periods steps; scratch_dev holds the per-env lead-time rings while the rollout runs

@@ -103,12 +103,13 @@ class NetInfo(C.Structure):
 class NetRolloutIn(C.Structure):
     _fields_ = [("policy", C.c_int32), ("actions", C.c_void_p), ("act_stride_env", C.c_int64),
                 ("act_stride_t", C.c_int64), ("demand", C.c_void_p), ("dem_stride_env", C.c_int64),
-                ("dem_stride_t", C.c_int64)]
+                ("dem_stride_t", C.c_int64), ("mlp", C.POINTER(Mlp)), ("action_high", C.c_void_p)]
 
 
 class NetRolloutOut(C.Structure):
     _fields_ = [("ep_return", C.c_void_p), ("stats", C.c_void_p), ("reward_traj", C.c_void_p),
-                ("final_X", C.c_void_p), ("final_Y", C.c_void_p), ("final_U", C.c_void_p), ("summary", C.c_void_p)]
+                ("final_X", C.c_void_p), ("final_Y", C.c_void_p), ("final_U", C.c_void_p), ("summary", C.c_void_p),
+                ("action_traj", C.c_void_p)]
 
 
 # every symbol include/orgym_b200.h declares: name -> (restype, argtypes)

@@ -10,8 +10,11 @@
 //
 //   net_reset_kernel   reset (network_management.py:301-332) + first observation (:334-413)
 //   net_sim_kernel     STEP mode: one period (:436-635) + observation;  ROLLOUT mode: fused reset + T periods
+//   net_mlp_rollout_kernel  the fused rollout with an MLP actor evaluated on the device every period
 //
 // float64 throughout, evaluated in the reference's operation order (Python sum order = adjacency order).
+#include "launch_util.cuh"
+#include "mlp.cuh"
 #include "netinv.cuh"
 
 // t % d for 0 <= t < 2^20, 1 <= d <= 64 (exact, see invmgmt.cu)
@@ -84,8 +87,133 @@ __global__ void __launch_bounds__(128) net_reset_kernel(const __grid_constant__ 
 
 #include "netinv_args.cuh"
 
+// One period (:436-635) of one instance, the body shared by net_sim_kernel and net_mlp_rollout_kernel.  The work vectors
+// sX, sC, sR, sY, sU, sS are shared-memory rows of stride NTHR ([slot][NTHR], this instance's column is tid); the
+// lead-time rings live in ring[slot][NET_TILE] at column el and are written only when `valid`.
+//   arow()        the float32 actions of the period (before the env's rint / max(0, .) rule): link i at arow()[i * ASTRIDE]
+//   demand(r)     demand of retail link r before max(0, .): a replayed value (already rounded) or a draw
+//   on_demand(r, d), on_profit(j, pj)   per-market demand and per-node profit, for the STEP info tensors
+// Accumulates the episode statistics and returns the undiscounted profit of the period, in Python sum order.
+template <int NTHR, int ASTRIDE, class Arow, class Demand, class OnDemand, class OnProfit>
+__device__ __forceinline__ double net_period(const NetDev& P, int tid, int el, double* ring, bool valid, int t,
+                                             double* sX, double* sC, double* sR, double* sY, double* sU, double* sS,
+                                             Arow arow_of, Demand demand, OnDemand on_demand, OnProfit on_profit,
+                                             double& s_sales, double& s_dem, double& s_unf, double& s_inv) {
+    const int J = P.J, E = P.E, M = P.M;
+    constexpr int np_ = NET_TILE;
+    // ---- 0) place orders: sequential greedy allocation in sorted (supplier, purchaser) order (:448-490)
+    for (int j = 0; j < J; j++) sC[j * NTHR + tid] = 0.0;
+    double cons_s = 0.0;
+    const float* arow = arow_of();
+    for (int i = 0; i < E; i++) {
+        double req = rint((double)arow[i * ASTRIDE]);  // Python round(): half to even
+        req = req > 0.0 ? req : 0.0;                   // max(0, .)
+        const int s = P.sup[i];
+        double f = 0.0;
+        if (s == -1)
+            f = req;  // raw material: unlimited (:453-455)
+        else if (s >= 0) {
+            if (i == 0 || P.sup[i - 1] != s) cons_s = 0.0;
+            double avail = sX[s * NTHR + tid] - cons_s;  // :459
+            avail = avail > 0.0 ? avail : 0.0;           // :460
+            double oa = avail;
+            const double vs = P.v[s];
+            if (P.is_factory[s]) {  // :464-478
+                double mp = vs * avail;
+                double lim = mp < P.C[s] ? mp : P.C[s];
+                oa = lim < oa ? lim : oa;
+            }
+            f = oa < req ? oa : req;                 // :481
+            cons_s += vs == 1.0 ? f : f / vs;        // :484-485 (x / 1.0 == x)
+            if (i == E - 1 || P.sup[i + 1] != s) sC[s * NTHR + tid] = cons_s;
+        }
+        sR[i * NTHR + tid] = f;  // R[t] = S[t] = f (:488-490)
+    }
+    // ---- on-hand inventory (:516-528): arrivals R[t-L] summed in predecessor (adjacency) order
+    for (int j = 0; j < J; j++) {
+        double arr = 0.0;
+        for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
+            const int i = P.pred_idx[z], L = P.L[i];
+            arr += L == 0 ? sR[i * NTHR + tid]
+                          : ring[(P.roff[i] + net_mod(t, L, P.Lmagic[i])) * np_ + el];
+        }
+        sX[j * NTHR + tid] = (sX[j * NTHR + tid] + arr) - sC[j * NTHR + tid];
+    }
+    // ---- 1) pipeline inventory (:494-511) and ring commit: slot t % L held R[t-L] and now receives R[t]
+    for (int i = 0; i < E; i++) {
+        const int L = P.L[i];
+        const double rt = sR[i * NTHR + tid];
+        double arriving = rt;
+        if (L > 0) {
+            double* slot = ring + (P.roff[i] + net_mod(t, L, P.Lmagic[i])) * np_ + el;
+            arriving = *slot;
+            if (valid) *slot = rt;
+        }
+        sY[i * NTHR + tid] = (sY[i * NTHR + tid] - arriving) + rt;
+    }
+    // ---- 2-4) market demand, sales, backlog (:536-566)
+    for (int r = 0; r < M; r++) {
+        double d = demand(r);
+        d = d > 0.0 ? d : 0.0;  // max(0, int(round(.))) (:540)
+        const int j = P.rt_node[r];
+        double fill = d + sU[r * NTHR + tid];
+        double x = sX[j * NTHR + tid];
+        double invr = x > 0.0 ? x : 0.0;
+        double sl = invr < fill ? invr : fill;  // min(demand_to_fill, inv) (:548)
+        sS[r * NTHR + tid] = sl;
+        sX[j * NTHR + tid] = x - sl;
+        double un = fill - sl;
+        sU[r * NTHR + tid] = P.backlog ? un : 0.0;  // :560-563
+        s_sales += sl;
+        s_dem += d;
+        s_unf += P.backlog ? un : 0.0;
+        on_demand(r, d);
+    }
+    // ---- 5) profit per node, Python sum order (:578-613)
+    double total = 0.0;
+    for (int j = 0; j < J; j++) {
+        double SR = 0.0, PC = 0.0, HCp = 0.0, sold = 0.0, UP = 0.0;
+        for (int z = P.succ_ptr[j]; z < P.succ_ptr[j + 1]; z++) {
+            const int l = P.succ_idx[z];
+            double q, pr;
+            if (l < E) {
+                q = sR[l * NTHR + tid];
+                pr = P.p[l];
+            } else {
+                q = sS[(l - E) * NTHR + tid];
+                pr = P.rt_p[l - E];
+                UP += P.rt_b[l - E] * sU[(l - E) * NTHR + tid];  // :608
+            }
+            SR += pr * q;  // :582
+            sold += q;     // :599
+        }
+        for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
+            const int i = P.pred_idx[z];
+            PC += P.p[i] * sR[i * NTHR + tid];  // :586
+            double y = sY[i * NTHR + tid];
+            HCp += P.g[i] * (y > 0.0 ? y : 0.0);  // :591
+        }
+        double x = sX[j * NTHR + tid];
+        double xp = x > 0.0 ? x : 0.0;
+        double HC = P.h[j] * xp + HCp;  // :590-593
+        double OC = 0.0;
+        if (P.is_factory[j]) {  // :597-601
+            const double vj = P.v[j];
+            OC = vj > 0.0 ? P.o[j] * (vj == 1.0 ? sold : sold / vj) : 0.0;
+        }
+        if (!P.is_retail[j]) UP = 0.0;             // :605
+        double pj = (((SR - PC) - OC) - HC) - UP;  // :611
+        total += pj;
+        s_inv += xp;
+        on_profit(j, pj);
+    }
+    return total;
+}
+
+// 128 threads: at most 102 registers, so that 5 CTAs (the shared-memory work vectors of small graphs allow 6) stay
+// resident per SM; without the bound ptxas takes 125 and the ROLLOUT mode runs 12 % slower at 4 CTAs/SM.
 template <int NTHR>
-__global__ void __launch_bounds__(NTHR) net_sim_kernel(const __grid_constant__ NetDev P,
+__global__ void __launch_bounds__(NTHR, NTHR == 128 ? 5 : 0) net_sim_kernel(const __grid_constant__ NetDev P,
                                                        const __grid_constant__ NetSimArgs A) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int tid = threadIdx.x;
@@ -164,118 +292,24 @@ __global__ void __launch_bounds__(NTHR) net_sim_kernel(const __grid_constant__ N
     if (!A.rollout && !do_step) t1 = t0;  // nothing to simulate for this lane
 
     for (int t = t0; t < t1; t++) {
-        // ---- 0) place orders: sequential greedy allocation in sorted (supplier, purchaser) order (:448-490)
-        for (int j = 0; j < J; j++) sC[j * NTHR + tid] = 0.0;
-        double cons_s = 0.0;
-        const float* arow = A.policy == ORGYM_NET_POLICY_CONSTANT
-                                ? A.actions
-                                : A.actions + ec * A.a_se + (int64_t)(A.rollout ? t : 0) * A.a_st;
-        for (int i = 0; i < E; i++) {
-            double req = rint((double)arow[i]);  // Python round(): half to even
-            req = req > 0.0 ? req : 0.0;         // max(0, .)
-            const int s = P.sup[i];
-            double f = 0.0;
-            if (s == -1)
-                f = req;  // raw material: unlimited (:453-455)
-            else if (s >= 0) {
-                if (i == 0 || P.sup[i - 1] != s) cons_s = 0.0;
-                double avail = sX[s * NTHR + tid] - cons_s;  // :459
-                avail = avail > 0.0 ? avail : 0.0;           // :460
-                double oa = avail;
-                const double vs = P.v[s];
-                if (P.is_factory[s]) {  // :464-478
-                    double mp = vs * avail;
-                    double lim = mp < P.C[s] ? mp : P.C[s];
-                    oa = lim < oa ? lim : oa;
-                }
-                f = oa < req ? oa : req;                 // :481
-                cons_s += vs == 1.0 ? f : f / vs;        // :484-485 (x / 1.0 == x)
-                if (i == E - 1 || P.sup[i + 1] != s) sC[s * NTHR + tid] = cons_s;
-            }
-            sR[i * NTHR + tid] = f;  // R[t] = S[t] = f (:488-490)
-        }
-        // ---- on-hand inventory (:516-528): arrivals R[t-L] summed in predecessor (adjacency) order
-        for (int j = 0; j < J; j++) {
-            double arr = 0.0;
-            for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
-                const int i = P.pred_idx[z], L = P.L[i];
-                arr += L == 0 ? sR[i * NTHR + tid]
-                              : ring[(P.roff[i] + net_mod(t, L, P.Lmagic[i])) * np_ + el];
-            }
-            sX[j * NTHR + tid] = (sX[j * NTHR + tid] + arr) - sC[j * NTHR + tid];
-        }
-        // ---- 1) pipeline inventory (:494-511) and ring commit: slot t % L held R[t-L] and now receives R[t]
-        for (int i = 0; i < E; i++) {
-            const int L = P.L[i];
-            const double rt = sR[i * NTHR + tid];
-            double arriving = rt;
-            if (L > 0) {
-                double* slot = ring + (P.roff[i] + net_mod(t, L, P.Lmagic[i])) * np_ + el;
-                arriving = *slot;
-                if (valid) *slot = rt;
-            }
-            sY[i * NTHR + tid] = (sY[i * NTHR + tid] - arriving) + rt;
-        }
-        // ---- 2-4) market demand, sales, backlog (:536-566)
-        for (int r = 0; r < M; r++) {
-            double d;
-            if (A.demand) {
-                d = rint(A.demand[ec * A.d_se + (int64_t)(A.rollout ? t : 0) * A.d_st + r]);
-            } else
-                d = (double)sample_fixed(P.dem[r], P.dem[r].table, key, episode, t, (uint32_t)r);
-            d = d > 0.0 ? d : 0.0;  // max(0, int(round(.))) (:540)
-            const int j = P.rt_node[r];
-            double fill = d + sU[r * NTHR + tid];
-            double x = sX[j * NTHR + tid];
-            double invr = x > 0.0 ? x : 0.0;
-            double sl = invr < fill ? invr : fill;  // min(demand_to_fill, inv) (:548)
-            sS[r * NTHR + tid] = sl;
-            sX[j * NTHR + tid] = x - sl;
-            double un = fill - sl;
-            sU[r * NTHR + tid] = P.backlog ? un : 0.0;  // :560-563
-            s_sales += sl;
-            s_dem += d;
-            s_unf += P.backlog ? un : 0.0;
-            if (!A.rollout && A.info_demand && do_step) A.info_demand[NET_IIDX(A, e, M, r)] = d;
-        }
-        // ---- 5) profit per node, Python sum order (:578-613)
-        double total = 0.0;
-        for (int j = 0; j < J; j++) {
-            double SR = 0.0, PC = 0.0, HCp = 0.0, sold = 0.0, UP = 0.0;
-            for (int z = P.succ_ptr[j]; z < P.succ_ptr[j + 1]; z++) {
-                const int l = P.succ_idx[z];
-                double q, pr;
-                if (l < E) {
-                    q = sR[l * NTHR + tid];
-                    pr = P.p[l];
-                } else {
-                    q = sS[(l - E) * NTHR + tid];
-                    pr = P.rt_p[l - E];
-                    UP += P.rt_b[l - E] * sU[(l - E) * NTHR + tid];  // :608
-                }
-                SR += pr * q;  // :582
-                sold += q;     // :599
-            }
-            for (int z = P.pred_ptr[j]; z < P.pred_ptr[j + 1]; z++) {
-                const int i = P.pred_idx[z];
-                PC += P.p[i] * sR[i * NTHR + tid];  // :586
-                double y = sY[i * NTHR + tid];
-                HCp += P.g[i] * (y > 0.0 ? y : 0.0);  // :591
-            }
-            double x = sX[j * NTHR + tid];
-            double xp = x > 0.0 ? x : 0.0;
-            double HC = P.h[j] * xp + HCp;  // :590-593
-            double OC = 0.0;
-            if (P.is_factory[j]) {  // :597-601
-                const double vj = P.v[j];
-                OC = vj > 0.0 ? P.o[j] * (vj == 1.0 ? sold : sold / vj) : 0.0;
-            }
-            if (!P.is_retail[j]) UP = 0.0;             // :605
-            double pj = (((SR - PC) - OC) - HC) - UP;  // :611
-            total += pj;
-            s_inv += xp;
-            if (!A.rollout && A.info_profit && do_step) A.info_profit[NET_IIDX(A, e, J, j)] = pj;
-        }
+        const double total = net_period<NTHR, 1>(
+            P, tid, el, ring, valid, t, sX, sC, sR, sY, sU, sS,
+            [&] {
+                return A.policy == ORGYM_NET_POLICY_CONSTANT
+                           ? A.actions
+                           : A.actions + ec * A.a_se + (int64_t)(A.rollout ? t : 0) * A.a_st;
+            },
+            [&](int r) {
+                return A.demand ? rint(A.demand[ec * A.d_se + (int64_t)(A.rollout ? t : 0) * A.d_st + r])
+                                : (double)sample_fixed(P.dem[r], P.dem[r].table, key, episode, t, (uint32_t)r);
+            },
+            [&](int r, double d) {
+                if (!A.rollout && A.info_demand && do_step) A.info_demand[NET_IIDX(A, e, M, r)] = d;
+            },
+            [&](int j, double pj) {
+                if (!A.rollout && A.info_profit && do_step) A.info_profit[NET_IIDX(A, e, J, j)] = pj;
+            },
+            s_sales, s_dem, s_unf, s_inv);
         last_reward = P.disc[t] * total;  // :619
         ret += last_reward;
         if (A.rollout && A.reward_traj && valid) A.reward_traj[e * P.T + t] = last_reward;
@@ -544,6 +578,195 @@ static void net_launch(const NetHandle* H, const NetSimArgs& A, size_t smem, cud
         net_sim_kernel<64><<<grid, 64, smem, s>>>(H->dev, A);
     else
         net_sim_kernel<32><<<grid, 32, smem, s>>>(H->dev, A);
+}
+
+// ---- fused rollout driven by an MLP actor (ORGYM_NET_POLICY_MLP) -----------------------------------------------------
+// One CTA of MLP_THREADS threads = the NET_TILE = 128 consecutive envs of one rollout scratch tile (their lead-time rings
+// stay there, [slot][128], as in net_sim_kernel's ROLLOUT mode) and one row of the partial sums.  The CTA runs them as
+// 128 / ESUB sub-tiles of ESUB envs one after the other; weights and biases are staged in shared memory once per CTA
+// (mlp.cuh).  Thread tid < ESUB owns env e0 + tid of the current sub-tile: its float64 work vectors are column tid of
+// [slot][ESUB] rows, its accumulators live in its registers.  The float32 observation tile [obs_dim][ESUB] is the
+// network's input: U and X rows are rewritten after each period, the pipeline rows shifted left in place and appended
+// with the orders fulfilled (R[t], what the ring receives).  Per period the whole CTA runs the hidden layers and then
+// the last layer into the action tile [E][ESUB] (one barrier each); the owner threads take the period through
+// net_period, the same code as net_sim_kernel, with that tile as the requests.
+struct NetMlpArgs {
+    MlpNet net;
+    int obs_off, buf_off[2], act_off;  // float offsets in dynamic shared memory (the weights start at 0)
+    int work_off;                      // byte offset of the float64 work vectors
+    float* action_traj;                // [N,T,E] or NULL
+    float hi[NE];                      // upper bound of the action Box
+};
+
+template <int ESUB>
+__global__ void __launch_bounds__(MLP_THREADS, 2) net_mlp_rollout_kernel(const __grid_constant__ NetDev P,
+                                                                        const __grid_constant__ NetSimArgs A,
+                                                                        const __grid_constant__ NetMlpArgs M) {
+    static_assert(NET_TILE % ESUB == 0 && ESUB % 32 == 0 && ESUB <= MLP_THREADS, "sub-tiles of whole warps");
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ double red[NET_TILE / 32][7];
+    constexpr int log2E = ESUB == 64 ? 6 : 5;
+    const int tid = threadIdx.x, NL = M.net.L, J = P.J, E = P.E, Mk = P.M, T = P.T;
+    float* fs = (float*)smem;
+    float* obs = fs + M.obs_off;
+    float* act = fs + M.act_off;
+    double* sX = (double*)(smem + M.work_off);  // [J]
+    double* sC = sX + J * ESUB;                 // [J]
+    double* sR = sC + J * ESUB;                 // [E]
+    double* sY = sR + E * ESUB;                 // [E]
+    double* sU = sY + E * ESUB;                 // [M]
+    double* sS = sU + Mk * ESUB;                // [M]
+    mlp_stage_weights(M.net, fs);
+    const int Klast = M.net.K[NL - 1];
+    const float* Wlast = fs + M.net.w_off[NL - 1];
+    const float* blast = fs + M.net.b_off[NL - 1];
+    const float* hin = NL == 1 ? obs : fs + M.buf_off[(NL - 2) & 1];  // input of the last layer
+    double* ring = NetState((char*)A.state + (int64_t)blockIdx.x * net_tile_bytes(P), P).ring;
+    const bool owner = tid < ESUB;
+    for (int sub = 0; sub < NET_TILE / ESUB; sub++) {
+        const int64_t e0 = (int64_t)blockIdx.x * NET_TILE + (int64_t)sub * ESUB;
+        const int64_t e = e0 + tid;
+        const bool valid = owner && e < A.N;
+        const int64_t ec = valid ? e : 0;  // clamp so that idle lanes stay in bounds
+        const int el = sub * ESUB + tid;   // column of the scratch tile
+        if (e0 >= A.N) {  // CTA-uniform: the sums of the missing warps are zero, like idle lanes of net_sim_kernel
+            if (tid < 7 * (ESUB / 32)) red[sub * (ESUB / 32) + tid / 7][tid % 7] = 0.0;
+            continue;
+        }
+        const uint64_t key = A.seed + (uint64_t)(A.env_offset + e);
+        double ret = 0.0, s_sales = 0.0, s_dem = 0.0, s_unf = 0.0, s_inv = 0.0;
+        if (owner) {  // reset (:326) and its observation [0 (M), I0 (J), 0 ...]
+            for (int j = 0; j < J; j++) sX[j * ESUB + tid] = P.I0[j];
+            for (int i = 0; i < E; i++) sY[i * ESUB + tid] = 0.0;
+            for (int r = 0; r < Mk; r++) sU[r * ESUB + tid] = 0.0;
+            if (valid)
+                for (int k = 0; k < P.sumL; k++) ring[k * NET_TILE + el] = 0.0;
+            for (int z = 0; z < P.obs_dim; z++)
+                obs[z * ESUB + tid] = (z >= Mk && z < Mk + J) ? (float)P.I0[z - Mk] : 0.0f;
+        }
+        __syncthreads();
+        for (int t = 0; t < T; t++) {
+            const float* in = obs;
+            for (int l = 0; l < NL - 1; l++) {
+                float* out = fs + M.buf_off[l & 1];
+                mlp_hidden_layer(in, out, fs + M.net.w_off[l], fs + M.net.b_off[l], M.net.K[l], M.net.Np[l], ESUB, log2E,
+                                 M.net.act);
+                __syncthreads();
+                in = out;
+            }
+            // last layer: acc = b, then K ascending FMAs, no activation; then np.clip to the action Box in float32, NaN kept
+            for (int idx = tid; idx < E * ESUB; idx += MLP_THREADS) {
+                const int n = idx >> log2E, c = idx & (ESUB - 1);
+                float y = blast[n];
+                for (int k = 0; k < Klast; k++) y = __fmaf_rn(Wlast[n * Klast + k], hin[k * ESUB + c], y);
+                float a = y > 0.0f ? y : 0.0f;
+                a = a < M.hi[n] ? a : M.hi[n];
+                a = y != y ? y : a;
+                act[idx] = a;
+                if (M.action_traj && e0 + c < A.N) M.action_traj[((e0 + c) * T + t) * E + n] = a;
+            }
+            __syncthreads();
+            if (owner) {
+                const double total = net_period<ESUB, ESUB>(
+                    P, tid, el, ring, valid, t, sX, sC, sR, sY, sU, sS, [&] { return (const float*)act + tid; },
+                    [&](int r) {
+                        return A.demand ? rint(A.demand[ec * A.d_se + (int64_t)t * A.d_st + r])
+                                        : (double)sample_fixed(P.dem[r], P.dem[r].table, key, A.episode, t, (uint32_t)r);
+                    },
+                    [](int, double) {}, [](int, double) {}, s_sales, s_dem, s_unf, s_inv);
+                const double rw = P.disc[t] * total;  // :619
+                ret += rw;
+                if (valid && A.reward_traj) A.reward_traj[e * T + t] = rw;
+                // observation of period t + 1 (:334-413)
+                for (int r = 0; r < Mk; r++) obs[r * ESUB + tid] = (float)sU[r * ESUB + tid];
+                for (int j = 0; j < J; j++) obs[(Mk + j) * ESUB + tid] = (float)sX[j * ESUB + tid];
+                int k = Mk + J;
+                for (int i = 0; i < E; i++) {
+                    const int L = P.L[i];
+                    if (L == 0) continue;  // :353
+                    for (int q = 0; q + 1 < L; q++) obs[(k + q) * ESUB + tid] = obs[(k + q + 1) * ESUB + tid];
+                    obs[(k + L - 1) * ESUB + tid] = (float)sR[i * ESUB + tid];
+                    k += L;
+                }
+            }
+            __syncthreads();
+        }
+        if (valid) {
+            if (A.ep_return) A.ep_return[e] = ret;
+            if (A.stats) {
+                A.stats[e * 4 + 0] = s_sales; A.stats[e * 4 + 1] = s_dem; A.stats[e * 4 + 2] = s_unf; A.stats[e * 4 + 3] = s_inv;
+            }
+            if (A.final_X) for (int j = 0; j < J; j++) A.final_X[e * J + j] = sX[j * ESUB + tid];
+            if (A.final_Y) for (int i = 0; i < E; i++) A.final_Y[e * E + i] = sY[i * ESUB + tid];
+            if (A.final_U) for (int r = 0; r < Mk; r++) A.final_U[e * Mk + r] = sU[r * ESUB + tid];
+        }
+        if (A.partials && owner) {  // warp of 32 consecutive envs: the xor tree of net_sim_kernel<128>
+            const double v[7] = {valid ? 1.0 : 0.0, valid ? ret : 0.0, valid ? ret * ret : 0.0, valid ? s_sales : 0.0,
+                                 valid ? s_dem : 0.0, valid ? s_unf : 0.0, valid ? s_inv : 0.0};
+#pragma unroll
+            for (int z = 0; z < 7; z++) {
+                double x = v[z];
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+                if ((tid & 31) == 0) red[sub * (ESUB / 32) + (tid >> 5)][z] = x;
+            }
+        }
+    }
+    if (A.partials) {
+        __syncthreads();
+        if (tid < 7) {  // the four warps in order, as net_sim_kernel<128>
+            double x = 0.0;
+            for (int wv = 0; wv < NET_TILE / 32; wv++) x += red[wv][tid];
+            A.partials[(size_t)blockIdx.x * 8 + tid] = x;
+        }
+    }
+}
+
+// Checks an orgym_mlp_t and the action bound against the graph (ORGYM_E_INVALID) and lays out one CTA's shared memory
+// for it: the largest sub-tile of ESUB in {64, 32} envs whose working set fits (ORGYM_E_UNSUPPORTED, with the sizes,
+// when none does).
+static int net_mlp_plan(const NetDev& P, const orgym_mlp_t* mlp, const float* action_high, NetMlpArgs* M, int* esub,
+                        size_t* smem_out) {
+    ORGYM_REQUIRE(mlp, "policy ORGYM_NET_POLICY_MLP needs in->mlp");
+    ORGYM_REQUIRE(action_high, "policy ORGYM_NET_POLICY_MLP needs in->action_high");
+    if (P.obs_dim > ORGYM_MLP_MAX_WIDTH && mlp->width[0] == P.obs_dim) {  // large graphs: the input alone does not fit
+        const size_t need = 4 * (size_t)P.obs_dim * (round_up(std::max(mlp->width[1], 1), MLP_TN) + 32);
+        orgym_set_error("mlp: the observation has %d values (at most %d): one CTA of 32 envs needs at least %zu bytes of "
+                        "shared memory for the first layer's weights and the observation tile; this build's limit is %d",
+                        P.obs_dim, ORGYM_MLP_MAX_WIDTH, need, MLP_SMEM_BUDGET);
+        return ORGYM_E_UNSUPPORTED;
+    }
+    memset(M, 0, sizeof(*M));
+    if (int rc = mlp_net_plan(mlp, P.obs_dim, P.E, "the number of reorder links", &M->net)) return rc;
+    for (int i = 0; i < P.E; i++) M->hi[i] = action_high[i];
+    const int L = M->net.L, hmax = M->net.hmax;
+    const int nbuf = L >= 3 ? 2 : (L == 2 ? 1 : 0);
+    const size_t work = 8 * (size_t)(2 * P.J + 2 * P.E + 2 * P.M);  // bytes per env
+    size_t smem = 0;
+    for (int E = 64; E >= 32; E /= 2) {
+        int g = M->net.wfloats;
+        M->obs_off = g;
+        g += (int)round_up((int64_t)P.obs_dim * E, 4);
+        M->buf_off[0] = g;
+        g += nbuf >= 1 ? hmax * E : 0;
+        M->buf_off[1] = g;
+        g += nbuf >= 2 ? hmax * E : 0;
+        M->act_off = g;
+        g += P.E * E;
+        M->work_off = (int)round_up((int64_t)g * 4, 16);
+        smem = (size_t)M->work_off + work * E;
+        *esub = E;
+        if (smem <= MLP_SMEM_BUDGET) break;
+    }
+    if (smem > MLP_SMEM_BUDGET) {
+        orgym_set_error("mlp: one CTA of 32 envs needs %zu bytes of shared memory (weights and biases %d floats, observation "
+                        "tile %d x 32, %d activation tile(s) %d x 32, action tile %d x 32, work vectors %zu bytes x 32); "
+                        "this build's limit is %d",
+                        smem, M->net.wfloats, P.obs_dim, nbuf, hmax, P.E, work, MLP_SMEM_BUDGET);
+        return ORGYM_E_UNSUPPORTED;
+    }
+    *smem_out = smem;
+    return ORGYM_OK;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -826,9 +1049,17 @@ extern "C" int orgym_netinv_rollout(orgym_handle_t h, void* scratch_dev, uint64_
     if (orgym_check_handle(h, FAM_NETINV)) return ORGYM_E_INVALID;
     NetHandle* H = (NetHandle*)h;
     ORGYM_REQUIRE(in && out && scratch_dev, "null argument");
-    ORGYM_REQUIRE(in->policy == ORGYM_NET_POLICY_ACTIONS || in->policy == ORGYM_NET_POLICY_CONSTANT, "unknown policy %d",
-                  in->policy);
-    ORGYM_REQUIRE(in->actions_dev, "actions_dev is required");
+    ORGYM_REQUIRE(in->policy == ORGYM_NET_POLICY_ACTIONS || in->policy == ORGYM_NET_POLICY_CONSTANT ||
+                      in->policy == ORGYM_NET_POLICY_MLP,
+                  "unknown policy %d", in->policy);
+    const bool mlp = in->policy == ORGYM_NET_POLICY_MLP;
+    ORGYM_REQUIRE(mlp || in->actions_dev, "actions_dev is required");
+    ORGYM_REQUIRE(mlp || !out->action_traj_dev, "action_traj_dev is written only by ORGYM_NET_POLICY_MLP rollouts");
+    NetMlpArgs MA;
+    int esub = 0;
+    size_t mlp_smem = 0;
+    if (mlp)
+        if (int rc = net_mlp_plan(H->dev, in->mlp, in->action_high, &MA, &esub, &mlp_smem)) return rc;
     DeviceGuard g(H->base.device);
     NetSimArgs A;
     memset(&A, 0, sizeof(A));
@@ -852,9 +1083,18 @@ extern "C" int orgym_netinv_rollout(orgym_handle_t h, void* scratch_dev, uint64_
     A.final_Y = out->final_Y_dev;
     A.final_U = out->final_U_dev;
     A.partials = out->summary_dev ? H->partials : nullptr;
-    const int thr = H->jit.fn ? NET_JIT_THREADS : H->threads;
+    const int thr = mlp ? NET_TILE : H->jit.fn ? NET_JIT_THREADS : H->threads;
     int nblocks = (int)((A.N + thr - 1) / thr);
-    if (H->jit.fn) {
+    if (mlp) {  // always the ahead-of-time kernel, whatever ORGYM_NET_JIT says
+        MA.action_traj = out->action_traj_dev;
+        if (esub == 64) {
+            orgym_ensure_dyn_smem<net_mlp_rollout_kernel<64>>(mlp_smem);
+            net_mlp_rollout_kernel<64><<<nblocks, MLP_THREADS, mlp_smem, (cudaStream_t)stream>>>(H->dev, A, MA);
+        } else {
+            orgym_ensure_dyn_smem<net_mlp_rollout_kernel<32>>(mlp_smem);
+            net_mlp_rollout_kernel<32><<<nblocks, MLP_THREADS, mlp_smem, (cudaStream_t)stream>>>(H->dev, A, MA);
+        }
+    } else if (H->jit.fn) {
         int rc = net_jit_launch(H, A, (cudaStream_t)stream);
         if (rc != ORGYM_OK) return rc;
     } else

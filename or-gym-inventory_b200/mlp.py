@@ -1,6 +1,7 @@
 """Actor networks evaluated inside the fused rollouts (orgym_mlp_t): which torch modules qualify and how they are packed.
 
-Shared by the serial env (InvManagement*Env.rollout / evaluate) and the newsvendor (NewsvendorEnv.rollout / evaluate)."""
+Shared by the serial env (InvManagement*Env.rollout / evaluate), the newsvendor (NewsvendorEnv.rollout / evaluate) and
+the network env (NetInvMgmt*Env.rollout / evaluate)."""
 from . import _capi
 from ._capi import MLP_RELU, MLP_TANH
 

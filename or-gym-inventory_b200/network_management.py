@@ -12,6 +12,7 @@ from typing import Any, Dict, List, Optional, Tuple
 import numpy as np
 
 from . import _capi
+from .mlp import pack_mlp
 from .spaces import Box
 from .vector import BatchedEnv, _AUTORESET, _torch
 
@@ -19,6 +20,9 @@ try:
     import networkx as nx
 except Exception:  # noqa: BLE001  pragma: no cover
     nx = None
+
+
+POLICY_MLP = 2
 
 
 def _np_poisson_marker(**p):  # stands in for `lambda **p: self.np_random.poisson(**p)` of the default graph
@@ -495,15 +499,28 @@ class NetInvMgmtMasterEnv(BatchedEnv):
                 time_major=False, want=("ep_return", "stats", "summary"), buffer_set=0):
         """Fused reset + num_periods steps (K5).  policy 'constant': the ConstantOrderAgent action
         (high * order_fraction as float32, benchmark_NetInvMgmtBacklogEnv.py:119-136) or an explicit float32[E]
-        `actions` vector; policy 'actions': float32 [N,T,E] ([T,N,E] if time_major).  demand: optional float64
+        `actions` vector; policy 'actions': float32 [N,T,E] ([T,N,E] if time_major); or an actor network -- a
+        torch.nn.Sequential (Linear, Tanh|ReLU, ..., Linear) or an SB3 ActorCriticPolicy (e.g. `model.policy` of a
+        trained PPO) -- evaluated on the device every period on the observation step() would return, its output
+        clipped to [0, single_action_space.high] like SB3's deterministic predict.  demand: optional float64
         [N,T,M].  Returns device tensors ep_return, stats [N,4] (sum retail sales, demand, backlog, on-hand),
-        summary [8]; on request reward_traj, final_X, final_Y, final_U."""
+        summary [8]; on request reward_traj, final_X, final_Y, final_U and, for a network, action_traj
+        (float32 [N,T,E], the actions it took)."""
         torch = _torch()
         N, T = self.num_envs, int(self.num_periods)
         J, E, M = len(self.main_nodes), len(self.reorder_links), len(self.retail_links)
         rin = _capi.NetRolloutIn()
         keep = []
-        if policy == "constant":
+        if not isinstance(policy, str):
+            mlp, tensors = pack_mlp(policy, self.obs_dim, E, self.device)
+            high = np.ascontiguousarray(self.single_action_space.high, dtype=np.float32)
+            keep += [mlp, tensors, high]
+            rin.policy = POLICY_MLP
+            rin.mlp = C.pointer(mlp)
+            rin.action_high = high.ctypes.data
+        elif "action_traj" in want:
+            raise ValueError("action_traj is recorded only for an actor network policy")
+        elif policy == "constant":
             rin.policy = 1
             if actions is None:
                 actions = (self.single_action_space.high * order_fraction).astype(np.float32)
@@ -514,8 +531,9 @@ class NetInvMgmtMasterEnv(BatchedEnv):
             rin.act_stride_env, rin.act_stride_t = (E, N * E) if time_major else (T * E, E)
         else:
             raise ValueError(policy)
-        keep.append(a)
-        rin.actions = a.data_ptr()
+        if rin.policy != POLICY_MLP:
+            keep.append(a)
+            rin.actions = a.data_ptr()
         if demand is not None:
             d = self._to_dev(demand, torch.float64, (T, N, M) if time_major else (N, T, M))
             keep.append(d)
@@ -523,7 +541,8 @@ class NetInvMgmtMasterEnv(BatchedEnv):
             rin.dem_stride_env, rin.dem_stride_t = (M, N * M) if time_major else (T * M, M)
         shapes = dict(ep_return=((N,), torch.float64), stats=((N, 4), torch.float64),
                       reward_traj=((N, T), torch.float64), final_X=((N, J), torch.float64),
-                      final_Y=((N, E), torch.float64), final_U=((N, M), torch.float64), summary=((8,), torch.float64))
+                      final_Y=((N, E), torch.float64), final_U=((N, M), torch.float64), summary=((8,), torch.float64),
+                      action_traj=((N, T, E), torch.float32))
         out = {}
         rout = _capi.NetRolloutOut()
         cache = self.__dict__.setdefault("_rollout_buf", {}).setdefault(int(buffer_set), {})
